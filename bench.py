@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- KKT factor+solves/sec on the BASELINE.json configurations.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config C4|C2|C1|C3]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config C4|C2|C1|C3] [--dump-outputs DIR]
 
 One "step" (= one KKT unit) = one interior-point iteration's KKT work (SURVEY 8d): NT scaling of (v,s) ->
 Atil = F^-T A -> H = Q + Atil'Atil (DMMA SYRK) -> [NCCL all-reduce of the partial Gram matrices when A is
@@ -62,7 +62,14 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the parity block")
     ap.add_argument("--cpu-budget", type=float, default=0.0,
                     help="seconds of CPU row work (default: 100 for --impl reference, 15 for the cpu_baseline leg)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed unit returned as DIR/<name>.npy (float64), to compare two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm times synthetic row slabs, not a KKT unit)")
+    return args
 
 
 def workload_name(cfg, n, m):
@@ -364,12 +371,12 @@ def device_qp(cb, torch, D, n, m, seed, ngpus_single=1):
 
 
 def timed_unit_loop(torch, D, eng, pts, rhs, steps, warmup, sample_clocks):
-    """W warm-up units, then exactly K timed units between barriers; CUDA events on the launching stream."""
+    """W warm-up units, then exactly K timed units between barriers; CUDA events on the launching stream.
+    Also returns what the last timed unit returned: lambda and one (dy, dw, dv) per right-hand side."""
     def unit(i):
         v, s = pts[i % len(pts)]
-        eng.factor_from_point(v, s)
-        for ry, rw, rv in rhs:
-            eng.solve(ry, rw, rv)
+        lam = eng.factor_from_point(v, s)
+        return lam, [eng.solve(ry, rw, rv) for ry, rw, rv in rhs]
     for i in range(warmup):
         unit(i)
     st0 = eng.stats()
@@ -381,7 +388,7 @@ def timed_unit_loop(torch, D, eng, pts, rhs, steps, warmup, sample_clocks):
     phases = {k: [] for k in ("ms_scale", "ms_syrk", "ms_allreduce", "ms_chol", "ms_schur", "ms_solve")}
     e0.record()
     for i in range(steps):
-        unit(i)
+        last = unit(i)
         st = eng.stats()
         for k in phases:
             phases[k].append(st[k])
@@ -391,7 +398,33 @@ def timed_unit_loop(torch, D, eng, pts, rhs, steps, warmup, sample_clocks):
     clocks = sampler.stop() if (sample_clocks and D.rank == 0) else None
     launches = eng.stats()["kernel_launches"] - st0["kernel_launches"]
     avg = {k: sum(v) / len(v) for k, v in phases.items()}
-    return ms_total / steps, clocks, int(launches), avg
+    return ms_total / steps, clocks, int(launches), avg, last
+
+
+DUMP_CAP_BYTES = 64 << 20
+
+
+def dump_outputs(torch, D, out_dir, lam, sols):
+    """Writes lambda and every solve's (dy, dw, dv) as out_dir/<name>.npy in float64.  m-length vectors of a torchrun
+    launch are gathered to rank 0 first.  A vector longer than its share of DUMP_CAP_BYTES is replaced by the entries
+    at a fixed seeded choice of indices, the same in every run of the same shape."""
+    import numpy as np
+    arrays = {"lambda": lam}
+    for k, (dy, dw, dv) in enumerate(sols):
+        arrays.update({f"dy{k}": dy, f"dw{k}": dw, f"dv{k}": dv})
+    arrays = {k: x for k, x in arrays.items() if x is not None and len(x) > 0}
+    if D.world > 1:                                   # lambda and dv are this rank's rows; dy is replicated
+        arrays.update({k: _gather(torch, D, x) for k, x in arrays.items() if k == "lambda" or k.startswith("dv")})
+    if D.rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_CAP_BYTES // 8 // len(arrays)
+    for k, x in arrays.items():
+        x = x.cpu().numpy() if hasattr(x, "cpu") else np.asarray(x)
+        if x.size > share:
+            x = x[np.sort(np.random.default_rng(0).choice(x.size, share, replace=False))]
+        np.save(os.path.join(out_dir, f"{k}.npy"), x.astype(np.float64))
+    print(f"[bench] wrote {', '.join(arrays)} to {out_dir}", file=sys.stderr, flush=True)
 
 
 def e2e_unit_loop(torch, D, eng, pts, rhs, steps, n, m_loc, p):
@@ -502,10 +535,13 @@ def run_b200(args, n, m):
         print(f"[bench] setup {t_setup:.1f} s ({cfg}, n={n}, m={m}, gpus={args.gpus}, "
               f"{'single process' if single_process else 'torchrun' if D.world > 1 else 'one GPU'})", file=sys.stderr, flush=True)
 
-    ms_step, clocks, launches, ph = timed_unit_loop(torch, D, eng, pts, rhs, args.steps, args.warmup, True)
+    ms_step, clocks, launches, ph, (lam_last, sols_last) = timed_unit_loop(torch, D, eng, pts, rhs, args.steps, args.warmup, True)
     value = 1e3 / ms_step
     if D.rank == 0:
         print(f"[bench] device-resident: {ms_step:.2f} ms/step", file=sys.stderr, flush=True)
+    if args.dump_outputs:
+        dump_outputs(torch, D, args.dump_outputs, lam_last, sols_last)
+    del lam_last, sols_last
     e2e = e2e_unit_loop(torch, D, eng, pts, rhs, max(2, min(args.steps, 3)), n, m_loc, p)
 
     # ---- roofline of the dominant kernel (gemm_nt as the SYRK), CUDA events recorded by the library on the
@@ -658,7 +694,7 @@ def run_b200(args, n, m):
         pts2 = [(rnd(m2, 0.5), rnd(m2, 0.5)) for _ in range(2)]
         rhs2 = [(torch.randn(n2, generator=g, dtype=torch.float64, device="cuda"), None,
                  torch.randn(m2, generator=g, dtype=torch.float64, device="cuda")) for _ in range(NSOLVES)]
-        ms2, _, l2, ph2 = timed_unit_loop(torch, D, pr2["eng"], pts2, rhs2, max(args.steps, 10), max(args.warmup, 3), False)
+        ms2, _, l2, ph2, _ = timed_unit_loop(torch, D, pr2["eng"], pts2, rhs2, max(args.steps, 10), max(args.warmup, 3), False)
         e2e2 = e2e_unit_loop(torch, D, pr2["eng"], pts2, rhs2, 5, n2, m2, 0)
         c2 = {"workload": workload_name("C2", n2, m2), "value": 1e3 / ms2, "unit": UNIT, "ms_per_step": ms2,
               "e2e": {k: e2e2[k] for k in ("value", "ms_per_step", "h2d_bytes_per_step", "d2h_bytes_per_step")},

@@ -1,7 +1,7 @@
 """C5-shaped LP (R rows + one S(64) block + sparse equalities): iteration counts of the device path with and
 without the H + rho G'G augmentation, against the oracle's 29 (kktsolver_qr and kktsolver_chol agree)."""
-import sys
-sys.path.insert(0, '/root/repo')
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import conicip_b200 as cb
 from conicip_b200 import problems as P

@@ -1,7 +1,7 @@
 """Cholesky alone (cip_factor_H after cip_form_H) at several n: CUDA-event time and TFLOP/s.
 usage: python scripts/chol_timing.py [n ...]   (env CIP_CHOL_OUTER selects the outer panel width)"""
-import sys
-sys.path.insert(0, '/root/repo')
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch, scipy.sparse as sp
 import conicip_b200 as cb
 

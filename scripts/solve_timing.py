@@ -1,5 +1,5 @@
-import sys, time
-sys.path.insert(0, '/root/repo')
+import os, sys, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, scipy.sparse as sp
 import conicip_b200 as cb
 from conicip_b200 import problems as P

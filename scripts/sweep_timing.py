@@ -1,7 +1,7 @@
 """Triangular sweeps alone (cip_solve_H): correctness against the factor read back, and CUDA-event timing.
 usage: python scripts/sweep_timing.py [n ...]"""
-import sys
-sys.path.insert(0, '/root/repo')
+import os, sys
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, scipy.sparse as sp
 import conicip_b200 as cb
 

@@ -195,9 +195,7 @@ def test_shard_plan_matches_python_mirror():
                 off += k
 
 
-def test_bench_host_problem_c5_and_cpu_unit():
-    """The host side of `bench.py --config C5` at a reduced size: the MOI-shaped LP with an S block of order 64, the
-    synthetic interior points (S rows: vecm of a positive definite matrix) and one CPU unit through the oracle."""
+def _load_bench():
     import importlib.util
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -205,6 +203,13 @@ def test_bench_host_problem_c5_and_cpu_unit():
     bench = importlib.util.module_from_spec(spec)
     sys.modules["bench_mod"] = bench
     spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_host_problem_c5_and_cpu_unit():
+    """The host side of `bench.py --config C5` at a reduced size: the MOI-shaped LP with an S block of order 64, the
+    synthetic interior points (S rows: vecm of a positive definite matrix) and one CPU unit through the oracle."""
+    bench = _load_bench()
     prob, pts, rhs = bench.host_problem("C5", 2200, 2200 + 2080)
     assert prob["cone_dims"] == [("R", 2200), ("S", 2080)] and prob["A"].shape == (4280, 2200) and prob["G"].shape[0] > 0
     for v, s in pts:
@@ -212,6 +217,28 @@ def test_bench_host_problem_c5_and_cpu_unit():
             assert x[:2200].min() > 0 and np.linalg.eigvalsh(O.mat(x[2200:])).min() > 0
     assert len(rhs) == bench.NSOLVES
     assert 0 < bench.cpu_unit_oracle(prob, pts, rhs, repeats=1) < 120
+
+
+def test_bench_dump_outputs_files_and_size_cap(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs DIR`: lambda and every solve's (dy, dv) as float64 .npy (an empty dw, p = 0, is left
+    out); a vector over its share of the size cap becomes a sample that is the same in every run."""
+    import types
+    bench = _load_bench()
+    D = types.SimpleNamespace(world=1, rank=0)
+    rng = np.random.default_rng(3)
+    lam = rng.standard_normal(1000)
+    sols = [(rng.standard_normal(10), np.zeros(0), rng.standard_normal(1000)) for _ in range(bench.NSOLVES)]
+    bench.dump_outputs(None, D, str(tmp_path / "a"), lam, sols)
+    got = {p.stem: np.load(p) for p in (tmp_path / "a").iterdir()}
+    assert sorted(got) == ["dv0", "dv1", "dy0", "dy1", "lambda"]
+    assert all(x.dtype == np.float64 for x in got.values())
+    assert np.array_equal(got["lambda"], lam) and np.array_equal(got["dv1"], sols[1][2])
+    monkeypatch.setattr(bench, "DUMP_CAP_BYTES", 5 * 8 * 100)           # 100 entries for each of the 5 vectors
+    for d in ("b", "c"):
+        bench.dump_outputs(None, D, str(tmp_path / d), lam, sols)
+    b, c = np.load(tmp_path / "b" / "lambda.npy"), np.load(tmp_path / "c" / "lambda.npy")
+    assert len(b) == 100 and np.array_equal(b, c) and np.isin(b, lam).all()
+    assert np.array_equal(np.load(tmp_path / "b" / "dy0.npy"), sols[0][0])
 
 
 def test_ncu_traffic_table_matches_the_committed_captures():
