@@ -19,7 +19,12 @@ CONE_CODE = {"R": CONE_R, "Q": CONE_Q, "S": CONE_S}
 class Options(C.Structure):
     _fields_ = [("struct_size", C.c_int), ("device", C.c_int), ("reg_delta", C.c_double),
                 ("reg_eps_G", C.c_double), ("q_kind", C.c_int), ("verbose", C.c_int), ("dist_chol", C.c_int), ("aug_rho", C.c_double),
-                ("ngpus", C.c_int), ("fold_scaling", C.c_int)]
+                ("ngpus", C.c_int), ("fold_scaling", C.c_int), ("row_structure", C.c_int)]
+
+
+class StructureInfo(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("enabled", C.c_int), ("singleton_rows", C.c_int), ("empty_rows", C.c_int),
+                ("rest_rows", C.c_int), ("rest_cols", C.c_int), ("compressed", C.c_int), ("base_has_gtg", C.c_int)]
 
 
 class Stats(C.Structure):
@@ -89,6 +94,7 @@ SIGNATURES = {
     "cip_mul_Q": (C.c_int, [C.c_void_p, _P, _P]),
     "cip_ipm_solve": (C.c_int, [C.c_void_p, _P, _P, _P, C.POINTER(IpmOptions), _P, _P, _P, C.POINTER(IpmResult)]),
     "cip_stats": (C.c_int, [C.c_void_p, C.POINTER(Stats)]),
+    "cip_structure_info": (C.c_int, [C.c_void_p, C.POINTER(StructureInfo)]),
     "cip_get_H": (C.c_int, [C.c_void_p, _P, C.c_int]),
     "cip_form_H": (C.c_int, [C.c_void_p]),
     "cip_factor_H": (C.c_int, [C.c_void_p]),

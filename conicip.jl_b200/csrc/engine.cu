@@ -135,8 +135,6 @@ int finish(cip_engine* h) {
   return 0;
 }
 
-size_t opts_size(const cip_options* o) { return o ? (size_t)o->struct_size : 0; }
-
 int check(cip_handle h) {
   if (!h) {
     set_error("null handle");
@@ -288,6 +286,12 @@ int form_H(cip_engine* h) {
   }
   cudaStream_t s = h->stream;
   CIP_CUDA(cudaEventRecord(h->ev[0], s));
+  if (h->rs.on) {
+    CIP_TRY(structure_form_H(h));
+    if (h->opt.reg_delta != 0.0) CIP_TRY(add_diag_q4(h->H4, h->n_pad, 0, h->n, h->opt.reg_delta, 0, s));
+    CIP_CUDA(cudaEventRecord(h->ev[3], s));
+    return 0;
+  }
   if (h->m_pad > 0 && !h->fold) CIP_TRY(cone_scale_panel(h->cd, h->Fi, h->At4, h->Atil4, h->n_pad, h->m_pad, h->n, s));
   CIP_CUDA(cudaEventRecord(h->ev[1], s));
   const double* cin = (h->rank == 0) ? h->Qq4 : nullptr;
@@ -447,6 +451,21 @@ int engine_setup_comm(cip_engine* h) {
   return 0;
 }
 const char* last_error_string() { return g_err; }
+int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold) {
+  // fold the scaling into the SYRK (no Atil4) for pure R-cone rows: on request, or when the second copy of A would
+  // not fit next to what is still to be allocated (Q, H, workspaces: ~ 3 n_pad^2 + 2.2 GB)
+  int mode = can ? h->opt.fold_scaling : 2;
+  if (const char* env = getenv("CIP_FOLD_SCALING")) { if (can) mode = atoi(env); }
+  if (mode == 0) {
+    size_t free_b = 0, total_b = 0;
+    CIP_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    const size_t nn = (size_t)h->n_pad * h->n_pad;
+    const size_t need = mn * 8 + 3 * nn * 8 + (size_t)GEMM_WS_DOUBLES * 8 + (size_t(1) << 30);
+    mode = (free_b < need) ? 1 : 2;
+  }
+  *fold = (mode == 1);
+  return 0;
+}
 }  // namespace cip
 
 // =================================================================== C ABI
@@ -494,19 +513,19 @@ int upload_csc(cip_engine* h, double* dst, int ld, const cip_csc* M, int transpo
 
 int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,
                 const double* G, int ldg, const cip_csc* Qs, const cip_csc* As, const cip_csc* Gs, int ncones,
-                const int* cone_type, const int* cone_dim, const cip_options* opts);
+                const int* cone_type, const int* cone_dim, const cip_options* opts, bool shard);
 
 // allocates the handle, builds it, and releases everything again if any step fails
 int create_impl(cip_handle* out, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,
                 const double* G, int ldg, const cip_csc* Qs, const cip_csc* As, const cip_csc* Gs, int ncones,
-                const int* cone_type, const int* cone_dim, const cip_options* opts) {
+                const int* cone_type, const int* cone_dim, const cip_options* opts, bool shard = false) {
   if (out) *out = nullptr;
   if (!out || n <= 0 || m < 0 || p < 0 || ncones < 0 || (ncones > 0 && (!cone_type || !cone_dim))) {
     set_error("cip_create: bad dimensions n=%d m=%d p=%d ncones=%d", n, m, p, ncones);
     return -1;
   }
   cip_engine* h = new cip_engine();
-  const int rc = create_body(h, n, m, p, Q, ldq, A, lda, G, ldg, Qs, As, Gs, ncones, cone_type, cone_dim, opts);
+  const int rc = create_body(h, n, m, p, Q, ldq, A, lda, G, ldg, Qs, As, Gs, ncones, cone_type, cone_dim, opts, shard);
   if (rc != 0) {
     cip_destroy(h);            // every member is null-checked there
     return rc;
@@ -517,11 +536,21 @@ int create_impl(cip_handle* out, int n, int m, int p, const double* Q, int ldq, 
 
 int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,
                 const double* G, int ldg, const cip_csc* Qs, const cip_csc* As, const cip_csc* Gs, int ncones,
-                const int* cone_type, const int* cone_dim, const cip_options* opts) {
+                const int* cone_type, const int* cone_dim, const cip_options* opts, bool shard) {
   h->opt.dist_chol = -1;
   h->opt.aug_rho = -1.0;
   if (opts) memcpy(&h->opt, opts, std::min<size_t>(sizeof(cip_options), (size_t)opts->struct_size));
   else h->opt.device = -1;
+  {
+    // (0 when the caller's struct does not reach the field: h->opt starts zeroed)
+    int rs = h->opt.row_structure;
+    if (const char* env = getenv("CIP_ROW_STRUCTURE")) { if (!shard) rs = atoi(env); }
+    if (rs != 0 && rs != 1) {
+      set_error("cip_create: row_structure must be 0 or 1 (got %d)", rs);
+      return -1;
+    }
+    h->rs.on = (rs == 1) && m > 0;     // no rows: nothing to classify
+  }
   if (h->opt.device < 0) CIP_CUDA(cudaGetDevice(&h->device));
   else h->device = h->opt.device;
   CIP_CUDA(cudaSetDevice(h->device));
@@ -630,7 +659,7 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   // ---- matrices
   const size_t nn = (size_t)h->n_pad * h->n_pad;
   const size_t mn = (size_t)h->m_pad * h->n_pad;
-  CIP_TRY(dev_alloc(h, &h->At4, mn));
+  if (!(h->rs.on && As)) CIP_TRY(dev_alloc(h, &h->At4, mn));     // CSC input with row structure: never dense
   // augmentation rows (H + rho G'G keeps the Cholesky valid when H is singular on range(G'), as kktsolver_qr allows)
   {
     double rho = h->opt.aug_rho;
@@ -638,22 +667,9 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
     h->aug_rho = (p > 0) ? rho : 0.0;
     h->aug_rows = (h->aug_rho > 0) ? round_up(p, 32) : 0;
   }
-  {
-    // fold the scaling into the SYRK (no Atil4) for pure R-cone problems: on request, or when the second copy of
-    // A would not fit next to what is still to be allocated (Q, H, workspaces: ~ 3 n_pad^2 + 2.2 GB)
-    const bool can = slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0;
-    const bool has_field = opts_size(opts) >= offsetof(cip_options, fold_scaling) + sizeof(int);
-    int mode = !can ? 2 : (has_field ? h->opt.fold_scaling : 0);
-    if (const char* env = getenv("CIP_FOLD_SCALING")) { if (can) mode = atoi(env); }
-    if (mode == 0) {
-      size_t free_b = 0, total_b = 0;
-      CIP_CUDA(cudaMemGetInfo(&free_b, &total_b));
-      const size_t need = mn * 8 + 3 * nn * 8 + (size_t)GEMM_WS_DOUBLES * 8 + (size_t(1) << 30);
-      mode = (free_b < need) ? 1 : 2;
-    }
-    h->fold = (mode == 1);
-  }
-  if (!h->fold) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
+  // (h->opt.fold_scaling is 0 when the caller's struct does not reach the field: h->opt starts zeroed)
+  if (!h->rs.on) CIP_TRY(engine_decide_fold(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0, mn, &h->fold));
+  if (!h->fold && !h->rs.on) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
   CIP_TRY(dev_alloc(h, &h->Qq4, nn));
   CIP_TRY(dev_alloc(h, &h->H4, nn));
   CIP_TRY(dev_alloc(h, &h->gemm_ws, (size_t)GEMM_WS_DOUBLES));
@@ -698,7 +714,9 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   // A (transposed into Q4: rows = columns of A)
   if (m > 0) {
     if (!A && !As) { set_error("A is null"); return -1; }
-    if (As) {
+    if (As && h->rs.on) {
+      CIP_TRY(structure_build_csc(h, As));
+    } else if (As) {
       CIP_TRY(upload_csc(h, h->At4, h->n_pad, As, 1));
     } else if (kernel_readable(A, h->device)) {
       CIP_TRY(pack_trans_q4(h->At4, h->n_pad, 0, A, lda, m, h->m_pad, n, s));
@@ -715,10 +733,15 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
       }
       cudaFree(stg);
     }
+    if (h->rs.on && !As) CIP_TRY(structure_build_dense(h));
   }
-  if (h->fold) CIP_TRY(make_q4_tensor_map(&h->mapAt.map, h->At4, h->n_pad, h->m_pad / 4));
-  else if (h->m_pad + h->aug_rows > 0)
+  if (h->rs.on) {
+    // (structure_finish makes the operand map of the rest rows)
+  } else if (h->fold) {
+    CIP_TRY(make_q4_tensor_map(&h->mapAt.map, h->At4, h->n_pad, h->m_pad / 4));
+  } else if (h->m_pad + h->aug_rows > 0) {
     CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (h->m_pad + h->aug_rows) / 4));
+  }
   CIP_TRY(chol_make_plan(&h->cholH, h->H4, h->n_pad, h->Winv, h->info));
 
   // G
@@ -746,13 +769,14 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
       CIP_CUDA(cudaStreamSynchronize(s));
       if (stg) cudaFree(stg);
     }
-    if (h->aug_rows > 0)
+    if (h->aug_rows > 0 && !h->rs.on)
       CIP_TRY(transpose_scale_q4(h->Atil4, h->n_pad, h->m_pad, h->G4, h->p_pad, p, n, sqrt(h->aug_rho), s));
     CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, p, h->p_pad, 1.0, 1, s));
     if (h->opt.reg_eps_G != 0.0) CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, 0, p, h->opt.reg_eps_G, 1, s));
     CIP_TRY(make_q4_tensor_map(&h->mapZ.map, h->Z4, h->p_pad, h->n_pad / 4));
     CIP_TRY(chol_make_plan(&h->cholS, h->S4, h->p_pad, h->WinvS, h->info + 1));
   }
+  if (h->rs.on) CIP_TRY(structure_finish(h));
 
   // ---- work vectors
   for (auto& v : h->nv) CIP_TRY(dev_alloc(h, &v, h->n_pad + 4));
@@ -772,7 +796,8 @@ namespace cip {
 int engine_create_single(cip_handle* out, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,
                          const double* G, int ldg, const cip_csc* Qs, const cip_csc* As, const cip_csc* Gs,
                          int ncones, const int* cone_type, const int* cone_dim, const cip_options* opts) {
-  return create_impl(out, n, m, p, Q, ldq, A, lda, G, ldg, Qs, As, Gs, ncones, cone_type, cone_dim, opts);
+  return create_impl(out, n, m, p, Q, ldq, A, lda, G, ldg, Qs, As, Gs, ncones, cone_type, cone_dim, opts,
+                     /*shard=*/true);
 }
 }  // namespace cip
 
@@ -780,6 +805,15 @@ namespace {
 // opts.ngpus > 1 (and the field is inside the caller's struct): single-process multi-GPU handle
 bool wants_multi(const cip_options* opts) {
   return opts && (size_t)opts->struct_size >= offsetof(cip_options, ngpus) + sizeof(int) && opts->ngpus > 1;
+}
+// a sharded handle with opts.row_structure = 1: refused before any device work
+bool reject_sharded_structure(const cip_options* opts) {
+  if (opts && (size_t)opts->struct_size >= offsetof(cip_options, row_structure) + sizeof(int) &&
+      opts->row_structure != 0) {
+    set_error("row_structure is supported on single-device handles only (ngpus = %d)", opts->ngpus);
+    return true;
+  }
+  return false;
 }
 }  // namespace
 
@@ -793,6 +827,7 @@ int cip_create(cip_handle* out, int n, int m, int p, const double* Q, int ldq, c
       set_error("cip_create: bad dimensions n=%d m=%d p=%d ncones=%d", n, m, p, ncones);
       return -1;
     }
+    if (reject_sharded_structure(opts)) return -1;
     return multi_create(out, n, m, p, Q, ldq, A, lda, G, ldg, nullptr, nullptr, nullptr, ncones, cone_type,
                         cone_dim, opts);
   }
@@ -819,6 +854,7 @@ int cip_create_csc(cip_handle* out, int n, const cip_csc* Q, const cip_csc* A, c
       set_error("cip_create_csc: bad arguments");
       return -1;
     }
+    if (reject_sharded_structure(&o)) return -1;
     return multi_create(out, n, A->nrows, p, nullptr, 0, nullptr, 0, nullptr, 0, Q, A, (p > 0) ? G : nullptr, ncones,
                         cone_type, cone_dim, &o);
   }
@@ -839,6 +875,7 @@ int cip_destroy(cip_handle h) {
                   h->d_type, h->d_off, h->d_rowcone, h->d_qlist, h->d_slist, h->F.kind, h->F.a, h->F.b, h->F.D,
                   h->Fi.kind, h->Fi.a, h->Fi.b, h->Fi.D, h->partial, h->scalar, h->F.R, h->F.Ri, h->d_sord, h->d_roff, h->gemm_ws};
   for (void* p : ptrs) if (p) cudaFree(p);
+  for (void* p : h->owned) cudaFree(p);
   for (auto v : h->nv) if (v) cudaFree(v);
   for (auto v : h->mv) if (v) cudaFree(v);
   for (auto v : h->pv) if (v) cudaFree(v);
@@ -876,6 +913,7 @@ int cip_comm_init(cip_handle h, int nranks, int rank, const unsigned char id[128
   CIP_TRY(check(h));
   if (h->multi) { set_error("cip_comm_init: a single-process multi-GPU handle (opts.ngpus) owns its communicators"); return -1; }
   if (nranks <= 1) return 0;
+  if (h->rs.on) { set_error("cip_comm_init: row_structure is supported on single-device handles only"); return -1; }
   const NcclApi* api = nccl_api();
   if (!api) return -1;
   NcclId nid;
@@ -1043,7 +1081,9 @@ int cip_solve(cip_handle h, const double* ry, const double* rw, const double* rv
   //  what the 3x3 system requires -- the reference's pivot is only right for symmetric F, SURVEY 3b)
   CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, rvp, h->mv[2], nullptr, h->mv[1], s));
   // rhs = y + A' t1                                      (:327); single GPU: y is added in the mat-vec's second pass
-  if (h->m && !h->comm) {
+  if (h->rs.on) {
+    CIP_TRY(structure_AT(h, h->nv[2], h->mv[2], ryp, 0));
+  } else if (h->m && !h->comm) {
     CIP_TRY(q4_mv_rows(h->nv[2], h->At4, h->n_pad, h->n, h->m, h->mv[2], h->partial, h->partial_cap, s, ryp));
   } else {
     if (h->m) CIP_TRY(q4_mv_rows(h->nv[1], h->At4, h->n_pad, h->n, h->m, h->mv[2], h->partial, h->partial_cap, s));
@@ -1068,7 +1108,8 @@ int cip_solve(cip_handle h, const double* ry, const double* rw, const double* rv
   CIP_TRY(chol_bwd(h->cholH, h->nv[3], h->nv[5], s));
   // dv = t1 - F^-T F^-T (A dy)                           (:328)
   if (h->m) {
-    CIP_TRY(q4_mv_k(h->mv[3], h->At4, h->n_pad, h->n, h->m, h->nv[5], s));
+    if (h->rs.on) CIP_TRY(structure_A(h, h->mv[3], h->nv[5], 0));
+    else CIP_TRY(q4_mv_k(h->mv[3], h->At4, h->n_pad, h->n, h->m, h->nv[5], s));
     CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, h->mv[3], dvp, h->mv[2], h->mv[1], s));   // t1 - (F'F)^-1 (A dy)
   }
   CIP_CUDA(cudaEventRecord(h->ev[7], s));
@@ -1132,7 +1173,9 @@ int cip_solve_multi(cip_handle h, int nrhs, const double* ry, int ldy, const dou
       CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, rvp[b], mv[2], nullptr, mv[1], s));          // t1 (:326)
     }
     // rhs = y + A' t1 (:327) for both columns in one pass over A
-    if (h->m && !h->comm) {
+    if (h->rs.on) {
+      CIP_TRY(structure_AT2(h, h->nv[2], h->nv2[2], h->mv[2], h->mv2[2], ryp[0], ryp[1]));
+    } else if (h->m && !h->comm) {
       CIP_TRY(q4_mv_rows2(h->nv[2], h->nv2[2], h->At4, h->n_pad, h->n, h->m, h->mv[2], h->mv2[2], h->partial,
                           h->partial_cap, s, ryp[0], ryp[1]));
     } else {
@@ -1167,7 +1210,8 @@ int cip_solve_multi(cip_handle h, int nrhs, const double* ry, int ldy, const dou
     }
     // dv = t1 - F^-T F^-T (A dy) (:328): A dy for both columns in one pass over A
     if (h->m) {
-      CIP_TRY(q4_mv_k2(h->mv[3], h->mv2[3], h->At4, h->n_pad, h->n, h->m, h->nv[5], h->nv2[5], s));
+      if (h->rs.on) CIP_TRY(structure_A2(h, h->mv[3], h->mv2[3], h->nv[5], h->nv2[5]));
+      else CIP_TRY(q4_mv_k2(h->mv[3], h->mv2[3], h->At4, h->n_pad, h->n, h->m, h->nv[5], h->nv2[5], s));
       for (int b = 0; b < 2; ++b)
         CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, MVs[b][3], dvp[b], MVs[b][2], MVs[b][1], s));
     }
@@ -1218,13 +1262,15 @@ int cip_mul_A(cip_handle h, int trans, const double* x, double* y) {
     const double* xp;
     CIP_TRY(vec_in(h, h->nv[6], x, h->n, &xp));
     double* yp = vec_out(h, h->mv[6], y, h->m);
-    CIP_TRY(q4_mv_k(yp, h->At4, h->n_pad, h->n, h->m, xp, s));
+    if (h->rs.on) CIP_TRY(structure_A(h, yp, xp, 0));
+    else CIP_TRY(q4_mv_k(yp, h->At4, h->n_pad, h->n, h->m, xp, s));
     CIP_TRY(vec_out_done(h, y, yp, h->m));
   } else {
     const double* xp;
     CIP_TRY(vec_in(h, h->mv[6], x, h->m, &xp, /*padded=*/true));
     double* yp = vec_out(h, h->nv[6], y, h->n);
-    if (h->m) CIP_TRY(q4_mv_rows(yp, h->At4, h->n_pad, h->n, h->m, xp, h->partial, h->partial_cap, s));
+    if (h->rs.on) CIP_TRY(structure_AT(h, yp, xp, nullptr, 0));
+    else if (h->m) CIP_TRY(q4_mv_rows(yp, h->At4, h->n_pad, h->n, h->m, xp, h->partial, h->partial_cap, s));
     else CIP_TRY(fill_zero(yp, h->n, s));
     CIP_TRY(allreduce(h, yp, h->n));
     CIP_TRY(vec_out_done(h, y, yp, h->n));
@@ -1277,6 +1323,28 @@ int cip_stats(cip_handle h, cip_stats_t* out) {
   h->st.device_bytes = h->bytes;
   h->st.kernel_launches = cip::g_launches;
   *out = h->st;
+  return 0;
+}
+
+int cip_structure_info(cip_handle h, cip_structure_t* out) {
+  CIP_TRY(check(h));
+  if (!out || out->struct_size < (int)sizeof(int)) {
+    set_error("cip_structure_info: out->struct_size must be set");
+    return -1;
+  }
+  cip_structure_t r{};
+  r.struct_size = out->struct_size;
+  const RowStructure& rs = h->rs;      // (a multi-GPU front never has it on)
+  if (rs.on) {
+    r.enabled = 1;
+    r.singleton_rows = rs.nsing;
+    r.empty_rows = rs.nempty;
+    r.rest_rows = rs.nr;
+    r.rest_cols = rs.nJ;
+    r.compressed = rs.compressed;
+    r.base_has_gtg = rs.base_has_gtg;
+  }
+  memcpy(out, &r, std::min<size_t>(sizeof(r), (size_t)out->struct_size));
   return 0;
 }
 

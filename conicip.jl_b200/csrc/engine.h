@@ -10,7 +10,32 @@ constexpr int NV = 8;   // n-length work vectors
 constexpr int MV = 10;  // m-length work vectors
 constexpr int PV = 6;   // p-length work vectors
 
-namespace cip { struct Multi; }
+namespace cip {
+struct Multi;
+
+// cip_options.row_structure (structure.cu).  The rows of A split into singletons (R rows with one non-zero, sorted
+// by (column, row) behind a column pointer), empty R rows, and the rest (every Q / S row and the R rows with >= 2
+// non-zeros, ascending), which keep a compact Q4 copy At4r (ld = nJ_pad, k = rest rows) over the column support J.
+struct RowStructure {
+  bool on = false;
+  int nsing = 0, nempty = 0, nr = 0, nr_pad = 0, nJ = 0, nJ_pad = 0;
+  bool compressed = false, base_has_gtg = false, fold = false;
+  double *At4r = nullptr, *Atil4r = nullptr, *Hr4 = nullptr;   // Hr4: nJ_pad^2 Gram scratch (compressed only)
+  double* Base4 = nullptr;          // Q + rho G'G (owned when base_has_gtg, else an alias of Qq4)
+  GemmOperand map{};                // over Atil4r, or over At4r when folded
+  int *rest_row = nullptr, *J = nullptr, *Jinv = nullptr;      // [nr], [nJ], [n] (-1: column outside J)
+  int* row_code = nullptr;          // [m]: >= 0 rest index, -1 - s singleton s, INT_MIN empty
+  int *sing_ptr = nullptr, *sing_row = nullptr, *sing_col = nullptr;   // [n+1], [nsing], [nsing]
+  double* sing_val = nullptr;       // [nsing]
+  // cone descriptor of the rest rows: whole Q / S cones and the rest rows of each R cone, in global order
+  ConeDesc cd{};
+  int *d_type = nullptr, *d_off = nullptr, *d_rowcone = nullptr, *d_qlist = nullptr, *d_slist = nullptr;
+  int* cone_map = nullptr;          // [cones of cd] -> global cone
+  Scaling Fi{};                     // Fi gathered into rest order (R / Ri shared with the handle's)
+  // work vectors of the mat-vecs, two sets (cip_solve_multi pairs): x[rest], y[J], products
+  double *xr[2] = {}, *yJ[2] = {}, *outr[2] = {}, *outJ[2] = {};
+};
+}  // namespace cip
 
 struct cip_engine {
   // single-process multi-GPU: a handle created with opts.ngpus > 1 is only a front for `multi` (one shard
@@ -44,6 +69,8 @@ struct cip_engine {
   cip::GemmOperand mapAt{};
   int aug_rows = 0;        // rows of Atil4 beyond m_pad holding sqrt(aug_rho) * G
   double aug_rho = 0.0;
+  cip::RowStructure rs;    // opts.row_structure: At4 / Atil4 are not allocated
+  std::vector<void*> owned;   // further device buffers freed by cip_destroy
   // work vectors
   double* nv[NV] = {};
   double* mv[MV] = {};
@@ -80,8 +107,28 @@ int engine_create_single(cip_handle* out, int n, int m, int p, const double* Q, 
                          const double* G, int ldg, const cip_csc* Qs, const cip_csc* As, const cip_csc* Gs,
                          int ncones, const int* cone_type, const int* cone_dim, const cip_options* opts);
 const char* last_error_string();
+// fold the scaling into the SYRK? (opts.fold_scaling / CIP_FOLD_SCALING, else free memory against the mn-double
+// second copy); `can`: every row of the SYRK is an R row
+int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold);
 // buffers / streams of the overlapped Gram reduction, once the communicator exists (engine.cu)
 int engine_setup_comm(cip_engine* h);
+
+// ---- row structure (structure.cu)
+// LEVEL 1, dense input: classify the rows of the packed At4, build the compact arrays, free At4
+int structure_build_dense(cip_engine* h);
+// LEVEL 1, CSC input: classify from the CSC arrays and scatter only the rest rows (no dense At4)
+int structure_build_csc(cip_engine* h, const cip_csc* A);
+// LEVEL 1, after G4: Base4 = Q + rho G'G (or an alias of Qq4), the tensor map of the SYRK operand
+int structure_finish(cip_engine* h);
+// LEVEL 2: H4 = Base4 + Atil_r'Atil_r (scattered at J x J) + the singleton diagonal; records ev[1], ev[2]
+int structure_form_H(cip_engine* h);
+// out[n] = add + A' x  (x: m-vector readable up to m); b selects the work vector set
+int structure_AT(cip_engine* h, double* out, const double* x, const double* add, int b);
+int structure_AT2(cip_engine* h, double* outa, double* outb, const double* xa, const double* xb, const double* adda,
+                  const double* addb);
+// out[m] = A y  (y: n-vector)
+int structure_A(cip_engine* h, double* out, const double* y, int b);
+int structure_A2(cip_engine* h, double* outa, double* outb, const double* ya, const double* yb);
 
 // ---- single-process multi-GPU front (multi.cu): same contracts as the C ABI entry points, global vectors
 int multi_create(cip_handle* out, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,

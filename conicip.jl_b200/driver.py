@@ -63,12 +63,14 @@ class LocalReducer:
         return list(xs)
 
 
-def conicIP_native(Q, c, A, b, cone_dims, G=None, d=None, *, engine=None, ngpus=1, **opts):
+def conicIP_native(Q, c, A, b, cone_dims, G=None, d=None, *, engine=None, ngpus=1, row_structure=0, **opts):
     """Same problem statement and options as `conicIP`, but the loop itself runs inside the library
     (`cip_ipm_solve`, SURVEY 8f rank 1): one C call per solve.  Pass `engine=` to reuse a handle;
-    `ngpus > 1` row-shards A over that many devices of this process (`cip_options.ngpus`)."""
+    `ngpus > 1` row-shards A over that many devices of this process (`cip_options.ngpus`);
+    `row_structure=1` exploits the row structure of A when forming H (`cip_options.row_structure`)."""
     from .engine import Engine
-    eng = engine or Engine(Q, A, G if (G is not None and G.shape[0]) else None, cone_dims, ngpus=ngpus)
+    eng = engine or Engine(Q, A, G if (G is not None and G.shape[0]) else None, cone_dims, ngpus=ngpus,
+                           row_structure=row_structure)
     y, w, v, info = eng.ipm_solve(np.asarray(c, dtype=np.float64), np.asarray(b, dtype=np.float64),
                                   None if d is None else np.asarray(d, dtype=np.float64), **opts)
     sol = Solution(np.asarray(y), np.asarray(w), np.asarray(v), status=info["status"], Iter=info["Iter"],

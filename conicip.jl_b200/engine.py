@@ -36,7 +36,7 @@ class Engine:
     """LEVEL-1 object: `kktsolver(Q, A, G, cone_dims)` (src/ConicIP.jl:667)."""
 
     def __init__(self, Q, A, G, cone_dims, *, reg_delta=0.0, reg_eps_G=0.0, device=-1,
-                 use_torch_stream=True, dist_chol=-1, aug_rho=-1.0, ngpus=1, fold_scaling=0):
+                 use_torch_stream=True, dist_chol=-1, aug_rho=-1.0, ngpus=1, fold_scaling=0, row_structure=0):
         L = lib()
         self.cone_dims = [(t, int(k)) for t, k in cone_dims]
         self.cone_type = np.array([CONE_CODE[t] for t, _ in self.cone_dims], dtype=np.int32)
@@ -54,6 +54,7 @@ class Engine:
         opts.aug_rho = aug_rho
         opts.ngpus = int(ngpus)            # > 1: single-process multi-GPU handle (global vectors in and out)
         opts.fold_scaling = int(fold_scaling)   # 0 auto, 1 always, 2 never (R-only problems: no Atil copy of A)
+        opts.row_structure = int(row_structure)  # 1: singleton R rows on the diagonal, compact SYRK for the rest
         self.ngpus = max(1, int(ngpus))
         self._torch = None
         self._use_torch_stream = use_torch_stream
@@ -405,6 +406,14 @@ class Engine:
         st = Stats()
         check(lib().cip_stats(self._h, C.byref(st)))
         return {k: getattr(st, k) for k, _ in Stats._fields_}
+
+    def structure_info(self):
+        """How `row_structure=1` split the rows of A (`cip_structure_info`); all zero when the option is off."""
+        from ._lib import StructureInfo
+        si = StructureInfo()
+        si.struct_size = C.sizeof(StructureInfo)
+        check(lib().cip_structure_info(self._h, C.byref(si)))
+        return {k: getattr(si, k) for k, _ in StructureInfo._fields_ if k != "struct_size"}
 
     def get_H(self):
         out = np.zeros((self.n, self.n), order="F")

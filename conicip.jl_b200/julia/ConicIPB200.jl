@@ -32,10 +32,11 @@ struct Options            # mirrors cip_options
     aug_rho::Cdouble
     ngpus::Cint           # > 1: this one process drives that many GPUs behind the handle (rows of A sliced on cone boundaries)
     fold_scaling::Cint    # 0 auto, 1 always, 2 never: R-only problems without a second (scaled) copy of A
+    row_structure::Cint   # 1: singleton R rows go onto the diagonal of H, the SYRK runs on the other rows (one GPU)
 end
-make_options(; device = -1, reg_delta = 0.0, q_kind = 0, ngpus = 1, fold_scaling = 0) =
+make_options(; device = -1, reg_delta = 0.0, q_kind = 0, ngpus = 1, fold_scaling = 0, row_structure = 0) =
     Options(Cint(sizeof(Options)), Cint(device), reg_delta, 0.0, Cint(q_kind), Cint(0), Cint(-1), -1.0, Cint(ngpus),
-            Cint(fold_scaling))
+            Cint(fold_scaling), Cint(row_structure))
 
 lasterr() = unsafe_string(ccall((:cip_last_error, LIB), Cstring, ()))
 function check(rc::Cint)
@@ -56,13 +57,13 @@ Csc(M::SparseMatrixCSC{Float64,Int64}) = Csc(size(M, 1), size(M, 2), pointer(M.c
 mutable struct Engine
     h::Ptr{Cvoid}
     n::Int; m::Int; p::Int
-    function Engine(Q, A, G, cone_dims; reg_delta = 0.0, ngpus = 1, device = -1, fold_scaling = 0)
+    function Engine(Q, A, G, cone_dims; reg_delta = 0.0, ngpus = 1, device = -1, fold_scaling = 0, row_structure = 0)
         n = size(Q, 1); m = size(A, 1); p = size(G, 1)
         if A isa SparseMatrixCSC          # sparse LEVEL 1: no dense copy on the host (cip_create_csc)
             Qs = SparseMatrixCSC{Float64,Int64}(sparse(Q)); As = SparseMatrixCSC{Float64,Int64}(A)
             Gs = SparseMatrixCSC{Float64,Int64}(sparse(G))
             ct = Cint[CONE_CODE[t] for (t, _) in cone_dims]; cdim = Cint[k for (_, k) in cone_dims]
-            opts = Ref(make_options(; device, reg_delta, q_kind = 2, ngpus, fold_scaling))
+            opts = Ref(make_options(; device, reg_delta, q_kind = 2, ngpus, fold_scaling, row_structure))
             hp = Ref{Ptr{Cvoid}}(C_NULL)
             GC.@preserve Qs As Gs begin
                 rc = ccall((:cip_create_csc, LIB), Cint,
@@ -81,7 +82,7 @@ mutable struct Engine
         Gd = Matrix{Float64}(G)
         ct = Cint[CONE_CODE[t] for (t, _) in cone_dims]
         cdim = Cint[k for (_, k) in cone_dims]
-        opts = Ref(make_options(; device, reg_delta, q_kind = qk, ngpus, fold_scaling))
+        opts = Ref(make_options(; device, reg_delta, q_kind = qk, ngpus, fold_scaling, row_structure))
         hp = Ref{Ptr{Cvoid}}(C_NULL)
         rc = ccall((:cip_create, LIB), Cint,
                    (Ref{Ptr{Cvoid}}, Cint, Cint, Cint, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Cint,
@@ -172,6 +173,27 @@ function solve_multi(eng, Y::Matrix{Float64}, W::Matrix{Float64}, V::Matrix{Floa
                 (Ptr{Cvoid}, Cint, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Ptr{Cdouble}, Ptr{Cdouble}),
                 eng.h, k, Y, eng.n, W, max(eng.p, 1), V, eng.m, A, B, C))
     return (A, B, C)
+end
+
+struct StructureInfo      # mirrors cip_structure_t
+    struct_size::Cint
+    enabled::Cint
+    singleton_rows::Cint
+    empty_rows::Cint
+    rest_rows::Cint
+    rest_cols::Cint
+    compressed::Cint
+    base_has_gtg::Cint
+end
+"""
+    structure_info(eng) -> StructureInfo
+
+How an engine created with `row_structure = 1` split the rows of `A` (`cip_structure_info`).
+"""
+function structure_info(eng::Engine)
+    r = Ref(StructureInfo(Cint(sizeof(StructureInfo)), 0, 0, 0, 0, 0, 0, 0))
+    check(ccall((:cip_structure_info, LIB), Cint, (Ptr{Cvoid}, Ref{StructureInfo}), eng.h, r))
+    return r[]
 end
 """
     kktsolver_b200(; ngpus = 8, ...) -> kktsolver

@@ -70,6 +70,13 @@ typedef struct cip_options {
                            SYRK instead of materialising Atil = F^-T A (src/kktsolvers.jl:33) -- halves the resident
                            bytes (no second copy of A), costs ~1.5 % of the SYRK.  0: auto (fold when the second copy
                            would not fit in free device memory), 1: always, 2: never */
+  int    row_structure; /* single-device handles: 1 = classify the rows of A at LEVEL 1 and exploit them when forming
+                           H (the reference keeps A sparse through this product, src/kktsolvers.jl:289-290).  R rows
+                           with one non-zero go straight onto the diagonal of H; the other rows ("rest": every Q / S
+                           row and the R rows with >= 2 non-zeros) are kept in a compact copy of A that spans only
+                           the columns they touch, and the constant Q + rho*G'G is formed once.  0 = off (default).
+                           The environment variable CIP_ROW_STRUCTURE=1 turns it on for single-device handles.
+                           Sharded handles (ngpus > 1, cip_comm_init) reject it. */
 } cip_options;
 
 typedef struct cip_stats_t {
@@ -222,6 +229,18 @@ int cip_ipm_solve(cip_handle h, const double* c, const double* b, const double* 
 
 /* ---------------------------------------------------------------- introspection */
 int cip_stats(cip_handle h, cip_stats_t* out);
+/* How a handle with cip_options.row_structure = 1 split the rows of A (all zero when the option is off). */
+typedef struct cip_structure_t {
+  int struct_size;      /* = sizeof(cip_structure_t), set by the caller                                */
+  int enabled;          /* 1: the structured path runs                                                  */
+  int singleton_rows;   /* R rows with exactly one non-zero: added to the diagonal of H                 */
+  int empty_rows;       /* R rows without a non-zero                                                    */
+  int rest_rows;        /* Q / S rows plus R rows with >= 2 non-zeros: the rows of the SYRK             */
+  int rest_cols;        /* |J|: the columns the rest rows touch                                         */
+  int compressed;       /* 1: the SYRK runs on the columns J only (round_up(|J|,128) <= n_pad/2)       */
+  int base_has_gtg;     /* 1: the constant part Q + rho*G'G was formed once at creation                 */
+} cip_structure_t;
+int cip_structure_info(cip_handle h, cip_structure_t* out);
 /* copy the current reduced matrix H (after cip_factor: its Cholesky factor L in the
  * lower triangle) into a column-major n*n buffer -- test/debug hook */
 int cip_get_H(cip_handle h, double* out, int ldo);
