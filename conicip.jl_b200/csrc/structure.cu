@@ -10,6 +10,8 @@
 //               kept as a compact Q4 matrix At4r (k = rest rows) over the columns J they touch
 // and the constant Q + rho G'G is formed once.  LEVEL 2 then runs the SYRK on the rest only (on J x J when J is
 // at most half the columns), scatters it onto the constant part and adds the singletons to the diagonal.
+// J can be empty while the rest has rows (a Q or S cone whose rows of A are all zero): those rows add nothing to
+// H, A y or A'x, so the operand map, the SYRK, the scatter and the rest mat-vecs are skipped.
 // A non-zero is a stored value != 0.0, for dense and CSC input alike.
 #include <climits>
 #include <math.h>
@@ -160,14 +162,14 @@ __global__ void finish_at_kernel(double* __restrict__ out, const double* __restr
   out[j] = add ? add[j] + r : r;
 }
 
-// out[i] = (At4r y_J)[rest index] on rest rows, a_ij y_j on singletons, 0 on empty rows
+// out[i] = (At4r y_J)[rest index] on rest rows (0 without outr: J is empty), a_ij y_j on singletons, 0 on empty rows
 __global__ void finish_a_kernel(double* __restrict__ out, const double* __restrict__ outr,
                                 const int* __restrict__ code, const int* __restrict__ scol,
                                 const double* __restrict__ sval, const double* __restrict__ y, int m) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= m) return;
   const int c = code[i];
-  out[i] = c >= 0 ? outr[c] : (c == EMPTY_ROW ? 0.0 : sval[-1 - c] * y[scol[-1 - c]]);
+  out[i] = c >= 0 ? (outr ? outr[c] : 0.0) : (c == EMPTY_ROW ? 0.0 : sval[-1 - c] * y[scol[-1 - c]]);
 }
 
 inline unsigned nb(long long n, int per) { return (unsigned)std::max<long long>(1, (n + per - 1) / per); }
@@ -491,7 +493,7 @@ int structure_finish(cip_engine* h) {
   } else {
     rs.Base4 = h->Qq4;
   }
-  if (rs.nr > 0) {
+  if (rs.nJ > 0) {
     if (rs.fold) CIP_TRY(make_q4_tensor_map(&rs.map.map, rs.At4r, rs.nJ_pad, rs.nr_pad / 4));
     else CIP_TRY(make_q4_tensor_map(&rs.map.map, rs.Atil4r, rs.nJ_pad, rs.nr_pad / 4));
   }
@@ -503,14 +505,14 @@ int structure_form_H(cip_engine* h) {
   cudaStream_t s = h->stream;
   const size_t nn = (size_t)h->n_pad * h->n_pad;
   const int ncr = rs.cd.ncones;
-  if (rs.nr > 0) {
+  if (rs.nJ > 0) {
     gather_scaling_kernel<<<nb(std::max(rs.nr, ncr), 256), 256, 0, s>>>(h->Fi, rs.Fi, rs.rest_row, rs.nr,
                                                                        rs.cone_map, ncr);
     CIP_CHECK_LAUNCH();
     if (!rs.fold) CIP_TRY(cone_scale_panel(rs.cd, rs.Fi, rs.At4r, rs.Atil4r, rs.nJ_pad, rs.nr_pad, rs.nJ, s));
   }
   CIP_CUDA(cudaEventRecord(h->ev[1], s));
-  if (rs.nr > 0) {
+  if (rs.nJ > 0) {
     GemmArgs a{};
     a.lower = 1; a.ntm = a.ntn = rs.nJ_pad / TILE; a.sym = 1; a.nk = rs.nr_pad / 32;
     a.Cin = rs.compressed ? nullptr : rs.Base4;
@@ -520,8 +522,8 @@ int structure_form_H(cip_engine* h) {
     if (rs.fold) a.kscale = rs.Fi.a;
     CIP_TRY(launch_gemm_nt(rs.map, rs.map, a, s));
   }
-  if (rs.nr == 0 || rs.compressed) CIP_TRY(vec_copy(h->H4, rs.Base4, nn, s));
-  if (rs.compressed) {
+  if (rs.nJ == 0 || rs.compressed) CIP_TRY(vec_copy(h->H4, rs.Base4, nn, s));
+  if (rs.nJ > 0 && rs.compressed) {
     dim3 grid(nb(rs.nJ, 128), (unsigned)std::min(rs.nJ, 65535));
     scatter_gram_kernel<<<grid, 128, 0, s>>>(h->H4, h->n_pad, rs.Hr4, rs.nJ_pad, rs.J, rs.nJ);
     CIP_CHECK_LAUNCH();
@@ -539,12 +541,12 @@ int structure_form_H(cip_engine* h) {
 int structure_AT(cip_engine* h, double* out, const double* x, const double* add, int b) {
   RowStructure& rs = h->rs;
   cudaStream_t s = h->stream;
-  if (rs.nr > 0) {
+  if (rs.nJ > 0) {
     gather_vec_kernel<<<nb(rs.nr, 256), 256, 0, s>>>(rs.xr[b], x, rs.rest_row, rs.nr);
     CIP_CHECK_LAUNCH();
     CIP_TRY(q4_mv_rows(rs.outJ[b], rs.At4r, rs.nJ_pad, rs.nJ, rs.nr, rs.xr[b], h->partial, h->partial_cap, s));
   }
-  finish_at_kernel<<<nb(h->n, 256), 256, 0, s>>>(out, add, rs.nr > 0 ? rs.outJ[b] : nullptr, rs.Jinv, rs.sing_ptr,
+  finish_at_kernel<<<nb(h->n, 256), 256, 0, s>>>(out, add, rs.nJ > 0 ? rs.outJ[b] : nullptr, rs.Jinv, rs.sing_ptr,
                                                  rs.sing_row, rs.sing_val, x, h->n);
   CIP_CHECK_LAUNCH();
   return 0;
@@ -555,7 +557,7 @@ int structure_AT2(cip_engine* h, double* outa, double* outb, const double* xa, c
   RowStructure& rs = h->rs;
   cudaStream_t s = h->stream;
   const double* xs[2] = {xa, xb};
-  if (rs.nr > 0) {
+  if (rs.nJ > 0) {
     for (int b = 0; b < 2; ++b) {
       gather_vec_kernel<<<nb(rs.nr, 256), 256, 0, s>>>(rs.xr[b], xs[b], rs.rest_row, rs.nr);
       CIP_CHECK_LAUNCH();
@@ -566,7 +568,7 @@ int structure_AT2(cip_engine* h, double* outa, double* outb, const double* xa, c
   double* outs[2] = {outa, outb};
   const double* adds[2] = {adda, addb};
   for (int b = 0; b < 2; ++b) {
-    finish_at_kernel<<<nb(h->n, 256), 256, 0, s>>>(outs[b], adds[b], rs.nr > 0 ? rs.outJ[b] : nullptr, rs.Jinv,
+    finish_at_kernel<<<nb(h->n, 256), 256, 0, s>>>(outs[b], adds[b], rs.nJ > 0 ? rs.outJ[b] : nullptr, rs.Jinv,
                                                    rs.sing_ptr, rs.sing_row, rs.sing_val, xs[b], h->n);
     CIP_CHECK_LAUNCH();
   }
@@ -589,12 +591,13 @@ int gather_J(cip_engine* h, const double* y, int b, const double** out) {
 int structure_A(cip_engine* h, double* out, const double* y, int b) {
   RowStructure& rs = h->rs;
   cudaStream_t s = h->stream;
-  if (rs.nr > 0) {
+  const double* outr = rs.nJ > 0 ? rs.outr[b] : nullptr;
+  if (outr) {
     const double* yj;
     CIP_TRY(gather_J(h, y, b, &yj));
     CIP_TRY(q4_mv_k(rs.outr[b], rs.At4r, rs.nJ_pad, rs.nJ, rs.nr, yj, s));
   }
-  finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(out, rs.outr[b], rs.row_code, rs.sing_col, rs.sing_val, y, h->m);
+  finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(out, outr, rs.row_code, rs.sing_col, rs.sing_val, y, h->m);
   CIP_CHECK_LAUNCH();
   return 0;
 }
@@ -602,15 +605,16 @@ int structure_A(cip_engine* h, double* out, const double* y, int b) {
 int structure_A2(cip_engine* h, double* outa, double* outb, const double* ya, const double* yb) {
   RowStructure& rs = h->rs;
   cudaStream_t s = h->stream;
-  if (rs.nr > 0) {
+  const bool rest = rs.nJ > 0;
+  if (rest) {
     const double *ja, *jb;
     CIP_TRY(gather_J(h, ya, 0, &ja));
     CIP_TRY(gather_J(h, yb, 1, &jb));
     CIP_TRY(q4_mv_k2(rs.outr[0], rs.outr[1], rs.At4r, rs.nJ_pad, rs.nJ, rs.nr, ja, jb, s));
   }
-  finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(outa, rs.outr[0], rs.row_code, rs.sing_col, rs.sing_val, ya, h->m);
+  finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(outa, rest ? rs.outr[0] : nullptr, rs.row_code, rs.sing_col, rs.sing_val, ya, h->m);
   CIP_CHECK_LAUNCH();
-  finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(outb, rs.outr[1], rs.row_code, rs.sing_col, rs.sing_val, yb, h->m);
+  finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(outb, rest ? rs.outr[1] : nullptr, rs.row_code, rs.sing_col, rs.sing_val, yb, h->m);
   CIP_CHECK_LAUNCH();
   return 0;
 }
