@@ -27,6 +27,11 @@ class StructureInfo(C.Structure):
                 ("rest_rows", C.c_int), ("rest_cols", C.c_int), ("compressed", C.c_int), ("base_has_gtg", C.c_int)]
 
 
+class SplitInfo(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("enabled", C.c_int), ("coupled_cols", C.c_int), ("diagonal_cols", C.c_int),
+                ("cols_from_rest", C.c_int), ("cols_from_Q", C.c_int), ("cols_from_G", C.c_int)]
+
+
 class Stats(C.Structure):
     _fields_ = [("n", C.c_int), ("m", C.c_int), ("p", C.c_int),
                 ("n_pad", C.c_int), ("m_pad", C.c_int), ("p_pad", C.c_int),
@@ -95,6 +100,7 @@ SIGNATURES = {
     "cip_ipm_solve": (C.c_int, [C.c_void_p, _P, _P, _P, C.POINTER(IpmOptions), _P, _P, _P, C.POINTER(IpmResult)]),
     "cip_stats": (C.c_int, [C.c_void_p, C.POINTER(Stats)]),
     "cip_structure_info": (C.c_int, [C.c_void_p, C.POINTER(StructureInfo)]),
+    "cip_split_info": (C.c_int, [C.c_void_p, C.POINTER(SplitInfo)]),
     "cip_get_H": (C.c_int, [C.c_void_p, _P, C.c_int]),
     "cip_form_H": (C.c_int, [C.c_void_p]),
     "cip_factor_H": (C.c_int, [C.c_void_p]),

@@ -6,6 +6,7 @@
 //                         -> [NCCL all-reduce of the partial Gram matrices] -> blocked Cholesky
 //                         -> Schur complement on G (same DMMA tiles).
 // LEVEL 3 (cip_solve)   : the pivot algebra of src/kktsolvers.jl:324-332 on the resident data.
+#include <climits>
 #include <stdarg.h>
 #include <stdlib.h>
 #include <string.h>
@@ -125,6 +126,11 @@ double* vec_out(cip_engine* h, double* stage, double* dst, size_t n) {
 int vec_out_done(cip_engine* h, double* dst, const double* produced, size_t n) {
   if (n == 0 || !dst || produced == dst) return 0;
   return stage_out(h, dst, produced, n);
+}
+
+// give-up flag of the persistent sweeps with H's factor (none when row_structure = 2 left K empty)
+int* h_sweep_err(const cip_engine* h) {
+  return h->rs.sp.on ? (h->rs.sp.nK > 0 ? h->rs.sp.chol.sweep_err : nullptr) : h->cholH.sweep_err;
 }
 
 int finish(cip_engine* h) {
@@ -288,7 +294,10 @@ int form_H(cip_engine* h) {
   CIP_CUDA(cudaEventRecord(h->ev[0], s));
   if (h->rs.on) {
     CIP_TRY(structure_form_H(h));
-    if (h->opt.reg_delta != 0.0) CIP_TRY(add_diag_q4(h->H4, h->n_pad, 0, h->n, h->opt.reg_delta, 0, s));
+    if (h->opt.reg_delta != 0.0) {
+      if (h->rs.sp.on) CIP_TRY(split_add_delta(h, h->opt.reg_delta));
+      else CIP_TRY(add_diag_q4(h->H4, h->n_pad, 0, h->n, h->opt.reg_delta, 0, s));
+    }
     CIP_CUDA(cudaEventRecord(h->ev[3], s));
     return 0;
   }
@@ -346,21 +355,27 @@ int form_H(cip_engine* h) {
 
 int factor_H(cip_engine* h) {
   cudaStream_t s = h->stream;
-  // block-cyclic distributed factorisation when A is row-sharded (every rank holds the reduced H);
-  // opts.dist_chol: 0 = replicated, 1 = distributed, -1/unset = distributed iff >= 2 outer panels per rank
-  bool dist = false;
-  if (h->comm && h->nranks > 1) {
-    const int outer_panels = (h->cholH.npanels + 3) / 4;   // 512-column units
-    int mode = h->opt.dist_chol;
-    if (const char* env = getenv("CIP_DIST_CHOL")) mode = atoi(env);
-    dist = (mode == 1) || (mode != 0 && outer_panels >= 2 * h->nranks);
-  }
-  if (dist) {
-    CholDist d;
-    d.nranks = h->nranks; d.rank = h->rank; d.comm = h->comm;
-    CIP_TRY(chol_factor_dist(h->cholH, s, d));
+  // row_structure = 2: H_KK is factored on its own plan and D by split_factor; the Schur block below runs on Z_K
+  const RowStructure::Split& sp = h->rs.sp;
+  if (sp.on) {
+    CIP_TRY(split_factor(h));
   } else {
-    CIP_TRY(chol_factor(h->cholH, s));
+    // block-cyclic distributed factorisation when A is row-sharded (every rank holds the reduced H);
+    // opts.dist_chol: 0 = replicated, 1 = distributed, -1/unset = distributed iff >= 2 outer panels per rank
+    bool dist = false;
+    if (h->comm && h->nranks > 1) {
+      const int outer_panels = (h->cholH.npanels + 3) / 4;   // 512-column units
+      int mode = h->opt.dist_chol;
+      if (const char* env = getenv("CIP_DIST_CHOL")) mode = atoi(env);
+      dist = (mode == 1) || (mode != 0 && outer_panels >= 2 * h->nranks);
+    }
+    if (dist) {
+      CholDist d;
+      d.nranks = h->nranks; d.rank = h->rank; d.comm = h->comm;
+      CIP_TRY(chol_factor_dist(h->cholH, s, d));
+    } else {
+      CIP_TRY(chol_factor(h->cholH, s));
+    }
   }
   CIP_CUDA(cudaEventRecord(h->ev[4], s));
   if (h->p > 0) {
@@ -368,21 +383,25 @@ int factor_H(cip_engine* h) {
     // Two-level like the Cholesky: inside an outer panel of four 128-column panels every panel is solved against
     // inv(L_jj) and applied to the rest of the outer panel only; everything right of the outer panel gets ONE update
     // with K = 512, which amortises the C-tile read-modify-write that holds K = 128 tiles at a third of the pipe.
-    CIP_TRY(vec_copy(h->Z4, h->G4, (size_t)h->p_pad * h->n_pad, s));
-    const int np = h->n_pad / TILE, ptiles = h->p_pad / TILE;
+    // (row_structure = 2: Z_K = G_K L_KK^-T over the K columns)
+    const CholPlan& L = sp.on ? sp.chol : h->cholH;
+    double* Z = sp.on ? sp.ZK4 : h->Z4;
+    const GemmOperand& mapZ = sp.on ? sp.mapZK : h->mapZ;
+    const int np = (sp.on ? sp.nK_pad : h->n_pad) / TILE, ptiles = h->p_pad / TILE;
+    if (np > 0) CIP_TRY(vec_copy(Z, sp.on ? sp.GK4 : h->G4, (size_t)h->p_pad * np * TILE, s));
     auto z_trsm = [&](int jb) -> int {                       // Z[:, jb] <- Z[:, jb] inv(L_jj)'
       GemmArgs t{};
       t.lower = 0; t.ntm = ptiles; t.ntn = 1; t.sym = 0;
       t.x_row0 = 0; t.y_row0 = 0; t.x_kq0 = jb * TILE / 4; t.y_kq0 = 32 * jb; t.nk = TILE / 32;
-      t.Cin = nullptr; t.Cout = h->Z4; t.ldc = h->p_pad; t.c_row0 = 0; t.c_col0 = jb * TILE; t.alpha = 1.0;
-      return launch_gemm_nt(h->mapZ, h->cholH.mapWinv, t, s);
+      t.Cin = nullptr; t.Cout = Z; t.ldc = h->p_pad; t.c_row0 = 0; t.c_col0 = jb * TILE; t.alpha = 1.0;
+      return launch_gemm_nt(mapZ, L.mapWinv, t, s);
     };
     auto z_update = [&](int k0, int kn, int c0, int cn) -> int {   // Z[:, c0..c0+cn) -= Z[:, k0..k0+kn) L[c0..c0+cn, k0..k0+kn)'   (panel units)
       GemmArgs u{};
       u.lower = 0; u.ntm = ptiles; u.ntn = cn; u.sym = 0;
       u.x_row0 = 0; u.y_row0 = c0 * TILE; u.x_kq0 = k0 * TILE / 4; u.y_kq0 = k0 * TILE / 4; u.nk = kn * TILE / 32;
-      u.Cin = h->Z4; u.Cout = h->Z4; u.ldc = h->p_pad; u.c_row0 = 0; u.c_col0 = c0 * TILE; u.alpha = -1.0;
-      return launch_gemm_nt(h->mapZ, h->cholH.mapH, u, s);
+      u.Cin = Z; u.Cout = Z; u.ldc = h->p_pad; u.c_row0 = 0; u.c_col0 = c0 * TILE; u.alpha = -1.0;
+      return launch_gemm_nt(mapZ, L.mapH, u, s);
     };
     // (few right-hand-side tiles, p <= 384: every launch is latency-bound and the extra level only lengthens the chain --
     //  config 3, p = 256: 1.73 ms single-level against 2.07 ms two-level; config 5, p = 1000: 22.0 ms against 35.6 ms)
@@ -397,15 +416,26 @@ int factor_H(cip_engine* h) {
     }
     GemmArgs a{};
     a.lower = 1; a.ntm = a.ntn = ptiles; a.sym = 1;
-    a.x_row0 = a.y_row0 = 0; a.x_kq0 = a.y_kq0 = 0; a.nk = h->n_pad / 32;
+    a.x_row0 = a.y_row0 = 0; a.x_kq0 = a.y_kq0 = 0;
     a.Cin = h->Sbase4; a.Cout = h->S4; a.ldc = h->p_pad; a.c_row0 = a.c_col0 = 0; a.alpha = 1.0;
     a.ws = h->gemm_ws; a.ws_doubles = GEMM_WS_DOUBLES;
-    CIP_TRY(launch_gemm_nt(h->mapZ, h->mapZ, a, s));
+    if (sp.on && sp.g_in_D) {
+      // + G_D diag(1/h) G_D': the folded-scaling SYRK over all of G with kscale = h^-1/2 on D and 0 on K
+      GemmArgs g = a;
+      g.nk = h->n_pad / 32;
+      g.kscale = sp.kscale;
+      CIP_TRY(launch_gemm_nt(sp.mapG, sp.mapG, g, s));
+      a.Cin = h->S4;
+    }
+    a.nk = np * TILE / 32;
+    if (np > 0) CIP_TRY(launch_gemm_nt(mapZ, mapZ, a, s));
+    else if (a.Cin != h->S4) CIP_TRY(vec_copy(h->S4, h->Sbase4, (size_t)h->p_pad * h->p_pad, s));
     CIP_TRY(chol_factor(h->cholS, s));
   }
   CIP_CUDA(cudaEventRecord(h->ev[5], s));
-  int hinfo[2] = {0, 0};
+  int hinfo[2] = {0, 0}, dfail = INT_MAX;
   CIP_CUDA(cudaMemcpyAsync(hinfo, h->info, sizeof(hinfo), cudaMemcpyDeviceToHost, s));
+  if (sp.on) CIP_CUDA(cudaMemcpyAsync(&dfail, sp.fail, sizeof(int), cudaMemcpyDeviceToHost, s));
   CIP_CUDA(cudaStreamSynchronize(s));
   float ms = 0;
   cudaEventElapsedTime(&ms, h->ev[0], h->ev[1]); h->st.ms_scale = ms;
@@ -414,9 +444,17 @@ int factor_H(cip_engine* h) {
   cudaEventElapsedTime(&ms, h->ev[3], h->ev[4]); h->st.ms_chol = ms;
   cudaEventElapsedTime(&ms, h->ev[4], h->ev[5]); h->st.ms_schur = ms;
   cudaGetLastError();
-  h->st.chol_flops = (double)h->n * h->n * h->n / 3.0;
+  const double nf = sp.on ? sp.nK : h->n;
+  h->st.chol_flops = nf * nf * nf / 3.0;
   h->st.factors++;
   h->have_factor = true;
+  if (sp.on) {
+    // the first failing pivot in natural column order: the smallest failing D column or the K column where the
+    // factorisation of H_KK stopped (1-based, as the dense path reports it)
+    int col = std::min(dfail, h->n);
+    if (hinfo[0] != 0) col = std::min(col, sp.K[hinfo[0] - 1]);
+    hinfo[0] = col < h->n ? col + 1 : 0;
+  }
   if (hinfo[0] != 0) {
     set_error("Cholesky of H failed: non-positive pivot at column %d", hinfo[0]);
     return hinfo[0];
@@ -545,11 +583,12 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
     // (0 when the caller's struct does not reach the field: h->opt starts zeroed)
     int rs = h->opt.row_structure;
     if (const char* env = getenv("CIP_ROW_STRUCTURE")) { if (!shard) rs = atoi(env); }
-    if (rs != 0 && rs != 1) {
-      set_error("cip_create: row_structure must be 0 or 1 (got %d)", rs);
+    if (rs != 0 && rs != 1 && rs != 2) {
+      set_error("cip_create: row_structure must be 0, 1 or 2 (got %d)", rs);
       return -1;
     }
-    h->rs.on = (rs == 1) && m > 0;     // no rows: nothing to classify
+    h->rs.on = (rs == 1 || rs == 2) && m > 0;     // no rows: nothing to classify
+    h->rs.sp.on = (rs == 2) && m > 0;
   }
   if (h->opt.device < 0) CIP_CUDA(cudaGetDevice(&h->device));
   else h->device = h->opt.device;
@@ -670,15 +709,19 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   // (h->opt.fold_scaling is 0 when the caller's struct does not reach the field: h->opt starts zeroed)
   if (!h->rs.on) CIP_TRY(engine_decide_fold(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0, mn, &h->fold));
   if (!h->fold && !h->rs.on) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
-  CIP_TRY(dev_alloc(h, &h->Qq4, nn));
-  CIP_TRY(dev_alloc(h, &h->H4, nn));
+  // row_structure = 2 keeps no n_pad^2 buffer: dense Q is staged in Qq4 until split_build has gathered Q_KK
+  const bool split = h->rs.sp.on;
+  if (!split || (!Qs && h->opt.q_kind == 0)) CIP_TRY(dev_alloc(h, &h->Qq4, nn));
+  if (!split) CIP_TRY(dev_alloc(h, &h->H4, nn));
   CIP_TRY(dev_alloc(h, &h->gemm_ws, (size_t)GEMM_WS_DOUBLES));
-  CIP_TRY(dev_alloc(h, &h->Winv, (size_t)h->n_pad * TILE));
+  if (!split) CIP_TRY(dev_alloc(h, &h->Winv, (size_t)h->n_pad * TILE));
   CIP_TRY(dev_alloc(h, &h->info, 4));
   cudaStream_t s = h->stream;
 
   // Q
-  if (Qs) {
+  if (Qs && split) {
+    CIP_TRY(split_classify_csc_Q(h, Qs));
+  } else if (Qs) {
     CIP_TRY(upload_csc(h, h->Qq4, h->n_pad, Qs, 0));
   } else if (h->opt.q_kind == 0) {
     if (!Q) { set_error("Q is null"); return -1; }
@@ -702,14 +745,18 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
     }
   } else if (h->opt.q_kind == 1) {
     if (!Q) { set_error("Q (diagonal) is null"); return -1; }
-    double* dq = nullptr;
-    CIP_CUDA(cudaMalloc(&dq, sizeof(double) * n));
-    CIP_CUDA(cudaMemcpyAsync(dq, Q, sizeof(double) * n, cudaMemcpyDefault, s));
-    CIP_TRY(set_diag_vec_q4(h->Qq4, h->n_pad, n, dq, s));
-    CIP_CUDA(cudaStreamSynchronize(s));
-    cudaFree(dq);
+    if (split) {
+      CIP_TRY(split_diag_Q(h, Q));
+    } else {
+      double* dq = nullptr;
+      CIP_CUDA(cudaMalloc(&dq, sizeof(double) * n));
+      CIP_CUDA(cudaMemcpyAsync(dq, Q, sizeof(double) * n, cudaMemcpyDefault, s));
+      CIP_TRY(set_diag_vec_q4(h->Qq4, h->n_pad, n, dq, s));
+      CIP_CUDA(cudaStreamSynchronize(s));
+      cudaFree(dq);
+    }
   }
-  CIP_TRY(add_diag_q4(h->Qq4, h->n_pad, n, h->n_pad, 1.0, 1, s));  // identity on the padding
+  if (h->Qq4) CIP_TRY(add_diag_q4(h->Qq4, h->n_pad, n, h->n_pad, 1.0, 1, s));  // identity on the padding
 
   // A (transposed into Q4: rows = columns of A)
   if (m > 0) {
@@ -742,14 +789,14 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   } else if (h->m_pad + h->aug_rows > 0) {
     CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (h->m_pad + h->aug_rows) / 4));
   }
-  CIP_TRY(chol_make_plan(&h->cholH, h->H4, h->n_pad, h->Winv, h->info));
+  if (!split) CIP_TRY(chol_make_plan(&h->cholH, h->H4, h->n_pad, h->Winv, h->info));
 
   // G
   if (p > 0) {
     if (!G && !Gs) { set_error("G is null"); return -1; }
     const size_t pn = (size_t)h->p_pad * h->n_pad;
     CIP_TRY(dev_alloc(h, &h->G4, pn));
-    CIP_TRY(dev_alloc(h, &h->Z4, pn));
+    if (!split) CIP_TRY(dev_alloc(h, &h->Z4, pn));
     CIP_TRY(dev_alloc(h, &h->S4, (size_t)h->p_pad * h->p_pad));
     CIP_TRY(dev_alloc(h, &h->Sbase4, (size_t)h->p_pad * h->p_pad));
     CIP_TRY(dev_alloc(h, &h->WinvS, (size_t)h->p_pad * TILE));
@@ -773,7 +820,7 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
       CIP_TRY(transpose_scale_q4(h->Atil4, h->n_pad, h->m_pad, h->G4, h->p_pad, p, n, sqrt(h->aug_rho), s));
     CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, p, h->p_pad, 1.0, 1, s));
     if (h->opt.reg_eps_G != 0.0) CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, 0, p, h->opt.reg_eps_G, 1, s));
-    CIP_TRY(make_q4_tensor_map(&h->mapZ.map, h->Z4, h->p_pad, h->n_pad / 4));
+    if (!split) CIP_TRY(make_q4_tensor_map(&h->mapZ.map, h->Z4, h->p_pad, h->n_pad / 4));
     CIP_TRY(chol_make_plan(&h->cholS, h->S4, h->p_pad, h->WinvS, h->info + 1));
   }
   if (h->rs.on) CIP_TRY(structure_finish(h));
@@ -884,6 +931,7 @@ int cip_destroy(cip_handle h) {
   for (auto v : h->pv2) if (v) cudaFree(v);
   chol_free_plan(&h->cholH);
   chol_free_plan(&h->cholS);
+  chol_free_plan(&h->rs.sp.chol);
   if (h->Hp) cudaFree(h->Hp);
   if (h->d_sws) cudaFree(h->d_sws);
   if (h->cs) cudaStreamDestroy(h->cs);
@@ -1096,16 +1144,20 @@ int cip_solve(cip_handle h, const double* ry, const double* rw, const double* rv
     CIP_TRY(vec_axpby(h->nv[2], 1.0, h->nv[2], h->aug_rho, h->nv[4], h->n, s));
   }
   // 2x2 solve with H = L L' and the Schur complement on G (:299)
-  CIP_TRY(chol_fwd(h->cholH, h->nv[2], h->nv[3], s));
-  if (h->p) {
-    CIP_TRY(q4_mv_rows(h->pv[1], h->Z4, h->p_pad, h->p, h->n, h->nv[3], h->partial, h->partial_cap, s));
-    CIP_TRY(vec_axpby(h->pv[2], 1.0, h->pv[1], -1.0, h->pv[0], h->p, s));
-    CIP_TRY(chol_fwd(h->cholS, h->pv[2], h->pv[3], s));
-    CIP_TRY(chol_bwd(h->cholS, h->pv[3], h->pv[4], s));
-    CIP_TRY(q4_mv_k(h->nv[4], h->Z4, h->p_pad, h->p, h->n, h->pv[4], s));
-    CIP_TRY(vec_axpby(h->nv[3], 1.0, h->nv[3], -1.0, h->nv[4], h->n, s));
+  if (h->rs.sp.on) {
+    CIP_TRY(split_solve(h, h->nv, h->pv, 0, h->p > 0));
+  } else {
+    CIP_TRY(chol_fwd(h->cholH, h->nv[2], h->nv[3], s));
+    if (h->p) {
+      CIP_TRY(q4_mv_rows(h->pv[1], h->Z4, h->p_pad, h->p, h->n, h->nv[3], h->partial, h->partial_cap, s));
+      CIP_TRY(vec_axpby(h->pv[2], 1.0, h->pv[1], -1.0, h->pv[0], h->p, s));
+      CIP_TRY(chol_fwd(h->cholS, h->pv[2], h->pv[3], s));
+      CIP_TRY(chol_bwd(h->cholS, h->pv[3], h->pv[4], s));
+      CIP_TRY(q4_mv_k(h->nv[4], h->Z4, h->p_pad, h->p, h->n, h->pv[4], s));
+      CIP_TRY(vec_axpby(h->nv[3], 1.0, h->nv[3], -1.0, h->nv[4], h->n, s));
+    }
+    CIP_TRY(chol_bwd(h->cholH, h->nv[3], h->nv[5], s));
   }
-  CIP_TRY(chol_bwd(h->cholH, h->nv[3], h->nv[5], s));
   // dv = t1 - F^-T F^-T (A dy)                           (:328)
   if (h->m) {
     if (h->rs.on) CIP_TRY(structure_A(h, h->mv[3], h->nv[5], 0));
@@ -1121,7 +1173,7 @@ int cip_solve(cip_handle h, const double* ry, const double* rw, const double* rv
     // the call synchronises anyway: also read the give-up flag of the persistent sweeps (a hand-off that never
     // arrived -- a bug, not a numerical condition -- must not pass for a solution)
     int bad[2] = {0, 0};
-    CIP_CUDA(cudaMemcpyAsync(&bad[0], h->cholH.sweep_err, sizeof(int), cudaMemcpyDeviceToHost, s));
+    if (h_sweep_err(h)) CIP_CUDA(cudaMemcpyAsync(&bad[0], h_sweep_err(h), sizeof(int), cudaMemcpyDeviceToHost, s));
     if (h->p) CIP_CUDA(cudaMemcpyAsync(&bad[1], h->cholS.sweep_err, sizeof(int), cudaMemcpyDeviceToHost, s));
     CIP_TRY(finish(h));
     if (bad[0] || bad[1]) {
@@ -1197,6 +1249,10 @@ int cip_solve_multi(cip_handle h, int nrhs, const double* ry, int ldy, const dou
         CIP_TRY(q4_mv_k(nv[4], h->G4, h->p_pad, h->p, h->n, pv[0], s));
         CIP_TRY(vec_axpby(nv[2], 1.0, nv[2], h->aug_rho, nv[4], h->n, s));
       }
+      if (h->rs.sp.on) {
+        CIP_TRY(split_solve(h, nv, pv, b, h->p > 0));
+        continue;
+      }
       CIP_TRY(chol_fwd(h->cholH, nv[2], nv[3], s));
       if (h->p) {
         CIP_TRY(q4_mv_rows(pv[1], h->Z4, h->p_pad, h->p, h->n, nv[3], h->partial, h->partial_cap, s));
@@ -1224,7 +1280,7 @@ int cip_solve_multi(cip_handle h, int nrhs, const double* ry, int ldy, const dou
     h->st.solves += 2;
     int bad[2] = {0, 0};
     if (h->need_sync || h->always_sync) {
-      CIP_CUDA(cudaMemcpyAsync(&bad[0], h->cholH.sweep_err, sizeof(int), cudaMemcpyDeviceToHost, s));
+      if (h_sweep_err(h)) CIP_CUDA(cudaMemcpyAsync(&bad[0], h_sweep_err(h), sizeof(int), cudaMemcpyDeviceToHost, s));
       if (h->p) CIP_CUDA(cudaMemcpyAsync(&bad[1], h->cholS.sweep_err, sizeof(int), cudaMemcpyDeviceToHost, s));
     }
     CIP_TRY(finish(h));
@@ -1246,8 +1302,12 @@ int cip_solve_H(cip_handle h, const double* rhs, double* x) {
   cudaStream_t s = h->stream;
   CIP_TRY(stage_in(h, h->nv[2], rhs, h->n));
   CIP_CUDA(cudaEventRecord(h->ev[6], s));
-  CIP_TRY(chol_fwd(h->cholH, h->nv[2], h->nv[3], s));
-  CIP_TRY(chol_bwd(h->cholH, h->nv[3], h->nv[5], s));
+  if (h->rs.sp.on) {
+    CIP_TRY(split_solve(h, h->nv, h->pv, 0, false));
+  } else {
+    CIP_TRY(chol_fwd(h->cholH, h->nv[2], h->nv[3], s));
+    CIP_TRY(chol_bwd(h->cholH, h->nv[3], h->nv[5], s));
+  }
   CIP_CUDA(cudaEventRecord(h->ev[7], s));
   CIP_TRY(stage_out(h, x, h->nv[5], h->n));
   h->st.solves++;
@@ -1308,7 +1368,8 @@ int cip_mul_Q(cip_handle h, const double* x, double* y) {
   const double* xp;
   CIP_TRY(vec_in(h, h->nv[6], x, h->n, &xp, /*padded=*/true));
   double* yp = (y != x) ? vec_out(h, h->nv[7], y, h->n) : h->nv[7];
-  CIP_TRY(q4_mv_rows(yp, h->Qq4, h->n_pad, h->n, h->n, xp, h->partial, h->partial_cap, s));
+  if (h->rs.sp.on) CIP_TRY(split_mul_Q(h, yp, xp));
+  else CIP_TRY(q4_mv_rows(yp, h->Qq4, h->n_pad, h->n, h->n, xp, h->partial, h->partial_cap, s));
   CIP_TRY(vec_out_done(h, y, yp, h->n));
   return finish(h);
 }
@@ -1341,8 +1402,29 @@ int cip_structure_info(cip_handle h, cip_structure_t* out) {
     r.empty_rows = rs.nempty;
     r.rest_rows = rs.nr;
     r.rest_cols = rs.nJ;
-    r.compressed = rs.compressed;
+    r.compressed = rs.compressed || rs.sp.on;
     r.base_has_gtg = rs.base_has_gtg;
+  }
+  memcpy(out, &r, std::min<size_t>(sizeof(r), (size_t)out->struct_size));
+  return 0;
+}
+
+int cip_split_info(cip_handle h, cip_split_t* out) {
+  CIP_TRY(check(h));
+  if (!out || out->struct_size < (int)sizeof(int)) {
+    set_error("cip_split_info: out->struct_size must be set");
+    return -1;
+  }
+  cip_split_t r{};
+  r.struct_size = out->struct_size;
+  const RowStructure::Split& sp = h->rs.sp;      // (a multi-GPU front never has it on)
+  if (sp.on) {
+    r.enabled = 1;
+    r.coupled_cols = sp.nK;
+    r.diagonal_cols = h->n - sp.nK;
+    r.cols_from_rest = sp.from_rest;
+    r.cols_from_Q = sp.from_Q;
+    r.cols_from_G = sp.from_G;
   }
   memcpy(out, &r, std::min<size_t>(sizeof(r), (size_t)out->struct_size));
   return 0;
@@ -1353,7 +1435,9 @@ int cip_get_H(cip_handle h, double* out, int ldo) {
   if (h->multi) return multi_simple(h, 3, out, ldo);
   double* tmp = nullptr;
   CIP_CUDA(cudaMalloc(&tmp, (size_t)h->n * h->n * 8));
-  CIP_TRY(unpack_rows_q4(tmp, h->n, h->H4, h->n_pad, h->n, h->n, h->stream));
+  const int rc = h->rs.sp.on ? split_get_H(h, tmp) : unpack_rows_q4(tmp, h->n, h->H4, h->n_pad, h->n, h->n, h->stream);
+  if (rc != 0) cudaFree(tmp);
+  CIP_TRY(rc);
   CIP_CUDA(cudaMemcpy2DAsync(out, (size_t)ldo * 8, tmp, (size_t)h->n * 8, (size_t)h->n * 8, h->n, cudaMemcpyDefault,
                              h->stream));
   CIP_CUDA(cudaStreamSynchronize(h->stream));

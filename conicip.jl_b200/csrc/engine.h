@@ -34,6 +34,28 @@ struct RowStructure {
   Scaling Fi{};                     // Fi gathered into rest order (R / Ri shared with the handle's)
   // work vectors of the mat-vecs, two sets (cip_solve_multi pairs): x[rest], y[J], products
   double *xr[2] = {}, *yJ[2] = {}, *outr[2] = {}, *outJ[2] = {};
+
+  // row_structure = 2: the columns of H split into K (coupled: touched by a rest row, by an off-diagonal entry of Q,
+  // or -- when rho > 0 -- by G) and D (all others, where H holds only its diagonal h_j).  H_KK is dense and factored
+  // with a Cholesky plan over nK_pad; D is factored as sqrt(h_j).  No n_pad^2 buffer exists.
+  struct Split {
+    bool on = false;
+    int nK = 0, nK_pad = 0, from_rest = 0, from_Q = 0, from_G = 0;
+    bool g_in_D = false;            // some column of G lies in D: S gets G diag(kscale^2) G' and the solves G u
+    bool factored = false;          // HK4 holds L_KK (cip_get_H shows L), else H_KK
+    std::vector<int> K;             // host copy: failing K pivot -> global column
+    std::vector<char> q_couple;     // per column: Q couples it (LEVEL 1, until K is built)
+    struct QEntry { int i, j; double v; };
+    std::vector<QEntry> qtrip;      // CSC Q: summed diagonal entries and those between coupled columns (LEVEL 1)
+    int *dK = nullptr, *Kpos = nullptr, *JK = nullptr;   // [nK], [n] (-1: column in D), [nJ]: K position of J[a]
+    double *QK4 = nullptr, *BaseK4 = nullptr, *HK4 = nullptr, *WinvK = nullptr;   // nK_pad^2, nK_pad * TILE
+    double *qD = nullptr, *hD = nullptr, *kscale = nullptr;   // [n_pad]: diagonal of Q, h on D, h^-1/2 on D
+    double *GK4 = nullptr, *ZK4 = nullptr;   // p_pad x nK_pad
+    CholPlan chol{};
+    GemmOperand mapZK{}, mapG{};
+    int* fail = nullptr;            // smallest global D column with h_j <= 0 (INT_MAX-ish when none)
+    double* kv[2][3] = {};          // per column set b: rhs_K, t_K, products on K (nK_pad + 4 each)
+  } sp;
 };
 }  // namespace cip
 
@@ -129,6 +151,19 @@ int structure_AT2(cip_engine* h, double* outa, double* outb, const double* xa, c
 // out[m] = A y  (y: n-vector)
 int structure_A(cip_engine* h, double* out, const double* y, int b);
 int structure_A2(cip_engine* h, double* outa, double* outb, const double* ya, const double* yb);
+// row_structure = 2 (structure.cu).  LEVEL 1, dense Q in h->Qq4 or CSC / diagonal / no Q: the Q diagonal and which
+// columns Q couples (the dense staging copy stays until split_build)
+int split_classify_csc_Q(cip_engine* h, const cip_csc* Q);
+int split_diag_Q(cip_engine* h, const double* q);
+// LEVEL 1, after G4 and the row split: K, QK4, BaseK4, GK4, the K Cholesky plan; frees the dense Q staging copy
+int split_build(cip_engine* h);
+// LEVEL 2: Cholesky of H_KK, the pivots of D (kscale, the smallest failing D column); the Schur block is factor_H's
+int split_factor(cip_engine* h);
+int split_add_delta(cip_engine* h, double delta);
+// LEVEL 3 on one column set: nv[2] = rhs in, nv[5] = dy out; pv[0] = rw, pv[4] = dw out (schur: p > 0)
+int split_solve(cip_engine* h, double** nv, double** pv, int b, bool schur);
+int split_mul_Q(cip_engine* h, double* y, const double* x);
+int split_get_H(cip_engine* h, double* tmp);   // n x n, column-major
 
 // ---- single-process multi-GPU front (multi.cu): same contracts as the C ABI entry points, global vectors
 int multi_create(cip_handle* out, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,

@@ -13,6 +13,7 @@
 // J can be empty while the rest has rows (a Q or S cone whose rows of A are all zero): those rows add nothing to
 // H, A y or A'x, so the operand map, the SYRK, the scatter and the rest mat-vecs are skipped.
 // A non-zero is a stored value != 0.0, for dense and CSC input alike.
+// row_structure = 2 splits the columns of H on top of this (second half of the file).
 #include <climits>
 #include <math.h>
 #include <stdlib.h>
@@ -126,10 +127,12 @@ __global__ void scatter_gram_kernel(double* __restrict__ H4, int ld, const doubl
   }
 }
 
-// H_jj += sum over the singletons of column j of (Fi.a[i] a_ij)^2, rows in ascending order
+// H_jj += sum over the singletons of column j of (Fi.a[i] a_ij)^2, rows in ascending order.  With a position map
+// (row_structure = 2) column j is row pos[j] of H4, or goes to hD[j] when pos[j] < 0.
 __global__ void singleton_diag_kernel(double* __restrict__ H4, int ld, int n, const int* __restrict__ ptr,
                                       const int* __restrict__ row, const double* __restrict__ val,
-                                      const double* __restrict__ ia) {
+                                      const double* __restrict__ ia, const int* __restrict__ pos,
+                                      double* __restrict__ hD) {
   const int j = blockIdx.x * blockDim.x + threadIdx.x;
   if (j >= n) return;
   const int e0 = ptr[j], e1 = ptr[j + 1];
@@ -139,7 +142,9 @@ __global__ void singleton_diag_kernel(double* __restrict__ H4, int ld, int n, co
     const double t = ia[row[e]] * val[e];
     acc += t * t;
   }
-  H4[q4_index(j, j, ld)] += acc;
+  const int k = pos ? pos[j] : j;
+  if (k >= 0) H4[q4_index(k, k, ld)] += acc;
+  else hD[j] += acc;
 }
 
 // ---------------------------------------------------------------- mat-vec kernels
@@ -249,7 +254,8 @@ int upload_plan(cip_engine* h, const Plan& P, const std::vector<int>& touched) {
   std::vector<int> J;
   for (int j = 0; j < n; ++j)
     if (touched[j]) J.push_back(j);
-  rs.compressed = rs.nr > 0 && round_up((int)J.size(), TILE) <= h->n_pad / 2;
+  // (row_structure = 2 always compresses: H has no n_pad-wide buffer to take the Gram matrix of all columns)
+  rs.compressed = rs.nr > 0 && (rs.sp.on || round_up((int)J.size(), TILE) <= h->n_pad / 2);
   if (!rs.compressed) {
     J.resize(n);
     for (int j = 0; j < n; ++j) J[j] = j;
@@ -364,9 +370,12 @@ int structure_build_dense(cip_engine* h) {
   return 0;
 }
 
-int structure_build_csc(cip_engine* h, const cip_csc* A) {
-  RowStructure& rs = h->rs;
-  const int m = h->m, n = h->n;
+namespace {
+// (row, column, value) of the non-zeros of a CSC matrix (host or device arrays), columns ascending, rows ascending
+// inside a column, duplicates summed in storage order (as the scatter of the dense path adds them)
+struct E { int i, j; double v; };
+int read_csc(const cip_csc* A, int m, std::vector<E>* out) {
+  std::vector<E>& ent = *out;
   const long long ncols = A->ncols;
   const int base = A->index_base;
   std::vector<long long> cp(ncols + 1);
@@ -378,9 +387,6 @@ int structure_build_csc(cip_engine* h, const cip_csc* A) {
     CIP_CUDA(cudaMemcpy(rv.data(), A->rowval, nnz * 8, cudaMemcpyDefault));
     CIP_CUDA(cudaMemcpy(nz.data(), A->nzval, nnz * 8, cudaMemcpyDefault));
   }
-  // (row, column, value) with duplicates summed in storage order, as the scatter of the dense path adds them
-  struct E { int i, j; double v; };
-  std::vector<E> ent;
   std::vector<std::pair<int, double>> colv;
   for (long long j = 0; j < ncols; ++j) {
     const long long e0 = cp[j] - base, e1 = cp[j + 1] - base;
@@ -406,6 +412,15 @@ int structure_build_csc(cip_engine* h, const cip_csc* A) {
       t = u;
     }
   }
+  return 0;
+}
+}  // namespace
+
+int structure_build_csc(cip_engine* h, const cip_csc* A) {
+  RowStructure& rs = h->rs;
+  const int m = h->m, n = h->n;
+  std::vector<E> ent;
+  CIP_TRY(read_csc(A, m, &ent));
   RowClass rc;
   rc.cnt.assign(m, 0); rc.col.assign(m, -1); rc.val.assign(m, 0.0);
   for (const E& e : ent) {       // columns ascending: the first entry of a row is its first non-zero column
@@ -469,7 +484,9 @@ int structure_finish(cip_engine* h) {
   RowStructure& rs = h->rs;
   cudaStream_t s = h->stream;
   rs.base_has_gtg = h->p > 0 && h->aug_rows > 0;
-  if (rs.base_has_gtg) {
+  if (rs.sp.on) {
+    CIP_TRY(split_build(h));
+  } else if (rs.base_has_gtg) {
     // Base4 = Q + (sqrt(rho) G)'(sqrt(rho) G): the aug rows leave the per-factor SYRK
     const size_t nn = (size_t)h->n_pad * h->n_pad;
     double* Gt4 = nullptr;
@@ -503,7 +520,6 @@ int structure_finish(cip_engine* h) {
 int structure_form_H(cip_engine* h) {
   RowStructure& rs = h->rs;
   cudaStream_t s = h->stream;
-  const size_t nn = (size_t)h->n_pad * h->n_pad;
   const int ncr = rs.cd.ncones;
   if (rs.nJ > 0) {
     gather_scaling_kernel<<<nb(std::max(rs.nr, ncr), 256), 256, 0, s>>>(h->Fi, rs.Fi, rs.rest_row, rs.nr,
@@ -512,25 +528,37 @@ int structure_form_H(cip_engine* h) {
     if (!rs.fold) CIP_TRY(cone_scale_panel(rs.cd, rs.Fi, rs.At4r, rs.Atil4r, rs.nJ_pad, rs.nr_pad, rs.nJ, s));
   }
   CIP_CUDA(cudaEventRecord(h->ev[1], s));
+  // row_structure = 2 forms H_KK (J mapped to K positions) and h on D; the SYRK writes H directly when its columns
+  // are all of H's (J == K, or J every column)
+  RowStructure::Split& sp = rs.sp;
+  double* H = sp.on ? sp.HK4 : h->H4;
+  const int ldH = sp.on ? sp.nK_pad : h->n_pad;
+  const double* base = sp.on ? sp.BaseK4 : rs.Base4;
+  const int* Jmap = sp.on ? sp.JK : rs.J;
+  const bool direct = sp.on ? rs.nJ == sp.nK : !rs.compressed;
   if (rs.nJ > 0) {
     GemmArgs a{};
     a.lower = 1; a.ntm = a.ntn = rs.nJ_pad / TILE; a.sym = 1; a.nk = rs.nr_pad / 32;
-    a.Cin = rs.compressed ? nullptr : rs.Base4;
-    a.Cout = rs.compressed ? rs.Hr4 : h->H4;
+    a.Cin = direct ? base : nullptr;
+    a.Cout = direct ? H : rs.Hr4;
     a.ldc = rs.nJ_pad; a.alpha = 1.0;
     a.ws = h->gemm_ws; a.ws_doubles = GEMM_WS_DOUBLES;
     if (rs.fold) a.kscale = rs.Fi.a;
     CIP_TRY(launch_gemm_nt(rs.map, rs.map, a, s));
   }
-  if (rs.nJ == 0 || rs.compressed) CIP_TRY(vec_copy(h->H4, rs.Base4, nn, s));
-  if (rs.nJ > 0 && rs.compressed) {
+  if ((rs.nJ == 0 || !direct) && ldH > 0) CIP_TRY(vec_copy(H, base, (size_t)ldH * ldH, s));
+  if (rs.nJ > 0 && !direct) {
     dim3 grid(nb(rs.nJ, 128), (unsigned)std::min(rs.nJ, 65535));
-    scatter_gram_kernel<<<grid, 128, 0, s>>>(h->H4, h->n_pad, rs.Hr4, rs.nJ_pad, rs.J, rs.nJ);
+    scatter_gram_kernel<<<grid, 128, 0, s>>>(H, ldH, rs.Hr4, rs.nJ_pad, Jmap, rs.nJ);
     CIP_CHECK_LAUNCH();
   }
+  if (sp.on) {
+    CIP_TRY(vec_copy(sp.hD, sp.qD, h->n, s));
+    sp.factored = false;
+  }
   if (rs.nsing > 0) {
-    singleton_diag_kernel<<<nb(h->n, 128), 128, 0, s>>>(h->H4, h->n_pad, h->n, rs.sing_ptr, rs.sing_row, rs.sing_val,
-                                                        h->Fi.a);
+    singleton_diag_kernel<<<nb(h->n, 128), 128, 0, s>>>(H, ldH, h->n, rs.sing_ptr, rs.sing_row, rs.sing_val,
+                                                        h->Fi.a, sp.on ? sp.Kpos : nullptr, sp.hD);
     CIP_CHECK_LAUNCH();
   }
   CIP_CUDA(cudaEventRecord(h->ev[2], s));
@@ -615,6 +643,419 @@ int structure_A2(cip_engine* h, double* outa, double* outb, const double* ya, co
   finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(outa, rest ? rs.outr[0] : nullptr, rs.row_code, rs.sing_col, rs.sing_val, ya, h->m);
   CIP_CHECK_LAUNCH();
   finish_a_kernel<<<nb(h->m, 256), 256, 0, s>>>(outb, rest ? rs.outr[1] : nullptr, rs.row_code, rs.sing_col, rs.sing_val, yb, h->m);
+  CIP_CHECK_LAUNCH();
+  return 0;
+}
+
+
+// ================================================================ row_structure = 2: H split into D and K
+// With the rows classified as above, column j of H = Q + (F^-T A)'(F^-T A) + rho G'G + delta I holds more than its
+// diagonal only when a rest row touches it (j in J), when Q has an off-diagonal non-zero in row or column j, or when
+// rho > 0 and G has a non-zero in column j.  Those columns are K (ascending); the others are D, where H_jj = h_j =
+// Q_jj + the singleton sum + delta.  The Cholesky factor in natural column order is then sqrt(h_j) on D and the
+// factor of the dense H_KK on K, with no permutation.  The Schur complement on G becomes
+//   S = Sbase + G_D diag(1/h) G_D' + Z_K Z_K',   Z_K = G_K L_KK^-T,
+// and a solve with H is u = rhs / h on D plus the two sweeps on K.  No n_pad^2 buffer survives cip_create; dense Q
+// input is packed into a transient n_pad^2 staging copy, classified and gathered from it, then freed.
+namespace {
+
+// flagK[k] = 1 (and flagR[r] = 1) for every non-zero X[r, k], r < R, k < Kc; with flagR, diagonal entries are skipped
+__global__ void mark_nz_kernel(const double* __restrict__ X, int ld, int R, int Kc, int* flagR, int* flagK) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= R) return;
+  for (int k = blockIdx.y; k < Kc; k += gridDim.y) {
+    if (flagR && r == k) continue;
+    if (X[q4_index(r, k, ld)] != 0.0) {
+      flagK[k] = 1;
+      if (flagR) flagR[r] = 1;
+    }
+  }
+}
+
+__global__ void get_diag_kernel(double* __restrict__ d, const double* __restrict__ X, int ld, int n) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n) d[j] = X[q4_index(j, j, ld)];
+}
+
+// Y[a, b] = X[rmap[a], cmap[b]] for a < R, b < Kc   (Q_KK from the staging Q; G_K from G4 with rmap = nullptr)
+__global__ void gather_q4_kernel(double* __restrict__ Y, int ldy, const double* __restrict__ X, int ldx,
+                                 const int* __restrict__ rmap, int R, const int* __restrict__ cmap, int Kc) {
+  const int a = blockIdx.x * blockDim.x + threadIdx.x;
+  if (a >= R) return;
+  const int ga = rmap ? rmap[a] : a;
+  for (int b = blockIdx.y; b < Kc; b += gridDim.y) Y[q4_index(a, b, ldy)] = X[q4_index(ga, cmap[b], ldx)];
+}
+
+__global__ void shift_kernel(double* __restrict__ x, int n, double v) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j < n) x[j] += v;
+}
+
+// the pivots of D: kscale_j = h_j^-1/2 on D, 0 on K and the padding; *fail = min over the D columns with
+// h_j <= 0 or NaN
+__global__ void split_pivots_kernel(double* __restrict__ kscale, const double* __restrict__ hD,
+                                    const int* __restrict__ Kpos, int n, int n_pad, int* fail) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n_pad) return;
+  double ks = 0.0;
+  if (j < n && Kpos[j] < 0) {
+    const double hj = hD[j];
+    if (hj > 0.0) ks = 1.0 / sqrt(hj);
+    else atomicMin(fail, j);
+  }
+  kscale[j] = ks;
+}
+
+// rhsK[Kpos[j]] = rhs[j] on K; u = rhs / h on D, 0 on K
+__global__ void split_rhs_kernel(double* __restrict__ rK, double* __restrict__ u, const double* __restrict__ rhs,
+                                 const int* __restrict__ Kpos, const double* __restrict__ hD, int n) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  const int k = Kpos[j];
+  if (k >= 0) {
+    rK[k] = rhs[j];
+    u[j] = 0.0;
+  } else {
+    u[j] = rhs[j] / hD[j];
+  }
+}
+
+// dy = dyK on K; u - g / h on D (u without g)
+__global__ void split_join_kernel(double* __restrict__ dy, const double* __restrict__ dyK,
+                                  const double* __restrict__ u, const double* __restrict__ g,
+                                  const int* __restrict__ Kpos, const double* __restrict__ hD, int n) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  const int k = Kpos[j];
+  dy[j] = k >= 0 ? dyK[k] : (g ? u[j] - g[j] / hD[j] : u[j]);
+}
+
+// y = yK on K, d .* x on D
+__global__ void diag_join_kernel(double* __restrict__ y, const double* __restrict__ yK, const double* __restrict__ d,
+                                 const double* __restrict__ x, const int* __restrict__ Kpos, int n) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= n) return;
+  const int k = Kpos[j];
+  y[j] = k >= 0 ? yK[k] : d[j] * x[j];
+}
+
+// out (n x n, column-major) = H_KK (or L_KK) at K x K, h_j (or sqrt(h_j)) on the diagonal of D, 0 elsewhere
+__global__ void split_unpack_kernel(double* __restrict__ out, int n, const double* __restrict__ HK4, int ldk,
+                                    const int* __restrict__ Kpos, const double* __restrict__ hD, int factored) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const int a = Kpos[r];
+  for (int c = blockIdx.y; c < n; c += gridDim.y) {
+    const int b = Kpos[c];
+    double v = 0.0;
+    if (a >= 0 && b >= 0) v = HK4[q4_index(a, b, ldk)];
+    else if (r == c) v = factored ? sqrt(hD[r]) : hD[r];
+    out[r + (size_t)c * n] = v;
+  }
+}
+
+int count(const std::vector<char>& f) {
+  int c = 0;
+  for (char x : f) c += x != 0;
+  return c;
+}
+
+// flags of a Q4 matrix on the device (see mark_nz_kernel) copied to the host
+int mark_nz(cip_engine* h, const double* X, int ld, int R, int Kc, bool sym, std::vector<char>* out) {
+  cudaStream_t s = h->stream;
+  int* d = nullptr;
+  CIP_CUDA(cudaMalloc(&d, sizeof(int) * std::max(Kc, 1)));
+  CIP_CUDA(cudaMemsetAsync(d, 0, sizeof(int) * std::max(Kc, 1), s));
+  dim3 grid(nb(R, 128), (unsigned)std::min(std::max(Kc, 1), 65535));
+  mark_nz_kernel<<<grid, 128, 0, s>>>(X, ld, R, Kc, sym ? d : nullptr, d);
+  const cudaError_t le = cudaGetLastError();
+  g_launches++;
+  std::vector<int> f(Kc);
+  cudaMemcpyAsync(f.data(), d, sizeof(int) * Kc, cudaMemcpyDeviceToHost, s);
+  const cudaError_t se = cudaStreamSynchronize(s);
+  cudaFree(d);
+  CIP_CUDA(le);
+  CIP_CUDA(se);
+  out->assign(f.begin(), f.end());
+  return 0;
+}
+
+}  // namespace
+
+int split_classify_csc_Q(cip_engine* h, const cip_csc* Q) {
+  RowStructure::Split& sp = h->rs.sp;
+  const int n = h->n;
+  std::vector<E> ent;
+  CIP_TRY(read_csc(Q, n, &ent));
+  sp.q_couple.assign(n, 0);
+  std::vector<double> qd(n, 0.0);
+  for (const E& e : ent) {
+    if (e.i == e.j) {
+      qd[e.j] = e.v;
+    } else {
+      sp.q_couple[e.i] = 1;
+      sp.q_couple[e.j] = 1;
+    }
+  }
+  CIP_TRY(salloc(h, &sp.qD, (size_t)h->n_pad + 4));
+  CIP_CUDA(cudaMemcpyAsync(sp.qD, qd.data(), sizeof(double) * n, cudaMemcpyHostToDevice, h->stream));
+  CIP_CUDA(cudaStreamSynchronize(h->stream));
+  // Q_KK is scattered from these once K is known (K also holds columns Q does not couple: their diagonal is needed)
+  sp.qtrip.clear();
+  for (const E& e : ent)
+    if (e.i == e.j || (sp.q_couple[e.i] && sp.q_couple[e.j])) sp.qtrip.push_back({e.i, e.j, e.v});
+  return 0;
+}
+
+int split_diag_Q(cip_engine* h, const double* q) {
+  RowStructure::Split& sp = h->rs.sp;
+  sp.q_couple.assign(h->n, 0);
+  CIP_TRY(salloc(h, &sp.qD, (size_t)h->n_pad + 4));
+  if (q) {
+    CIP_CUDA(cudaMemcpyAsync(sp.qD, q, sizeof(double) * h->n, cudaMemcpyDefault, h->stream));
+    CIP_CUDA(cudaStreamSynchronize(h->stream));
+  }
+  return 0;
+}
+
+int split_build(cip_engine* h) {
+  RowStructure& rs = h->rs;
+  RowStructure::Split& sp = rs.sp;
+  cudaStream_t s = h->stream;
+  const int n = h->n, p = h->p;
+  // ---- K
+  std::vector<char> inK(n, 0);
+  std::vector<int> J(rs.nJ);
+  if (rs.nJ > 0) CIP_CUDA(cudaMemcpy(J.data(), rs.J, sizeof(int) * rs.nJ, cudaMemcpyDeviceToHost));
+  for (int j : J) inK[j] = 1;
+  sp.from_rest = rs.nJ;
+  if (h->Qq4) {       // dense Q: classified from the staging copy
+    CIP_TRY(mark_nz(h, h->Qq4, h->n_pad, n, n, true, &sp.q_couple));
+    CIP_TRY(salloc(h, &sp.qD, (size_t)h->n_pad + 4));
+    get_diag_kernel<<<nb(n, 256), 256, 0, s>>>(sp.qD, h->Qq4, h->n_pad, n);
+    CIP_CHECK_LAUNCH();
+  }
+  if (sp.q_couple.empty()) sp.q_couple.assign(n, 0);
+  if (!sp.qD) CIP_TRY(salloc(h, &sp.qD, (size_t)h->n_pad + 4));      // no Q
+  sp.from_Q = count(sp.q_couple);
+  for (int j = 0; j < n; ++j) inK[j] |= sp.q_couple[j];
+  std::vector<char> gcol(n, 0);
+  if (p > 0) CIP_TRY(mark_nz(h, h->G4, h->p_pad, p, n, false, &gcol));
+  if (h->aug_rows > 0) {
+    sp.from_G = count(gcol);
+    for (int j = 0; j < n; ++j) inK[j] |= gcol[j];
+  }
+  sp.K.clear();
+  std::vector<int> Kpos(n, -1);
+  sp.g_in_D = false;
+  for (int j = 0; j < n; ++j) {
+    if (inK[j]) {
+      Kpos[j] = (int)sp.K.size();
+      sp.K.push_back(j);
+    } else if (gcol[j]) {
+      sp.g_in_D = true;
+    }
+  }
+  sp.nK = (int)sp.K.size();
+  sp.nK_pad = round_up(sp.nK, TILE);
+  std::vector<int> JK(rs.nJ);
+  for (int a = 0; a < rs.nJ; ++a) JK[a] = Kpos[J[a]];
+  CIP_TRY(supload(h, &sp.dK, sp.K));
+  CIP_TRY(supload(h, &sp.Kpos, Kpos));
+  CIP_TRY(supload(h, &sp.JK, JK));
+  CIP_TRY(salloc(h, &sp.hD, (size_t)h->n_pad + 4));
+  CIP_TRY(salloc(h, &sp.kscale, (size_t)h->n_pad + 4));
+  CIP_TRY(salloc(h, &sp.fail, 1));
+  if (p > 0) CIP_TRY(make_q4_tensor_map(&sp.mapG.map, h->G4, h->p_pad, h->n_pad / 4));
+  const int nK = sp.nK, nKp = sp.nK_pad;
+  if (nK > 0) {
+    // ---- Q_KK (both triangles, identity on the padding)
+    const size_t kk = (size_t)nKp * nKp;
+    CIP_TRY(salloc(h, &sp.QK4, kk));
+    if (h->Qq4) {
+      dim3 grid(nb(nK, 128), (unsigned)std::min(nK, 65535));
+      gather_q4_kernel<<<grid, 128, 0, s>>>(sp.QK4, nKp, h->Qq4, h->n_pad, sp.dK, nK, sp.dK, nK);
+      CIP_CHECK_LAUNCH();
+    } else if (!sp.qtrip.empty()) {
+      // CSC Q: the summed entries of K x K as a CSC matrix over K positions
+      std::vector<long long> cp(nK + 1, 0), rv;
+      std::vector<double> nz;
+      for (const auto& e : sp.qtrip)
+        if (Kpos[e.i] >= 0 && Kpos[e.j] >= 0) cp[Kpos[e.j] + 1]++;
+      for (int a = 0; a < nK; ++a) cp[a + 1] += cp[a];
+      rv.resize(cp[nK]);
+      nz.resize(cp[nK]);
+      std::vector<long long> pos(cp.begin(), cp.end() - 1);
+      for (const auto& e : sp.qtrip) {
+        if (Kpos[e.i] < 0 || Kpos[e.j] < 0) continue;
+        const long long at = pos[Kpos[e.j]]++;
+        rv[at] = Kpos[e.i];
+        nz[at] = e.v;
+      }
+      const long long nnz = (long long)rv.size();
+      if (nnz > 0) {
+        long long *dcp = nullptr, *drv = nullptr;
+        double* dnz = nullptr;
+        int* dbad = nullptr;
+        CIP_CUDA(cudaMalloc(&dcp, cp.size() * 8));
+        CIP_CUDA(cudaMalloc(&drv, nnz * 8));
+        CIP_CUDA(cudaMalloc(&dnz, nnz * 8));
+        CIP_CUDA(cudaMalloc(&dbad, sizeof(int)));
+        cudaMemcpyAsync(dcp, cp.data(), cp.size() * 8, cudaMemcpyHostToDevice, s);
+        cudaMemcpyAsync(drv, rv.data(), nnz * 8, cudaMemcpyHostToDevice, s);
+        cudaMemcpyAsync(dnz, nz.data(), nnz * 8, cudaMemcpyHostToDevice, s);
+        cudaMemsetAsync(dbad, 0, sizeof(int), s);
+        const int r = scatter_csc_q4(sp.QK4, nKp, nK, dcp, drv, dnz, 0, 0, nK, nnz, dbad, s);
+        const cudaError_t se = cudaStreamSynchronize(s);
+        cudaFree(dcp); cudaFree(drv); cudaFree(dnz); cudaFree(dbad);
+        CIP_TRY(r);
+        CIP_CUDA(se);
+      }
+    } else {
+      // diagonal or no Q: Q_KK is the diagonal of Q on K
+      double* t = nullptr;
+      CIP_CUDA(cudaMalloc(&t, sizeof(double) * nK));
+      gather_vec_kernel<<<nb(nK, 256), 256, 0, s>>>(t, sp.qD, sp.dK, nK);
+      const cudaError_t le = cudaGetLastError();
+      g_launches++;
+      const int r = le == cudaSuccess ? set_diag_vec_q4(sp.QK4, nKp, nK, t, s) : 0;
+      const cudaError_t se = cudaStreamSynchronize(s);
+      cudaFree(t);
+      CIP_CUDA(le);
+      CIP_TRY(r);
+      CIP_CUDA(se);
+    }
+    CIP_TRY(add_diag_q4(sp.QK4, nKp, nK, nKp, 1.0, 1, s));
+    // ---- G_K and BaseK4 = Q_KK + rho G_K'G_K
+    if (p > 0) {
+      CIP_TRY(salloc(h, &sp.GK4, (size_t)h->p_pad * nKp));
+      dim3 grid(nb(p, 128), (unsigned)std::min(nK, 65535));
+      gather_q4_kernel<<<grid, 128, 0, s>>>(sp.GK4, h->p_pad, h->G4, h->p_pad, nullptr, p, sp.dK, nK);
+      CIP_CHECK_LAUNCH();
+      CIP_TRY(salloc(h, &sp.ZK4, (size_t)h->p_pad * nKp));
+      CIP_TRY(make_q4_tensor_map(&sp.mapZK.map, sp.ZK4, h->p_pad, nKp / 4));
+    }
+    if (rs.base_has_gtg) {
+      double* Gt4 = nullptr;
+      CIP_CUDA(cudaMalloc(&Gt4, (size_t)h->aug_rows * nKp * sizeof(double)));
+      CIP_CUDA(cudaMemsetAsync(Gt4, 0, (size_t)h->aug_rows * nKp * sizeof(double), s));
+      CIP_TRY(salloc(h, &sp.BaseK4, kk));
+      int rc = transpose_scale_q4(Gt4, nKp, 0, sp.GK4, h->p_pad, p, nK, sqrt(h->aug_rho), s);
+      GemmOperand g{};
+      if (rc == 0) rc = make_q4_tensor_map(&g.map, Gt4, nKp, h->aug_rows / 4);
+      if (rc == 0) {
+        GemmArgs a{};
+        a.lower = 1; a.ntm = a.ntn = nKp / TILE; a.sym = 1; a.nk = h->aug_rows / 32;
+        a.Cin = sp.QK4; a.Cout = sp.BaseK4; a.ldc = nKp; a.alpha = 1.0;
+        a.ws = h->gemm_ws; a.ws_doubles = GEMM_WS_DOUBLES;
+        rc = launch_gemm_nt(g, g, a, s);
+      }
+      const cudaError_t se = cudaStreamSynchronize(s);
+      cudaFree(Gt4);
+      CIP_TRY(rc);
+      CIP_CUDA(se);
+    } else {
+      sp.BaseK4 = sp.QK4;
+    }
+    // ---- H_KK and its Cholesky plan
+    CIP_TRY(salloc(h, &sp.HK4, kk));
+    CIP_TRY(salloc(h, &sp.WinvK, (size_t)nKp * TILE));
+    CIP_TRY(chol_make_plan(&sp.chol, sp.HK4, nKp, sp.WinvK, h->info));
+    for (int b = 0; b < 2; ++b)
+      for (auto& v : sp.kv[b]) CIP_TRY(salloc(h, &v, (size_t)nKp + 4));
+  }
+  sp.qtrip.clear();
+  sp.qtrip.shrink_to_fit();
+  // the Gram scratch is not needed when the SYRK writes H_KK directly (J == K)
+  if (rs.Hr4 && rs.nJ == nK) {
+    CIP_CUDA(cudaStreamSynchronize(s));
+    cudaFree(rs.Hr4);
+    h->owned.erase(std::find(h->owned.begin(), h->owned.end(), (void*)rs.Hr4));
+    h->bytes -= std::max<size_t>((size_t)rs.nJ_pad * rs.nJ_pad, 1) * sizeof(double);
+    rs.Hr4 = nullptr;
+  }
+  if (h->Qq4) {       // the dense staging copy of Q
+    CIP_CUDA(cudaStreamSynchronize(s));
+    cudaFree(h->Qq4);
+    h->Qq4 = nullptr;
+    h->bytes -= (size_t)h->n_pad * h->n_pad * sizeof(double);
+  }
+  return 0;
+}
+
+int split_add_delta(cip_engine* h, double delta) {
+  RowStructure::Split& sp = h->rs.sp;
+  if (sp.nK > 0) CIP_TRY(add_diag_q4(sp.HK4, sp.nK_pad, 0, sp.nK, delta, 0, h->stream));
+  shift_kernel<<<nb(h->n, 256), 256, 0, h->stream>>>(sp.hD, h->n, delta);
+  CIP_CHECK_LAUNCH();
+  return 0;
+}
+
+int split_factor(cip_engine* h) {
+  RowStructure::Split& sp = h->rs.sp;
+  cudaStream_t s = h->stream;
+  CIP_CUDA(cudaMemsetAsync(sp.fail, 0x7f, sizeof(int), s));     // 0x7f7f7f7f: no failing D column
+  if (sp.nK > 0) CIP_TRY(chol_factor(sp.chol, s));
+  split_pivots_kernel<<<nb(h->n_pad, 256), 256, 0, s>>>(sp.kscale, sp.hD, sp.Kpos, h->n, h->n_pad, sp.fail);
+  CIP_CHECK_LAUNCH();
+  sp.factored = true;
+  return 0;
+}
+
+int split_solve(cip_engine* h, double** nv, double** pv, int b, bool schur) {
+  RowStructure::Split& sp = h->rs.sp;
+  cudaStream_t s = h->stream;
+  const int n = h->n, p = h->p, nK = sp.nK;
+  double *rK = sp.kv[b][0], *tK = sp.kv[b][1], *wK = sp.kv[b][2];
+  double* u = nv[3];
+  split_rhs_kernel<<<nb(n, 256), 256, 0, s>>>(rK, u, nv[2], sp.Kpos, sp.hD, n);
+  CIP_CHECK_LAUNCH();
+  if (nK > 0) CIP_TRY(chol_fwd(sp.chol, rK, tK, s));
+  const double* g = nullptr;
+  if (schur) {
+    // r = G u + Z_K t_K - rw;  dw = S^-1 r;  t_K -= Z_K' dw;  g = G' dw
+    if (nK > 0) CIP_TRY(q4_mv_rows(pv[1], sp.ZK4, h->p_pad, p, nK, tK, h->partial, h->partial_cap, s));
+    else CIP_TRY(fill_zero(pv[1], p, s));
+    if (sp.g_in_D) {
+      CIP_TRY(q4_mv_rows(pv[3], h->G4, h->p_pad, p, n, u, h->partial, h->partial_cap, s));
+      CIP_TRY(vec_axpby(pv[1], 1.0, pv[1], 1.0, pv[3], p, s));
+    }
+    CIP_TRY(vec_axpby(pv[2], 1.0, pv[1], -1.0, pv[0], p, s));
+    CIP_TRY(chol_fwd(h->cholS, pv[2], pv[3], s));
+    CIP_TRY(chol_bwd(h->cholS, pv[3], pv[4], s));
+    if (nK > 0) {
+      CIP_TRY(q4_mv_k(wK, sp.ZK4, h->p_pad, p, nK, pv[4], s));
+      CIP_TRY(vec_axpby(tK, 1.0, tK, -1.0, wK, nK, s));
+    }
+    if (sp.g_in_D) {
+      CIP_TRY(q4_mv_k(nv[4], h->G4, h->p_pad, p, n, pv[4], s));
+      g = nv[4];
+    }
+  }
+  if (nK > 0) CIP_TRY(chol_bwd(sp.chol, tK, rK, s));
+  split_join_kernel<<<nb(n, 256), 256, 0, s>>>(nv[5], rK, u, g, sp.Kpos, sp.hD, n);
+  CIP_CHECK_LAUNCH();
+  return 0;
+}
+
+int split_mul_Q(cip_engine* h, double* y, const double* x) {
+  RowStructure::Split& sp = h->rs.sp;
+  cudaStream_t s = h->stream;
+  const int nK = sp.nK;
+  if (nK > 0) {
+    gather_vec_kernel<<<nb(nK, 256), 256, 0, s>>>(sp.kv[0][0], x, sp.dK, nK);
+    CIP_CHECK_LAUNCH();
+    CIP_TRY(q4_mv_rows(sp.kv[0][1], sp.QK4, sp.nK_pad, nK, nK, sp.kv[0][0], h->partial, h->partial_cap, s));
+  }
+  diag_join_kernel<<<nb(h->n, 256), 256, 0, s>>>(y, sp.kv[0][1], sp.qD, x, sp.Kpos, h->n);
+  CIP_CHECK_LAUNCH();
+  return 0;
+}
+
+int split_get_H(cip_engine* h, double* out) {
+  RowStructure::Split& sp = h->rs.sp;
+  dim3 grid(nb(h->n, 128), (unsigned)std::min(h->n, 65535));
+  split_unpack_kernel<<<grid, 128, 0, h->stream>>>(out, h->n, sp.HK4, sp.nK_pad, sp.Kpos, sp.hD, sp.factored);
   CIP_CHECK_LAUNCH();
   return 0;
 }

@@ -67,7 +67,8 @@ def conicIP_native(Q, c, A, b, cone_dims, G=None, d=None, *, engine=None, ngpus=
     """Same problem statement and options as `conicIP`, but the loop itself runs inside the library
     (`cip_ipm_solve`, SURVEY 8f rank 1): one C call per solve.  Pass `engine=` to reuse a handle;
     `ngpus > 1` row-shards A over that many devices of this process (`cip_options.ngpus`);
-    `row_structure=1` exploits the row structure of A when forming H (`cip_options.row_structure`)."""
+    `row_structure=1` exploits the row structure of A when forming H (`cip_options.row_structure`);
+    `row_structure=2` also factors H as its diagonal plus the coupled block, with no n x n buffer."""
     from .engine import Engine
     eng = engine or Engine(Q, A, G if (G is not None and G.shape[0]) else None, cone_dims, ngpus=ngpus,
                            row_structure=row_structure)

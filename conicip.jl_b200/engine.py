@@ -54,7 +54,8 @@ class Engine:
         opts.aug_rho = aug_rho
         opts.ngpus = int(ngpus)            # > 1: single-process multi-GPU handle (global vectors in and out)
         opts.fold_scaling = int(fold_scaling)   # 0 auto, 1 always, 2 never (R-only problems: no Atil copy of A)
-        opts.row_structure = int(row_structure)  # 1: singleton R rows on the diagonal, compact SYRK for the rest
+        opts.row_structure = int(row_structure)  # 1: singleton R rows on the diagonal, compact SYRK for the rest;
+        #                                          2: also factor H as its diagonal plus the coupled block H_KK
         self.ngpus = max(1, int(ngpus))
         self._torch = None
         self._use_torch_stream = use_torch_stream
@@ -414,6 +415,14 @@ class Engine:
         si.struct_size = C.sizeof(StructureInfo)
         check(lib().cip_structure_info(self._h, C.byref(si)))
         return {k: getattr(si, k) for k, _ in StructureInfo._fields_ if k != "struct_size"}
+
+    def split_info(self):
+        """How `row_structure=2` split the columns of H (`cip_split_info`); all zero otherwise."""
+        from ._lib import SplitInfo
+        si = SplitInfo()
+        si.struct_size = C.sizeof(SplitInfo)
+        check(lib().cip_split_info(self._h, C.byref(si)))
+        return {k: getattr(si, k) for k, _ in SplitInfo._fields_ if k != "struct_size"}
 
     def get_H(self):
         out = np.zeros((self.n, self.n), order="F")

@@ -32,7 +32,8 @@ struct Options            # mirrors cip_options
     aug_rho::Cdouble
     ngpus::Cint           # > 1: this one process drives that many GPUs behind the handle (rows of A sliced on cone boundaries)
     fold_scaling::Cint    # 0 auto, 1 always, 2 never: R-only problems without a second (scaled) copy of A
-    row_structure::Cint   # 1: singleton R rows go onto the diagonal of H, the SYRK runs on the other rows (one GPU)
+    row_structure::Cint   # 1: singleton R rows go onto the diagonal of H, the SYRK runs on the other rows (one GPU);
+                          # 2: also factor H as its diagonal plus the coupled block H_KK (no n x n buffer)
 end
 make_options(; device = -1, reg_delta = 0.0, q_kind = 0, ngpus = 1, fold_scaling = 0, row_structure = 0) =
     Options(Cint(sizeof(Options)), Cint(device), reg_delta, 0.0, Cint(q_kind), Cint(0), Cint(-1), -1.0, Cint(ngpus),
@@ -193,6 +194,28 @@ How an engine created with `row_structure = 1` split the rows of `A` (`cip_struc
 function structure_info(eng::Engine)
     r = Ref(StructureInfo(Cint(sizeof(StructureInfo)), 0, 0, 0, 0, 0, 0, 0))
     check(ccall((:cip_structure_info, LIB), Cint, (Ptr{Cvoid}, Ref{StructureInfo}), eng.h, r))
+    return r[]
+end
+struct SplitInfo          # mirrors cip_split_t
+    struct_size::Cint
+    enabled::Cint
+    coupled_cols::Cint
+    diagonal_cols::Cint
+    cols_from_rest::Cint
+    cols_from_Q::Cint
+    cols_from_G::Cint
+end
+"""
+    split_info(eng) -> SplitInfo
+
+How an engine created with `row_structure = 2` split the columns of `H` (`cip_split_info`): `coupled_cols` columns
+form the dense block `H_KK`, `diagonal_cols` hold only their diagonal.  `cols_from_rest`, `cols_from_Q` and
+`cols_from_G` count why a column is coupled (a rest row of `A`, an off-diagonal entry of `Q`, `G` when
+`aug_rho > 0`); the sets overlap.  All zero for other engines.
+"""
+function split_info(eng::Engine)
+    r = Ref(SplitInfo(Cint(sizeof(SplitInfo)), 0, 0, 0, 0, 0, 0))
+    check(ccall((:cip_split_info, LIB), Cint, (Ptr{Cvoid}, Ref{SplitInfo}), eng.h, r))
     return r[]
 end
 """

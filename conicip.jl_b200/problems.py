@@ -253,3 +253,40 @@ def config5(n=20000, k=64, p=1000, seed=5):
     w0 = rng.standard_normal(p)
     c = G.T @ w0 - A.T @ v0                          # stationarity (src/ConicIP.jl:747,753): Qy + G'w - A'v = c
     return _prob("C5", np.zeros((n, n)), c, A, b, [("R", n), ("S", dim)], G, d, optTol=1e-8)
+
+
+def config5_sparse(n=20000, k=64, p=1000, seed=5):
+    """C5 built directly in sparse form: A and G as scipy CSC, Q as an empty CSC matrix.  It consumes the same
+    random stream as config5, so at equal arguments it is the same problem; it never forms a dense n-wide matrix, so
+    it reaches shapes (n = 150 000) where config5's dense A alone would not fit in host memory."""
+    rng = np.random.default_rng(seed)
+    dim = k * (k + 1) // 2
+    m = n + dim
+    A = sp.csc_matrix((np.ones(n + dim), (np.arange(m), np.concatenate([np.arange(n), np.arange(dim)]))),
+                      shape=(m, n))
+    B = rng.standard_normal((k, k)) / np.sqrt(k)
+    X0 = B @ B.T + 0.5 * np.eye(k)
+    y0 = rng.uniform(0.5, 1.5, n)
+    y0[:dim] = np.abs(_svec(X0)) + 0.05
+    Xs = _smat(y0[:dim])
+    Xs += (0.1 - min(0.0, np.linalg.eigvalsh(Xs).min())) * np.eye(k)
+    y0[:dim] = _svec(Xs)
+    assert np.linalg.eigvalsh(_smat(y0[:dim])).min() > 0 and y0.min() > 0
+    b = np.zeros(m)
+    rows, cols, vals = [], [], []
+    for i in range(p):
+        vals.append(rng.standard_normal(min(10, n)))     # config5's `G[i, choice] = normal` draws the values first
+        cols.append(rng.choice(n, min(10, n), replace=False))
+        rows.append(np.full(min(10, n), i))
+    if p > 0:
+        G = sp.csc_matrix((np.concatenate(vals), (np.concatenate(rows), np.concatenate(cols))), shape=(p, n))
+    else:
+        G = sp.csc_matrix((0, n))
+    d = G @ y0
+    v0 = np.zeros(m)
+    v0[:n] = rng.uniform(0.5, 1.5, n)
+    Bz = rng.standard_normal((k, k)) / np.sqrt(k)
+    v0[n:] = _svec(Bz @ Bz.T + 0.5 * np.eye(k))
+    w0 = rng.standard_normal(p)
+    c = G.T @ w0 - A.T @ v0
+    return _prob("C5", sp.csc_matrix((n, n)), c, A, b, [("R", n), ("S", dim)], G, d, optTol=1e-8)

@@ -76,7 +76,17 @@ typedef struct cip_options {
                            row and the R rows with >= 2 non-zeros) are kept in a compact copy of A that spans only
                            the columns they touch, and the constant Q + rho*G'G is formed once.  0 = off (default).
                            The environment variable CIP_ROW_STRUCTURE=1 turns it on for single-device handles.
-                           Sharded handles (ngpus > 1, cip_comm_init) reject it. */
+                           2 = the same row split, and the columns of H split too: K ("coupled") holds the columns
+                           a rest row touches, the columns where Q has an off-diagonal non-zero in the row or the
+                           column, and (resolved aug_rho > 0 and p > 0) the columns where G has a non-zero; D holds
+                           the others, where H has nothing but its diagonal.  H_KK is factored densely, D as
+                           sqrt(H_jj), the Schur complement gets G_D diag(1/H_jj) G_D' + Z_K Z_K'.  No n_pad x n_pad
+                           buffer remains after cip_create, so problems whose coupled columns are few can be solved
+                           at any n that fits the vectors, G and the rest rows of A (dense Q input still passes
+                           through one transient n_pad x n_pad staging copy; give Q as CSC, diagonal or NULL to
+                           avoid it).  cip_get_H scatters into n x n (zeros outside K x K and the diagonal); a
+                           failing pivot is still reported as 1 + its global column.  CIP_ROW_STRUCTURE=2 selects it.
+                           Sharded handles (ngpus > 1, cip_comm_init) reject 1 and 2. */
 } cip_options;
 
 typedef struct cip_stats_t {
@@ -237,10 +247,23 @@ typedef struct cip_structure_t {
   int empty_rows;       /* R rows without a non-zero                                                    */
   int rest_rows;        /* Q / S rows plus R rows with >= 2 non-zeros: the rows of the SYRK             */
   int rest_cols;        /* |J|: the columns the rest rows touch                                         */
-  int compressed;       /* 1: the SYRK runs on the columns J only (round_up(|J|,128) <= n_pad/2)       */
+  int compressed;       /* 1: the SYRK runs on the columns J only (round_up(|J|,128) <= n_pad/2; always
+                           with row_structure = 2)                                                      */
   int base_has_gtg;     /* 1: the constant part Q + rho*G'G was formed once at creation                 */
 } cip_structure_t;
 int cip_structure_info(cip_handle h, cip_structure_t* out);
+/* How a handle with cip_options.row_structure = 2 split the columns of H (all zero otherwise).  The three
+ * cols_from_* counts are of overlapping sets: a column can be coupled for more than one reason. */
+typedef struct cip_split_t {
+  int struct_size;      /* = sizeof(cip_split_t), set by the caller                                      */
+  int enabled;          /* 1: H is factored as a diagonal part plus its coupled block                      */
+  int coupled_cols;     /* |K|: columns of the dense block H_KK                                            */
+  int diagonal_cols;    /* |D| = n - |K|: columns where H holds only its diagonal                          */
+  int cols_from_rest;   /* columns touched by a rest row of A (|J| of cip_structure_t)                     */
+  int cols_from_Q;      /* columns with an off-diagonal non-zero of Q in their row or column               */
+  int cols_from_G;      /* columns where G has a non-zero, when aug_rho > 0 and p > 0 (else 0)             */
+} cip_split_t;
+int cip_split_info(cip_handle h, cip_split_t* out);
 /* copy the current reduced matrix H (after cip_factor: its Cholesky factor L in the
  * lower triangle) into a column-major n*n buffer -- test/debug hook */
 int cip_get_H(cip_handle h, double* out, int ldo);

@@ -1,12 +1,16 @@
-"""cip_options.row_structure on and off, alternating in one process: KKT unit time and its phases, resident bytes,
-time to 1e-8 through cip_ipm_solve, and how far the two modes' results are apart.
+"""cip_options.row_structure modes side by side, alternating in one process: KKT unit time and its phases, resident
+bytes, time to 1e-8 through cip_ipm_solve, and how far the modes' results are apart.
 
-    python scripts/structure_timing.py --out DIR [--units 5] [--warmup 2] [--only C5,C1,...]
+    python scripts/structure_timing.py --out DIR [--units 5] [--warmup 2] [--only C5,C1,...] [--modes 0,1]
 
 Workloads: C5 at full size through dense input and through a CSC copy of A, C1, a box QP (A = [I; -I], dense Q),
-and a dense R-only QP with n bound rows appended (C2 plus I: the rest stays full width).  A unit is what bench.py
-times: factor at an interior point (NT scaling, H, Cholesky, Schur complement) plus two solves.  Writes one JSON
-file per workload, r03_structure_<name>.json, into DIR."""
+and a dense R-only QP with n bound rows appended (C2 plus I: the rest stays full width).  With mode 2 among the
+modes (or when named in --only) also C5_rho0 (C5 with aug_rho = 0, so G couples no column) and C5_wide
+(config5_sparse at n = 150 000, CSC input, no Q, aug_rho = 0).  C5_wide runs in mode 2 only: modes 0 and 1 hold
+n_pad^2 doubles per H and Q, which the record computes from the shape instead of attempting.  A unit is what
+bench.py times: factor at an interior point (NT scaling, H, Cholesky, Schur complement) plus two solves.  Writes
+one JSON file per workload into DIR: r03_structure_<name>.json for the default modes 0,1 (keys "off" / "on"),
+r04_split_<name>.json otherwise (keys "mode<k>")."""
 import argparse
 import json
 import os
@@ -48,7 +52,7 @@ def interior(cone_dims, seed):
     return out
 
 
-def workloads(only):
+def workloads(only, modes):
     def c5():
         return P.config5()
 
@@ -74,7 +78,22 @@ def workloads(only):
         s0 = rng.uniform(0.1, 1.1, A.shape[0])
         return P._prob("C2_plus_bounds", base["Q"], base["c"], A, A @ y0 - s0, [("R", A.shape[0])], optTol=1e-8)
 
+    def c5_rho0():
+        p = P.config5()
+        p["engine_kw"] = dict(aug_rho=0.0)
+        return p
+
+    def c5_wide():
+        p = P.config5_sparse(n=150_000)
+        p["A_input"], p["Q"] = p["A"], None
+        p["engine_kw"] = dict(aug_rho=0.0)
+        p["modes"] = (2,)
+        return p
+
     table = {"C5": c5, "C5_csc": c5_csc, "C1": lambda: P.config1(), "box_qp": box, "C2_bounds": c2_bounds}
+    split_table = {"C5_rho0": c5_rho0, "C5_wide": c5_wide}
+    if 2 in modes or any(k in split_table for k in only):
+        table.update(split_table)
     return [(k, f) for k, f in table.items() if not only or k in only]
 
 
@@ -89,33 +108,39 @@ def unit(e, v, s, ry, rw, rv):
     return (time.perf_counter() - t0) * 1e3, ph, lam, d1, d2
 
 
-def run(name, make, units, warmup, out_dir, gpu):
+def run(name, make, units, warmup, out_dir, gpu, modes):
     prob = make()
     A = prob.get("A_input", prob["A"])
     G = prob["G"] if prob["G"].shape[0] else None
+    kw = prob.get("engine_kw", {})
+    # a workload that names its modes (C5_wide: 2 only) is too large for the others, whatever --modes asks for
+    skipped = [m for m in (0, 1, 2) if m not in prob["modes"]] if "modes" in prob else []
+    modes = tuple(m for m in modes if m in prob.get("modes", modes))
+    legacy = modes == (0, 1)
+    label = {0: "off", 1: "on"} if legacy else {m: f"mode{m}" for m in modes}
     t0 = time.perf_counter()
     eng = {}
     setup = {}
-    for mode in (0, 1):
+    for mode in modes:
         t = time.perf_counter()
-        eng[mode] = cb.Engine(prob["Q"], A, G, prob["cone_dims"], row_structure=mode)
+        eng[mode] = cb.Engine(prob["Q"], A, G, prob["cone_dims"], row_structure=mode, **kw)
         setup[mode] = time.perf_counter() - t
     gen_s = time.perf_counter() - t0
-    e1 = eng[1]
+    e1 = eng[modes[-1]]
     v, s = interior(prob["cone_dims"], 1)
     rng = np.random.default_rng(2)
     ry, rw, rv = rng.standard_normal(e1.n), rng.standard_normal(e1.p) if e1.p else None, rng.standard_normal(e1.m)
-    res = {m: {"unit_ms": [], "phases": []} for m in (0, 1)}
+    res = {m: {"unit_ms": [], "phases": []} for m in modes}
     outs = {}
     for it in range(warmup + units):
-        for mode in (0, 1):                       # alternate the two modes
+        for mode in modes:                        # alternate the modes
             ms, ph, lam, d1, d2 = unit(eng[mode], v, s, ry, rw, rv)
             outs[mode] = (lam, d1, d2)
             if it >= warmup:
                 res[mode]["unit_ms"].append(ms)
                 res[mode]["phases"].append(ph)
     summary = {}
-    for mode in (0, 1):
+    for mode in modes:
         r = res[mode]
         st = eng[mode].stats()
         summary[mode] = {
@@ -124,32 +149,45 @@ def run(name, make, units, warmup, out_dir, gpu):
             "syrk_flops": st["syrk_flops"], "device_bytes": int(st["device_bytes"]), "create_s": setup[mode],
             "structure": eng[mode].structure_info(),
         }
-    lam0, a0, b0 = outs[0]
-    lam1, a1, b1 = outs[1]
+        if mode == 2:
+            summary[mode]["split"] = eng[mode].split_info()
+    lo, hi = modes[0], modes[-1]
+    lam0, a0, b0 = outs[lo]
+    lam1, a1, b1 = outs[hi]
     diffs = {"lambda": rel(lam1, lam0), "dy": max(rel(a1[0], a0[0]), rel(b1[0], b0[0])),
              "dv": max(rel(a1[2], a0[2]), rel(b1[2], b0[2])),
              "dw": max(rel(a1[1], a0[1]), rel(b1[1], b0[1])) if e1.p else 0.0}
     full = {}
     sols = {}
-    for mode in (0, 1):
+    for mode in modes:
         t = time.perf_counter()
         y, w, vv, info = eng[mode].ipm_solve(prob["c"], prob["b"], prob["d"] if e1.p else None, optTol=1e-8)
         full[mode] = {"wall_s": time.perf_counter() - t, "seconds": info["seconds"], "status": info["status"],
                       "iterations": info["Iter"], "factors": info["factors"], "solves": info["solves"]}
         sols[mode] = (y, w, vv)
-    diffs.update({"full_y": rel(sols[1][0], sols[0][0]), "full_v": rel(sols[1][2], sols[0][2]),
-                  "full_w": rel(sols[1][1], sols[0][1]) if e1.p else 0.0})
+    diffs.update({"full_y": rel(sols[hi][0], sols[lo][0]), "full_v": rel(sols[hi][2], sols[lo][2]),
+                  "full_w": rel(sols[hi][1], sols[lo][1]) if e1.p else 0.0})
     for e in eng.values():
         e.close()
     rec = {"workload": name, "n": e1.n, "m": e1.m, "p": e1.p, "input": "csc" if "A_input" in prob else "dense",
-           "gpu": gpu, "units": units, "warmup": warmup, "setup_s": gen_s,
-           "off": {**summary[0], "full_solve": full[0]}, "on": {**summary[1], "full_solve": full[1]},
-           "max_rel_diff_on_vs_off": diffs,
-           "timer": "unit: host perf_counter around factor_from_point + 2 solves (host outputs: each call syncs); "
-                    "phases: CUDA events of cip_stats; full solve: cip_ipm_result.seconds"}
+           "gpu": gpu, "units": units, "warmup": warmup, "setup_s": gen_s}
+    if kw:
+        rec["engine_options"] = kw
+    for mode in modes:
+        rec[label[mode]] = {**summary[mode], "full_solve": full[mode]}
+    if len(modes) > 1:
+        rec["max_rel_diff_on_vs_off" if legacy else f"max_rel_diff_mode{hi}_vs_mode{lo}"] = diffs
+    if skipped:
+        n_pad = -(-e1.n // 128) * 128
+        rec["not_attempted"] = {f"mode{m}": f"computed from the shape, not run: needs n_pad^2 doubles for H and for Q, "
+                                            f"2 x {8 * n_pad * n_pad / 1e9:.0f} GB (n_pad = {n_pad}), more than the "
+                                            f"device holds" for m in skipped}
+    rec["timer"] = ("unit: host perf_counter around factor_from_point + 2 solves (host outputs: each call syncs); "
+                    "phases: CUDA events of cip_stats; full solve: cip_ipm_result.seconds")
     print(json.dumps(rec), flush=True)
     if out_dir:
-        with open(os.path.join(out_dir, f"r03_structure_{name}.json"), "w") as f:
+        fname = f"r03_structure_{name}.json" if legacy else f"r04_split_{name}.json"
+        with open(os.path.join(out_dir, fname), "w") as f:
             json.dump(rec, f, indent=1)
 
 
@@ -159,6 +197,7 @@ def main():
     ap.add_argument("--units", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=2)
     ap.add_argument("--only", default="")
+    ap.add_argument("--modes", default="0,1", help="row_structure modes to compare, e.g. 1,2")
     a = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -170,8 +209,9 @@ def main():
     if a.out:
         os.makedirs(a.out, exist_ok=True)
     only = [s for s in a.only.split(",") if s]
-    for name, make in workloads(only):
-        run(name, make, a.units, a.warmup, a.out, gpu)
+    modes = tuple(sorted({int(x) for x in a.modes.split(",") if x}))
+    for name, make in workloads(only, modes):
+        run(name, make, a.units, a.warmup, a.out, gpu, modes)
 
 
 if __name__ == "__main__":
