@@ -88,6 +88,43 @@ scale_panel_diag_kernel(const double* __restrict__ At4, double* __restrict__ Ati
     out[1] = v1;
   }
 }
+// The same pass for the fast SYRK (R rows only), which also needs the column norms of Atil: block (k chunk, 256
+// columns), a thread walks SCALE_KQ_CHUNK quads of one column and leaves its sum of squares in
+// colss[chunk * ld + j], which col_exponent_kernel reduces in a fixed order (deterministic).
+constexpr int SCALE_KQ_CHUNK = 256;
+__global__ void __launch_bounds__(256)
+scale_panel_diag_norms_kernel(const double* __restrict__ At4, double* __restrict__ Atil4, int ld, int kq_total,
+                              const double* __restrict__ ia, double* __restrict__ colss) {
+  const int j = blockIdx.y * blockDim.x + threadIdx.x;
+  const int kq0 = blockIdx.x * SCALE_KQ_CHUNK;
+  const int kq1 = min(kq0 + SCALE_KQ_CHUNK, kq_total);
+  double ss = 0.0;
+#pragma unroll 4
+  for (int kq = kq0; kq < kq1; ++kq) {
+    const double2 s0 = *reinterpret_cast<const double2*>(ia + 4 * kq);
+    const double2 s1 = *reinterpret_cast<const double2*>(ia + 4 * kq + 2);
+    const size_t at = ((size_t)kq * ld + j) * 4;
+    const double2* in = reinterpret_cast<const double2*>(At4 + at);
+    double2 v0 = __ldg(in), v1 = __ldg(in + 1);
+    v0.x *= s0.x; v0.y *= s0.y; v1.x *= s1.x; v1.y *= s1.y;
+    double2* out = reinterpret_cast<double2*>(Atil4 + at);
+    out[0] = v0;
+    out[1] = v1;
+    ss += v0.x * v0.x + v0.y * v0.y + v1.x * v1.x + v1.y * v1.y;
+  }
+  colss[(size_t)blockIdx.x * ld + j] = ss;
+}
+// e_j = round(log2 ||Atil[:, j]||), clamped to +-500 so that 2^-(e_i + e_j) stays a normal number (0 for a zero column)
+__global__ void __launch_bounds__(256)
+col_exponent_kernel(const double* __restrict__ colss, int nchunk, int ld, int* __restrict__ colexp) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= ld) return;
+  double ss = 0.0;
+  for (int c = 0; c < nchunk; ++c) ss += colss[(size_t)c * ld + j];
+  int e = 0;
+  if (ss > 0.0 && isfinite(ss)) e = max(-500, min(500, (int)lrint(0.5 * log2(ss))));
+  colexp[j] = e;
+}
 __global__ void __launch_bounds__(128)
 scale_panel_wood_kernel(ConeDesc c, Scaling Fi, const double* __restrict__ At4, double* __restrict__ Atil4,
                         int ld, int ncols) {
@@ -567,6 +604,25 @@ int cone_scale_panel(const ConeDesc& c, Scaling Fi, const double* At4, double* A
     CIP_CHECK_LAUNCH();
   }
   CIP_TRY(sdp_scale_panel(c, Fi, At4, Atil4, ld, ncols, st));
+  return 0;
+}
+
+int scale_panel_norms_chunks(int m_pad) { return (m_pad / 4 + SCALE_KQ_CHUNK - 1) / SCALE_KQ_CHUNK; }
+
+int cone_scale_panel_norms(Scaling Fi, const double* At4, double* Atil4, int ld, int m_pad, double* colss,
+                           int* colexp, cudaStream_t st) {
+  const int nchunk = scale_panel_norms_chunks(m_pad);
+  if (nchunk > 0) {
+    dim3 grid(nchunk, ld / 256 > 0 ? ld / 256 : 1);
+    if (ld % 256 != 0) {
+      set_error("cone_scale_panel_norms: ld = %d is not a multiple of 256", ld);
+      return -1;
+    }
+    scale_panel_diag_norms_kernel<<<grid, 256, 0, st>>>(At4, Atil4, ld, m_pad / 4, Fi.a, colss);
+    CIP_CHECK_LAUNCH();
+  }
+  col_exponent_kernel<<<(ld + 255) / 256, 256, 0, st>>>(colss, nchunk, ld, colexp);
+  CIP_CHECK_LAUNCH();
   return 0;
 }
 

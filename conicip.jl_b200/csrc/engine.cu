@@ -301,7 +301,9 @@ int form_H(cip_engine* h) {
     CIP_CUDA(cudaEventRecord(h->ev[3], s));
     return 0;
   }
-  if (h->m_pad > 0 && !h->fold) CIP_TRY(cone_scale_panel(h->cd, h->Fi, h->At4, h->Atil4, h->n_pad, h->m_pad, h->n, s));
+  const bool fast = h->fast.on && !h->comm;
+  if (fast) CIP_TRY(cone_scale_panel_norms(h->Fi, h->At4, h->Atil4, h->n_pad, h->m_pad, h->fast.colss, h->fast.colexp, s));
+  else if (h->m_pad > 0 && !h->fold) CIP_TRY(cone_scale_panel(h->cd, h->Fi, h->At4, h->Atil4, h->n_pad, h->m_pad, h->n, s));
   CIP_CUDA(cudaEventRecord(h->ev[1], s));
   const double* cin = (h->rank == 0) ? h->Qq4 : nullptr;
   // rows of Atil beyond m_pad hold sqrt(rho)*G (constant): H' = Q + Atil'Atil + rho G'G, added on rank 0 only
@@ -313,7 +315,9 @@ int form_H(cip_engine* h) {
     h->st.syrk_flops = (double)h->m * (double)h->n * (double)h->n;
     return 0;
   }
-  if (k_rows > 0) {
+  if (fast) {
+    CIP_TRY(fast_syrk_form(h, cin));       // sums, products, combination and the diagonal leaves: all inside ev[1..2]
+  } else if (k_rows > 0) {
     GemmArgs a{};
     a.lower = 1; a.ntm = a.ntn = h->n_pad / TILE; a.sym = 1;
     a.x_row0 = a.y_row0 = 0; a.x_kq0 = a.y_kq0 = 0; a.nk = k_rows / 32;
@@ -472,6 +476,7 @@ namespace cip {
 int engine_allreduce(cip_engine* h, double* buf, size_t count) { return allreduce(h, buf, count); }
 int engine_setup_comm(cip_engine* h) {
   if (!h->comm || h->Hp) return 0;
+  CIP_TRY(fast_syrk_drop(h));
   h->cholH.nranks_hint = h->nranks;        // the replicated fallback must schedule like the distributed one
   if (const char* env = getenv("CIP_OVERLAP_REDUCE")) if (atoi(env) == 0) return 0;   // A/B switch: plain all-reduce of H4
   CIP_CUDA(cudaSetDevice(h->device));
@@ -708,7 +713,9 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   }
   // (h->opt.fold_scaling is 0 when the caller's struct does not reach the field: h->opt starts zeroed)
   if (!h->rs.on) CIP_TRY(engine_decide_fold(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0, mn, &h->fold));
-  if (!h->fold && !h->rs.on) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
+  if (!h->rs.on && !h->fold) CIP_TRY(fast_syrk_plan(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0));
+  if (h->fast.on) CIP_TRY(dev_alloc(h, &h->Atil4, fast_syrk_atil_doubles(h)));
+  else if (!h->fold && !h->rs.on) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
   // row_structure = 2 keeps no n_pad^2 buffer: dense Q is staged in Qq4 until split_build has gathered Q_KK
   const bool split = h->rs.sp.on;
   if (!split || (!Qs && h->opt.q_kind == 0)) CIP_TRY(dev_alloc(h, &h->Qq4, nn));
@@ -786,6 +793,9 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
     // (structure_finish makes the operand map of the rest rows)
   } else if (h->fold) {
     CIP_TRY(make_q4_tensor_map(&h->mapAt.map, h->At4, h->n_pad, h->m_pad / 4));
+  } else if (h->fast.on) {
+    CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (long long)h->fast.K2));   // 4 K2 rows = K2 quads
+    CIP_TRY(fast_syrk_setup(h));
   } else if (h->m_pad + h->aug_rows > 0) {
     CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (h->m_pad + h->aug_rows) / 4));
   }

@@ -57,6 +57,22 @@ struct RowStructure {
     double* kv[2][3] = {};          // per column set b: rhs_K, t_K, products on K (nK_pad + 4 each)
   } sp;
 };
+
+// Fast SYRK (fast_syrk.cu): H = Q + Atil'Atil as a blocked SYRK whose off-diagonal blocks take one Strassen-Winograd
+// level on power-of-two equilibrated columns.  Dense single-device R-only handles at large n (CIP_FAST_SYRK = 0 / 1
+// forces it off / on where the handle allows it).  Atil4 then holds 4 K2 rows of contraction: the rows of A
+// (zero-padded to 2 K2), then the operand sums of the products.
+struct FastSyrk {
+  bool on = false;
+  int depth = 0;               // levels of halving of [0, n_pad)
+  int leaf = 0;                // n_pad >> depth: width of the diagonal blocks left to the plain SYRK
+  int K2 = 0;                  // half the contraction (rows of A, padded), a multiple of 32
+  int nchunk = 0;              // k chunks of the column sums of squares
+  int* colexp = nullptr;       // [n_pad] e_j = round(log2 ||Atil[:, j]||)
+  double* colss = nullptr;     // [nchunk * n_pad]
+  double* M = nullptr;         // the seven product tiles of every pair of one depth (7 n_pad^2 / 16)
+  int4* table = nullptr;       // GemmArgs::group entries: the leaves, then the products of depth 0, 1, ...
+};
 }  // namespace cip
 
 struct cip_engine {
@@ -92,6 +108,7 @@ struct cip_engine {
   int aug_rows = 0;        // rows of Atil4 beyond m_pad holding sqrt(aug_rho) * G
   double aug_rho = 0.0;
   cip::RowStructure rs;    // opts.row_structure: At4 / Atil4 are not allocated
+  cip::FastSyrk fast;      // the Winograd SYRK of form_H (sized at cip_create, dropped when a communicator is attached)
   std::vector<void*> owned;   // further device buffers freed by cip_destroy
   // work vectors
   double* nv[NV] = {};
@@ -134,6 +151,18 @@ const char* last_error_string();
 int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold);
 // buffers / streams of the overlapped Gram reduction, once the communicator exists (engine.cu)
 int engine_setup_comm(cip_engine* h);
+
+// ---- fast SYRK (fast_syrk.cu)
+// LEVEL 1, before Atil4 is allocated: take the fast path?  `can`: dense, unfolded, every row an R row, no
+// augmentation rows.  Sets h->fast (n_pad, free memory, CIP_FAST_SYRK, CIP_FAST_SYRK_LEAF).
+int fast_syrk_plan(cip_engine* h, bool can);
+size_t fast_syrk_atil_doubles(const cip_engine* h);     // the size of Atil4 when h->fast.on
+// LEVEL 1, after Atil4: exponents, scratch, product tiles, the launch table
+int fast_syrk_setup(cip_engine* h);
+// a communicator was attached: back to the plain Atil4 and the classical SYRK
+int fast_syrk_drop(cip_engine* h);
+// LEVEL 2, after cone_scale_panel_norms: H4 = cin + Atil'Atil (lower triangle)
+int fast_syrk_form(cip_engine* h, const double* cin);
 
 // ---- row structure (structure.cu)
 // LEVEL 1, dense input: classify the rows of the packed At4, build the compact arrays, free At4

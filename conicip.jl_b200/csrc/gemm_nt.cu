@@ -56,6 +56,23 @@ __device__ __forceinline__ void tile_of(const GemmArgs& a, int t, int& ti, int& 
   }
 }
 
+// where linear tile `tile` of a launch sits: its tile coordinates and the origins of its product (GemmArgs::group)
+struct TilePos {
+  int ti, tj, x_row0, x_kq0, y_row0, y_kq0, c_row0, c_col0;
+};
+__device__ __forceinline__ TilePos locate(const GemmArgs& a, int tile) {
+  TilePos p{0, 0, a.x_row0, a.x_kq0, a.y_row0, a.y_kq0, a.c_row0, a.c_col0};
+  if (a.group) {
+    const int e = tile / a.group_tiles;
+    tile -= e * a.group_tiles;
+    const int4 o = a.group[2 * e], c = a.group[2 * e + 1];
+    p.x_row0 = o.x; p.x_kq0 = o.y; p.y_row0 = o.z; p.y_kq0 = o.w;
+    p.c_row0 = c.x; p.c_col0 = c.y;
+  }
+  tile_of(a, tile, p.ti, p.tj);
+  return p;
+}
+
 template <bool SCALED>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmY,
@@ -66,12 +83,12 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
   uint64_t* empty = full + STAGES;
   double* kscales = reinterpret_cast<double*>(smem_raw + (size_t)STAGES * STAGE_DOUBLES * 8 + 128);   // [STAGES][KT]
 
-  int ti, tj;
   // CTAs below tail0 own a whole tile; above it, ksplit consecutive CTAs share one (k tiles [kt0, kt1))
   const bool split = (int)blockIdx.x >= a.tail0 && a.ksplit > 1;
   const int tile = a.tile_begin + (split ? a.tail0 + ((int)blockIdx.x - a.tail0) / a.ksplit : (int)blockIdx.x);
   const int sp = split ? ((int)blockIdx.x - a.tail0) % a.ksplit : 0;
-  tile_of(a, tile, ti, tj);
+  const TilePos P = locate(a, tile);
+  const int ti = P.ti, tj = P.tj;
   const int kt0 = split ? sp * a.kchunk : 0;
   const int kt1 = split ? ((kt0 + a.kchunk < a.nk) ? kt0 + a.kchunk : a.nk) : a.nk;
   const bool same = a.sym && (ti == tj);
@@ -92,8 +109,8 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
     if (lane == 0 && kt1 > kt0) {
       tma_prefetch_desc(&tmX);
       tma_prefetch_desc(&tmY);
-      const int xr = (a.x_row0 + ti * BM) * 4;
-      const int yr = (a.y_row0 + tj * BN) * 4;
+      const int xr = (P.x_row0 + ti * BM) * 4;
+      const int yr = (P.y_row0 + tj * BN) * 4;
       const uint32_t bytes = (same ? 2u * BOX_BYTES : 4u * BOX_BYTES) + (SCALED ? (uint32_t)(KT * 8) : 0u);
       for (int kt = kt0; kt < kt1; ++kt) {
         const int s = (kt - kt0) % STAGES;
@@ -101,16 +118,16 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
         mbar_wait(&empty[s], ph ^ 1u);
         double* st = tiles + (size_t)s * STAGE_DOUBLES;
         mbar_arrive_expect_tx(&full[s], bytes);
-        tma_load_2d(st, &tmX, &full[s], xr, a.x_kq0 + kt * KQ);
-        tma_load_2d(st + BOX_DOUBLES, &tmX, &full[s], xr + HALF * 4, a.x_kq0 + kt * KQ);
+        tma_load_2d(st, &tmX, &full[s], xr, P.x_kq0 + kt * KQ);
+        tma_load_2d(st + BOX_DOUBLES, &tmX, &full[s], xr + HALF * 4, P.x_kq0 + kt * KQ);
         if (!same) {
-          tma_load_2d(st + 2 * BOX_DOUBLES, &tmY, &full[s], yr, a.y_kq0 + kt * KQ);
-          tma_load_2d(st + 3 * BOX_DOUBLES, &tmY, &full[s], yr + HALF * 4, a.y_kq0 + kt * KQ);
+          tma_load_2d(st + 2 * BOX_DOUBLES, &tmY, &full[s], yr, P.y_kq0 + kt * KQ);
+          tma_load_2d(st + 3 * BOX_DOUBLES, &tmY, &full[s], yr + HALF * 4, P.y_kq0 + kt * KQ);
         }
         if (SCALED)      // the 32 row factors of this k tile (1-D bulk copy onto the same barrier)
           asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
                            smem_u32(kscales + s * KT)),
-                       "l"(a.kscale + (size_t)(a.y_kq0 + kt * KQ) * 4), "r"((uint32_t)(KT * 8)), "r"(smem_u32(&full[s]))
+                       "l"(a.kscale + (size_t)(P.y_kq0 + kt * KQ) * 4), "r"((uint32_t)(KT * 8)), "r"(smem_u32(&full[s]))
                        : "memory");
       }
     }
@@ -173,8 +190,8 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
             make_double2(alpha * acc[mi][ni][0], alpha * acc[mi][ni][1]);
     return;
   }
-  const int row_base = a.c_row0 + ti * BM + warp_m * 64 + g;
-  const int col_base = a.c_col0 + tj * BN + warp_n * 32 + 2 * t;
+  const int row_base = P.c_row0 + ti * BM + warp_m * 64 + g;
+  const int col_base = P.c_col0 + tj * BN + warp_n * 32 + 2 * t;
   double* tm = a.Ctm ? a.Ctm + (size_t)tile * (size_t)(BM * BN) : nullptr;
   // Cin and Cout are the same buffer for the Cholesky updates, so the compiler has to keep every load behind the
   // previous store: a load -> add -> store loop is a chain of 32 global-memory latencies (17 us, as long as the
@@ -204,9 +221,8 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
 
 // C tile = Cin tile + sum over splits (in split order) of the partial tiles in the workspace
 __global__ void __launch_bounds__(256) splitk_reduce_kernel(const GemmArgs a) {
-  int ti, tj;
   const int tile = a.tile_begin + a.tail0 + blockIdx.x;
-  tile_of(a, tile, ti, tj);
+  const TilePos P = locate(a, tile);
   double* tm = a.Ctm ? a.Ctm + (size_t)tile * (size_t)(BM * BN) : nullptr;
   const size_t slab = (size_t)(BM * BN);
   const double* wt = a.ws + (size_t)blockIdx.x * a.ksplit * slab;
@@ -218,7 +234,7 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const GemmArgs a) {
       v.y += w.y;
     }
     const int quad = e / (BM * 4), lr = (e % (BM * 4)) >> 2, c = e & 3;
-    const size_t idx = q4_index(a.c_row0 + ti * BM + lr, a.c_col0 + tj * BN + quad * 4 + c, a.ldc);
+    const size_t idx = q4_index(P.c_row0 + P.ti * BM + lr, P.c_col0 + P.tj * BN + quad * 4 + c, a.ldc);
     if (a.Cin) {
       const double2 ci = *reinterpret_cast<const double2*>(a.Cin + idx);
       v.x += ci.x;
@@ -231,13 +247,12 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const GemmArgs a) {
 
 // Cout tile <- tile-major tile (both Q4: 512-double runs move as they are)
 __global__ void __launch_bounds__(256) unpack_tiles_kernel(const GemmArgs a) {
-  int ti, tj;
   const int tile = a.tile_begin + blockIdx.x;
-  tile_of(a, tile, ti, tj);
+  const TilePos P = locate(a, tile);
   const double* tm = a.Ctm + (size_t)tile * (size_t)(BM * BN);
   for (int e = threadIdx.x * 2; e < BM * BN; e += 512) {
     const int quad = e / (BM * 4), lr = (e % (BM * 4)) >> 2, c = e & 3;
-    const size_t idx = q4_index(a.c_row0 + ti * BM + lr, a.c_col0 + tj * BN + quad * 4 + c, a.ldc);
+    const size_t idx = q4_index(P.c_row0 + P.ti * BM + lr, P.c_col0 + P.tj * BN + quad * 4 + c, a.ldc);
     *reinterpret_cast<double2*>(a.Cout + idx) = *reinterpret_cast<const double2*>(tm + e);
   }
 }

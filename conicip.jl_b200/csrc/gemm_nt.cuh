@@ -54,6 +54,12 @@ struct GemmArgs {
   // C += sum_k X[i,k] * kscale[k]^2 * Y[j,k].  The 32 factors of a k tile travel with it through the pipeline (one
   // 256-byte bulk copy per stage) and are applied to the Y fragments in registers.  nullptr: no scaling.
   const double* kscale;
+  // Grouped launch (the fast SYRK, fast_syrk.cu): the grid holds several products of the same tile grid and nk, each
+  // `group_tiles` consecutive linear tiles.  Linear tile t belongs to product e = t / group_tiles, whose origins come
+  // from device memory: group[2e] = {x_row0, x_kq0, y_row0, y_kq0}, group[2e + 1] = {c_row0, c_col0, -, -} (the
+  // fields above are ignored).  tile_count must then be set.  nullptr: one product.
+  const int4* group;
+  int group_tiles;
 };
 constexpr long long GEMM_WS_DOUBLES = 2048ll * 128 * 128;   // 2048 partial tiles (268 MB)
 

@@ -86,6 +86,11 @@ int cone_maxstep(const ConeDesc& c, const double* x, const double* d, double d_s
 // Atil = F^-T A on the Q4 transposed panel (rows = columns of A, k = rows of A)
 int cone_scale_panel(const ConeDesc& c, Scaling Fi, const double* At4, double* Atil4, int ld, int m_pad,
                      int ncols, cudaStream_t st);
+// The same for R rows only (the diagonal pass), which also leaves e_j = round(log2 ||Atil[:, j]||) in colexp[ld]
+// (the fast SYRK's column equilibration).  colss: scale_panel_norms_chunks(m_pad) * ld doubles of scratch; ld % 256 == 0.
+int scale_panel_norms_chunks(int m_pad);
+int cone_scale_panel_norms(Scaling Fi, const double* At4, double* Atil4, int ld, int m_pad, double* colss,
+                           int* colexp, cudaStream_t st);
 
 // ---------------------------------------------------------------- S (PSD) cones (sdp.cu)
 int sdp_max_order();
