@@ -794,7 +794,7 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   } else if (h->fold) {
     CIP_TRY(make_q4_tensor_map(&h->mapAt.map, h->At4, h->n_pad, h->m_pad / 4));
   } else if (h->fast.on) {
-    CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (long long)h->fast.K2));   // 4 K2 rows = K2 quads
+    CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (long long)(fast_syrk_atil_doubles(h) / h->n_pad / 4)));
     CIP_TRY(fast_syrk_setup(h));
   } else if (h->m_pad + h->aug_rows > 0) {
     CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (h->m_pad + h->aug_rows) / 4));

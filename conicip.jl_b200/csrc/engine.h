@@ -59,19 +59,22 @@ struct RowStructure {
 };
 
 // Fast SYRK (fast_syrk.cu): H = Q + Atil'Atil as a blocked SYRK whose off-diagonal blocks take one Strassen-Winograd
-// level on power-of-two equilibrated columns.  Dense single-device R-only handles at large n (CIP_FAST_SYRK = 0 / 1
-// forces it off / on where the handle allows it).  Atil4 then holds 4 K2 rows of contraction: the rows of A
-// (zero-padded to 2 K2), then the operand sums of the products.
+// level on power-of-two equilibrated columns, two where the blocks are wide.  Dense single-device R-only handles at
+// large n (CIP_FAST_SYRK = 0 / 1 forces it off / on where the handle allows it).  Atil4 then holds 4 K2 rows of
+// contraction: the rows of A (zero-padded to 2 K2), then the operand sums of the products; K2 / 2 more for the
+// level-2 sums when some depth takes two levels.
 struct FastSyrk {
   bool on = false;
   int depth = 0;               // levels of halving of [0, n_pad)
   int leaf = 0;                // n_pad >> depth: width of the diagonal blocks left to the plain SYRK
-  int K2 = 0;                  // half the contraction (rows of A, padded), a multiple of 32
+  int K2 = 0;                  // half the contraction (rows of A, padded), a multiple of 32 (of 64 when two != 0)
+  unsigned two = 0;            // bit d: depth d takes a second Winograd level
   int nchunk = 0;              // k chunks of the column sums of squares
   int* colexp = nullptr;       // [n_pad] e_j = round(log2 ||Atil[:, j]||)
   double* colss = nullptr;     // [nchunk * n_pad]
   double* M = nullptr;         // the seven product tiles of every pair of one depth (7 n_pad^2 / 16)
-  int4* table = nullptr;       // GemmArgs::group entries: the leaves, then the products of depth 0, 1, ...
+  double* M2 = nullptr;        // the level-2 sub-product tiles of one level-1 product, every pair (two != 0)
+  int4* table = nullptr;       // GemmArgs::group entries: the leaves, the products of depth 0, 1, ..., the level-2 ones
 };
 }  // namespace cip
 
@@ -154,7 +157,7 @@ int engine_setup_comm(cip_engine* h);
 
 // ---- fast SYRK (fast_syrk.cu)
 // LEVEL 1, before Atil4 is allocated: take the fast path?  `can`: dense, unfolded, every row an R row, no
-// augmentation rows.  Sets h->fast (n_pad, free memory, CIP_FAST_SYRK, CIP_FAST_SYRK_LEAF).
+// augmentation rows.  Sets h->fast (n_pad, free memory, CIP_FAST_SYRK, CIP_FAST_SYRK_LEAF, CIP_FAST_SYRK_LEVELS).
 int fast_syrk_plan(cip_engine* h, bool can);
 size_t fast_syrk_atil_doubles(const cip_engine* h);     // the size of Atil4 when h->fast.on
 // LEVEL 1, after Atil4: exponents, scratch, product tiles, the launch table
