@@ -140,6 +140,26 @@ scale_panel_wood_kernel(ConeDesc c, Scaling Fi, const double* __restrict__ At4, 
   for (int k = off; k < end; ++k) Atil4[q4_index(j, k, ld)] += Fi.b[k] * dot;
 }
 
+// block (cone, 128 columns), thread per column j: the Woodbury dot of scale_panel_wood_kernel, in the same order,
+// stored once per k tile of the cone instead of being added to every row
+__global__ void __launch_bounds__(128)
+qfold_t_kernel(ConeDesc c, Scaling Fi, const double* __restrict__ At4, int ld, int ncols,
+               const uint8_t* __restrict__ qslot, int qs, double* __restrict__ T4) {
+  const int ci = c.qlist[blockIdx.x];
+  const int j = blockIdx.y * blockDim.x + threadIdx.x;
+  if (j >= ncols) return;
+  const int off = c.off[ci], end = c.off[ci + 1];
+  double dot = 0;
+  if (Fi.kind[ci] == CIP_BLK_WOODBURY) {
+    for (int k = off; k < end; ++k) dot += Fi.b[k] * At4[q4_index(j, k, ld)];
+    dot *= Fi.D[ci];
+  }
+  for (int kt = off / 32; kt * 32 < end; ++kt) {
+    const int r = kt * 32 > off ? kt * 32 : off;
+    T4[q4_index(j, kt * qs + qslot[r], ld)] = dot;
+  }
+}
+
 inline int nblocks(int n, int per) {
   int b = (n + per - 1) / per;
   const int cap = sm_count() * 16;
@@ -604,6 +624,14 @@ int cone_scale_panel(const ConeDesc& c, Scaling Fi, const double* At4, double* A
     CIP_CHECK_LAUNCH();
   }
   CIP_TRY(sdp_scale_panel(c, Fi, At4, Atil4, ld, ncols, st));
+  return 0;
+}
+
+int cone_qfold_t(const ConeDesc& c, Scaling Fi, const double* At4, int ld, int ncols, const uint8_t* qslot, int qs,
+                 double* T4, cudaStream_t st) {
+  if (c.nq == 0 || ncols == 0) return 0;
+  qfold_t_kernel<<<dim3(c.nq, (ncols + 127) / 128), 128, 0, st>>>(c, Fi, At4, ld, ncols, qslot, qs, T4);
+  CIP_CHECK_LAUNCH();
   return 0;
 }
 

@@ -226,6 +226,14 @@ int set_scaling_from_user(cip_engine* h, const int* kind, const double* fa, cons
   return 0;
 }
 
+// Q-cone fold: the row factors, cone terms and slots of the contraction rows (GemmArgs::qalpha ..)
+void qfold_args(const cip_engine* h, GemmArgs& a) {
+  a.qalpha = h->Fi.a;       // R rows: 1/w; Q rows: the diagonal of the Woodbury inverse; aug rows: 1
+  a.qg = h->Fi.b;           // zero on R rows and on non-Woodbury blocks
+  a.qslot = h->qslot;
+  a.qs = h->qs;
+}
+
 // Row-sharded form of H: the partial Gram matrix is produced tile-major in a few ranges of the (reversed) tile
 // order; each range is all-reduced (NCCL, stream cs) and unpacked into H4 while the next ranges are still being
 // computed, so only the last, small range (the tip of the triangle) is exposed.  Ranges alternate between two
@@ -260,10 +268,12 @@ int form_H_sharded(cip_engine* h, const double* cin, int k_rows) {
     a.nk = k_rows / 32;
     a.Cin = cin; a.Cout = h->H4; a.Ctm = h->Hp; a.ldc = h->n_pad; a.alpha = 1.0;
     a.tile_begin = (int)t0; a.tile_count = (int)(ends[i] - t0);
-    if (h->fold) a.kscale = h->Fi.a;
+    if (h->fold && h->qs == 0) a.kscale = h->Fi.a;
+    if (h->qs > 0) qfold_args(h, a);
     if (i == nr - 1) { a.ws = h->gemm_ws; a.ws_doubles = GEMM_WS_DOUBLES; }     // split-K only for the very last wave
     const GemmOperand& op = h->fold ? h->mapAt : h->mapAtil;
-    CIP_TRY(launch_gemm_nt(op, op, a, st));
+    if (h->qs > 0) CIP_TRY(launch_gemm_nt_qfold(op, h->mapTq, a, st));
+    else CIP_TRY(launch_gemm_nt(op, op, a, st));
     CIP_CUDA(cudaEventRecord(h->evc[i], st));
     CIP_CUDA(cudaStreamWaitEvent(h->cs, h->evc[i], 0));
     double* seg = h->Hp + (size_t)t0 * TILE * TILE;
@@ -304,6 +314,7 @@ int form_H(cip_engine* h) {
   const bool fast = h->fast.on && !h->comm;
   if (fast) CIP_TRY(cone_scale_panel_norms(h->Fi, h->At4, h->Atil4, h->n_pad, h->m_pad, h->fast.colss, h->fast.colexp, s));
   else if (h->m_pad > 0 && !h->fold) CIP_TRY(cone_scale_panel(h->cd, h->Fi, h->At4, h->Atil4, h->n_pad, h->m_pad, h->n, s));
+  else if (h->qs > 0) CIP_TRY(cone_qfold_t(h->cd, h->Fi, h->At4, h->n_pad, h->n, h->qslot, h->qs, h->Tq4, s));
   CIP_CUDA(cudaEventRecord(h->ev[1], s));
   const double* cin = (h->rank == 0) ? h->Qq4 : nullptr;
   // rows of Atil beyond m_pad hold sqrt(rho)*G (constant): H' = Q + Atil'Atil + rho G'G, added on rank 0 only
@@ -323,7 +334,7 @@ int form_H(cip_engine* h) {
     a.x_row0 = a.y_row0 = 0; a.x_kq0 = a.y_kq0 = 0; a.nk = k_rows / 32;
     a.Cin = cin; a.Cout = h->H4; a.ldc = h->n_pad; a.c_row0 = a.c_col0 = 0; a.alpha = 1.0;
     a.ws = h->gemm_ws; a.ws_doubles = GEMM_WS_DOUBLES;        // tall-skinny A (n << m): split the contraction
-    if (h->fold) a.kscale = h->Fi.a;                          // W^-2 applied to the fragments: no Atil4
+    if (h->fold && h->qs == 0) a.kscale = h->Fi.a;           // W^-2 applied to the fragments: no Atil4
     const GemmOperand& op = h->fold ? h->mapAt : h->mapAtil;
     // Experiment knob (profiles/r02_syrk_traffic.md): CIP_SYRK_KCHUNK = rows of A per launch, every launch
     // accumulating into H.  Off by default: at C4 it did not lower the DRAM traffic of the operand panels (994 GB in
@@ -331,7 +342,10 @@ int form_H(cip_engine* h) {
     static const int kchunk_rows = [] { const char* e = getenv("CIP_SYRK_KCHUNK"); const int v = e ? atoi(e) : 0; return v > 0 ? (v + 31) / 32 * 32 : 0; }();
     const int total_kt = k_rows / 32;
     const int chunk_kt = (kchunk_rows > 0 && h->n_pad >= 4096) ? kchunk_rows / 32 : total_kt;
-    if (total_kt > chunk_kt + chunk_kt / 2) {
+    if (h->qs > 0) {                                          // F^-T A formed from At4 and Tq4 in registers
+      qfold_args(h, a);
+      CIP_TRY(launch_gemm_nt_qfold(op, h->mapTq, a, s));
+    } else if (total_kt > chunk_kt + chunk_kt / 2) {
       for (int kt0 = 0; kt0 < total_kt;) {
         int kn = chunk_kt;
         if (total_kt - (kt0 + kn) < chunk_kt / 2) kn = total_kt - kt0;       // fold a short remainder into the last chunk
@@ -494,16 +508,16 @@ int engine_setup_comm(cip_engine* h) {
   return 0;
 }
 const char* last_error_string() { return g_err; }
-int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold) {
-  // fold the scaling into the SYRK (no Atil4) for pure R-cone rows: on request, or when the second copy of A would
-  // not fit next to what is still to be allocated (Q, H, workspaces: ~ 3 n_pad^2 + 2.2 GB)
+int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold, size_t ahead) {
+  // fold the scaling into the SYRK (no Atil4): on request, or when the second copy of A would not fit next to what is
+  // still to be allocated (`ahead` bytes, Q, H, workspaces: ~ 3 n_pad^2 + 2.2 GB)
   int mode = can ? h->opt.fold_scaling : 2;
   if (const char* env = getenv("CIP_FOLD_SCALING")) { if (can) mode = atoi(env); }
   if (mode == 0) {
     size_t free_b = 0, total_b = 0;
     CIP_CUDA(cudaMemGetInfo(&free_b, &total_b));
     const size_t nn = (size_t)h->n_pad * h->n_pad;
-    const size_t need = mn * 8 + 3 * nn * 8 + (size_t)GEMM_WS_DOUBLES * 8 + (size_t(1) << 30);
+    const size_t need = ahead + mn * 8 + 3 * nn * 8 + (size_t)GEMM_WS_DOUBLES * 8 + (size_t(1) << 30);
     mode = (free_b < need) ? 1 : 2;
   }
   *fold = (mode == 1);
@@ -520,6 +534,46 @@ int cip_version(void) { return 100; }
 }  // extern "C"
 
 namespace {
+
+// The slots of the folded R + Q SYRK: in every 32-row k tile the Q cones that meet it, numbered in row order.  Returns
+// the slot count of the kernel (gemm_qfold_slots of the largest such number: 4, 8, 12 or 16), 0 when a tile meets more
+// than 16 cones (cones of dimension 1 or 2) -- the handle then materialises Atil4.  slot[k]: a byte per row of the
+// contraction (m_pad + aug_rows), 0 for R, padding and aug rows.
+int qfold_slot_plan(const cip_engine* h, const std::vector<int>& qlist, std::vector<uint8_t>* slot) {
+  slot->assign((size_t)h->m_pad + h->aug_rows, 0);
+  std::vector<int> used(((size_t)h->m_pad + h->aug_rows) / 32, 0);      // distinct Q cones met so far, per k tile
+  int need = 0;
+  for (int ci : qlist) {                                                // (qlist is in row order)
+    const int off = h->h_off[ci], end = h->h_off[ci + 1];
+    for (int kt = off / 32; kt * 32 < end; ++kt) {
+      const int sl = used[kt]++;
+      need = std::max(need, sl + 1);
+      if (sl > 255) return 0;
+      for (int r = std::max(off, kt * 32); r < std::min(end, kt * 32 + 32); ++r) (*slot)[r] = (uint8_t)sl;
+    }
+  }
+  return gemm_qfold_slots(need);
+}
+
+// buffers of the folded R + Q SYRK (h->qs set, At4 and the scaling arrays sized for the augmentation rows): the T rows,
+// the slot table, and Fi.a = 1 on the sqrt(rho) G rows that follow A in At4 (Fi.b stays 0 there)
+int qfold_alloc(cip_engine* h, const std::vector<uint8_t>& qslot) {
+  const size_t k_rows = (size_t)h->m_pad + h->aug_rows;
+  if (h->aug_rows > 0) {
+    const std::vector<double> ones(h->aug_rows, 1.0);
+    // (on the handle's stream, behind dev_alloc's zero fill: a plain cudaMemcpy does not wait for a non-blocking stream)
+    CIP_CUDA(cudaMemcpyAsync(h->Fi.a + h->m_pad, ones.data(), ones.size() * sizeof(double), cudaMemcpyHostToDevice,
+                             h->stream));
+    CIP_CUDA(cudaStreamSynchronize(h->stream));                // `ones` goes out of scope
+  }
+  CIP_TRY(dev_alloc(h, &h->Tq4, k_rows / 32 * h->qs * h->n_pad));
+  CIP_TRY(dev_alloc(h, &h->qslot, k_rows + 16));
+  CIP_CUDA(cudaMemcpyAsync(h->qslot, qslot.data(), k_rows, cudaMemcpyHostToDevice, h->stream));
+  CIP_CUDA(cudaStreamSynchronize(h->stream));                  // `qslot` is the caller's host vector
+  h->owned.push_back(h->Tq4);
+  h->owned.push_back(h->qslot);
+  return 0;
+}
 
 // upload a CSC matrix (host or device arrays) and scatter it into a zero-initialised Q4 buffer
 int upload_csc(cip_engine* h, double* dst, int ld, const cip_csc* M, int transpose) {
@@ -689,10 +743,36 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   h->cd.nr_rows = 0;
   for (int i = 0; i < ncones; ++i)
     if (cone_type[i] == CIP_CONE_R) h->cd.nr_rows += h->h_off[i + 1] - h->h_off[i];
+  // ---- how H is formed: from a materialised Atil4, or with the scaling folded into the SYRK.  Decided before A and F
+  //      are allocated, so that a folded R + Q handle sizes At4 and the scaling arrays for its augmentation rows at once.
+  const size_t nn = (size_t)h->n_pad * h->n_pad;
+  const size_t mn = (size_t)h->m_pad * h->n_pad;
+  // augmentation rows (H + rho G'G keeps the Cholesky valid when H is singular on range(G'), as kktsolver_qr allows)
+  {
+    double rho = h->opt.aug_rho;
+    if (rho < 0) rho = (p > 0) ? 1.0 : 0.0;
+    h->aug_rho = (p > 0) ? rho : 0.0;
+    h->aug_rows = (h->aug_rho > 0) ? round_up(p, 32) : 0;
+  }
+  // (h->opt.fold_scaling is 0 when the caller's struct does not reach the field: h->opt starts zeroed; the free-memory
+  //  rule counts At4 as still to come)
+  const size_t at4_ahead = (h->rs.on && As) ? 0 : mn * sizeof(double);
+  if (!h->rs.on)
+    CIP_TRY(engine_decide_fold(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0, mn, &h->fold, at4_ahead));
+  // R + Q cones: the fold forms F^-T A row by row inside the SYRK from the cones' T rows (launch_gemm_nt_qfold)
+  std::vector<uint8_t> qslot;
+  const int qs = (!h->rs.on && !qlist.empty() && slist.empty() && m > 0) ? qfold_slot_plan(h, qlist, &qslot) : 0;
+  if (qs > 0) {
+    CIP_TRY(engine_decide_fold(h, true, (size_t)(h->m_pad + h->aug_rows) * h->n_pad, &h->fold, at4_ahead));
+    if (h->fold) h->qs = qs;
+  }
+  // rows of the contraction the handle keeps in At4 and in the scaling arrays: a folded R + Q handle appends the
+  // sqrt(rho) G rows to A there, with the row factor 1 and no cone term (qfold_alloc)
+  const size_t k_rows = (size_t)h->m_pad + (h->qs > 0 ? h->aug_rows : 0);
   for (Scaling* S : {&h->F, &h->Fi}) {
     CIP_TRY(dev_alloc(h, &S->kind, ncones));
-    CIP_TRY(dev_alloc(h, &S->a, h->m_pad + 4));
-    CIP_TRY(dev_alloc(h, &S->b, h->m_pad + 4));
+    CIP_TRY(dev_alloc(h, &S->a, k_rows + 4));
+    CIP_TRY(dev_alloc(h, &S->b, k_rows + 4));
     CIP_TRY(dev_alloc(h, &S->D, ncones));
   }
   CIP_TRY(dev_alloc(h, &h->F.R, h->r_total));
@@ -701,18 +781,8 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   h->Fi.Ri = h->F.Ri;
 
   // ---- matrices
-  const size_t nn = (size_t)h->n_pad * h->n_pad;
-  const size_t mn = (size_t)h->m_pad * h->n_pad;
-  if (!(h->rs.on && As)) CIP_TRY(dev_alloc(h, &h->At4, mn));     // CSC input with row structure: never dense
-  // augmentation rows (H + rho G'G keeps the Cholesky valid when H is singular on range(G'), as kktsolver_qr allows)
-  {
-    double rho = h->opt.aug_rho;
-    if (rho < 0) rho = (p > 0) ? 1.0 : 0.0;
-    h->aug_rho = (p > 0) ? rho : 0.0;
-    h->aug_rows = (h->aug_rho > 0) ? round_up(p, 32) : 0;
-  }
-  // (h->opt.fold_scaling is 0 when the caller's struct does not reach the field: h->opt starts zeroed)
-  if (!h->rs.on) CIP_TRY(engine_decide_fold(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0, mn, &h->fold));
+  if (!(h->rs.on && As)) CIP_TRY(dev_alloc(h, &h->At4, k_rows * h->n_pad));   // CSC input with row structure: never dense
+  if (h->qs > 0) CIP_TRY(qfold_alloc(h, qslot));
   if (!h->rs.on && !h->fold) CIP_TRY(fast_syrk_plan(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0));
   if (h->fast.on) CIP_TRY(dev_alloc(h, &h->Atil4, fast_syrk_atil_doubles(h)));
   else if (!h->fold && !h->rs.on) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
@@ -791,6 +861,10 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   }
   if (h->rs.on) {
     // (structure_finish makes the operand map of the rest rows)
+  } else if (h->fold && h->qs > 0) {
+    CIP_TRY(make_q4_tensor_map(&h->mapAt.map, h->At4, h->n_pad, (h->m_pad + h->aug_rows) / 4));
+    CIP_TRY(make_q4_tensor_map(&h->mapTq.map, h->Tq4, h->n_pad, (long long)(h->m_pad + h->aug_rows) / 32 * h->qs / 4,
+                               h->qs / 4));
   } else if (h->fold) {
     CIP_TRY(make_q4_tensor_map(&h->mapAt.map, h->At4, h->n_pad, h->m_pad / 4));
   } else if (h->fast.on) {
@@ -826,8 +900,9 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
       CIP_CUDA(cudaStreamSynchronize(s));
       if (stg) cudaFree(stg);
     }
-    if (h->aug_rows > 0 && !h->rs.on)
-      CIP_TRY(transpose_scale_q4(h->Atil4, h->n_pad, h->m_pad, h->G4, h->p_pad, p, n, sqrt(h->aug_rho), s));
+    if (h->aug_rows > 0 && !h->rs.on)      // (folded R + Q: At4 carries them, with qalpha = 1 and qg = 0)
+      CIP_TRY(transpose_scale_q4(h->fold ? h->At4 : h->Atil4, h->n_pad, h->m_pad, h->G4, h->p_pad, p, n,
+                                 sqrt(h->aug_rho), s));
     CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, p, h->p_pad, 1.0, 1, s));
     if (h->opt.reg_eps_G != 0.0) CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, 0, p, h->opt.reg_eps_G, 1, s));
     if (!split) CIP_TRY(make_q4_tensor_map(&h->mapZ.map, h->Z4, h->p_pad, h->n_pad / 4));

@@ -106,9 +106,14 @@ struct cip_engine {
   cip::Scaling F{}, Fi{};
   bool have_scaling = false, have_factor = false;
   double* gemm_ws = nullptr;   // split-K workspace of gemm_nt (GEMM_WS_DOUBLES)
-  bool fold = false;           // R-only handle without Atil4: the SYRK reads At4 and scales in registers (opts.fold_scaling)
+  bool fold = false;           // no Atil4: the SYRK reads At4 and scales in registers (opts.fold_scaling; R or R + Q cones)
   cip::GemmOperand mapAt{};
-  int aug_rows = 0;        // rows of Atil4 beyond m_pad holding sqrt(aug_rho) * G
+  // folded R + Q handle (fold with Q cones): the SYRK forms alpha_k A + g_k T[slot(k)] in registers (launch_gemm_nt_qfold)
+  int qs = 0;                  // slots per 32-row k tile (4, 8, 12 or 16); 0: R-only fold or none
+  double* Tq4 = nullptr;       // (m_pad + aug_rows) / 32 * qs contraction rows, Q4 with ld = n_pad (cone_qfold_t)
+  uint8_t* qslot = nullptr;    // [m_pad + aug_rows]: slot of each row's Q cone in its k tile (0 for R / aug rows)
+  cip::GemmOperand mapTq{};
+  int aug_rows = 0;        // rows of Atil4 (folded R + Q: At4) beyond m_pad holding sqrt(aug_rho) * G
   double aug_rho = 0.0;
   cip::RowStructure rs;    // opts.row_structure: At4 / Atil4 are not allocated
   cip::FastSyrk fast;      // the Winograd SYRK of form_H (sized at cip_create, dropped when a communicator is attached)
@@ -150,8 +155,8 @@ int engine_create_single(cip_handle* out, int n, int m, int p, const double* Q, 
                          int ncones, const int* cone_type, const int* cone_dim, const cip_options* opts);
 const char* last_error_string();
 // fold the scaling into the SYRK? (opts.fold_scaling / CIP_FOLD_SCALING, else free memory against the mn-double
-// second copy); `can`: every row of the SYRK is an R row
-int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold);
+// second copy plus `ahead` bytes not allocated yet); `can`: the fold applies to the rows of the SYRK
+int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold, size_t ahead = 0);
 // buffers / streams of the overlapped Gram reduction, once the communicator exists (engine.cu)
 int engine_setup_comm(cip_engine* h);
 

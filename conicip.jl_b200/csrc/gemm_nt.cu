@@ -15,6 +15,13 @@ namespace {
 constexpr int BM = 128, BN = 128;
 constexpr int KT = 32;
 constexpr int KQ = KT / 4;
+// Q-fold consumers unroll the 8 quads of a k tile by 2.  The T operands push the 168-register budget (9 warps, one
+// CTA per SM) into spills in every unroll (ptxas -v at 2: 56-64 B stack, 84 B spill stores); measured on one B200 at the
+// C3 shape (profiles/r07_fold_qcones.md), 2 is the fastest: SYRK +28 % over the materialised one, against +32 % at 1
+// and +36 % fully unrolled (8).
+constexpr int QUNROLL = 2;
+
+
 constexpr int STAGES = 3;
 constexpr int HALF = 64;
 constexpr int BOX_DOUBLES = HALF * 4 * KQ;       // 2048 doubles
@@ -24,6 +31,15 @@ constexpr int CONSUMER_WARPS = 8;
 constexpr int BAND_DEFAULT = 12;      // tile rows per band of the lower-triangular rasterisation (GemmArgs::band; CIP_GEMM_BAND)
 constexpr int NUM_THREADS = (CONSUMER_WARPS + 1) * 32;
 constexpr int SMEM_BYTES = STAGES * STAGE_DOUBLES * 8 + 128 + STAGES * KT * 8;   // tiles | barriers | k scales per stage
+// Q-fold variant (QS slot rows of T per k tile, GemmArgs::qs: 4, 8, 12 or 16): the T slabs of X and Y sit between the
+// tiles and the barriers; after the row factors (qalpha, in the k-scale slots) come qg and the slot bytes.  Three
+// stages fit 4 slots only (3 x 72 KB); 8 to 16 slots run two.
+__host__ __device__ constexpr int qf_stages(int qs) { return qs > 4 ? 2 : STAGES; }
+__host__ __device__ constexpr int qf_tq_doubles(int qs) { return 4 * HALF * qs; }     // per stage: 2 operands x 2 halves
+__host__ __device__ constexpr int qf_smem_bytes(int qs) {
+  return qf_stages(qs) * (STAGE_DOUBLES + qf_tq_doubles(qs)) * 8 + 128 + qf_stages(qs) * KT * (8 + 8 + 1);
+}
+static_assert(qf_smem_bytes(4) <= 227 * 1024 && qf_smem_bytes(16) <= 227 * 1024, "Q-fold stage does not fit");
 
 __device__ __forceinline__ void tile_of(const GemmArgs& a, int t, int& ti, int& tj) {
   if (a.lower) {
@@ -56,6 +72,13 @@ __device__ __forceinline__ void tile_of(const GemmArgs& a, int t, int& ti, int& 
   }
 }
 
+// 1-D bulk copy global -> shared onto a stage's barrier (16-byte aligned, a multiple of 16 bytes)
+__device__ __forceinline__ void bulk_load(const void* smem_dst, const void* src, uint32_t bytes, uint64_t* bar) {
+  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+                   smem_u32(smem_dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar))
+               : "memory");
+}
+
 // where linear tile `tile` of a launch sits: its tile coordinates and the origins of its product (GemmArgs::group)
 struct TilePos {
   int ti, tj, x_row0, x_kq0, y_row0, y_kq0, c_row0, c_col0;
@@ -73,15 +96,23 @@ __device__ __forceinline__ TilePos locate(const GemmArgs& a, int tile) {
   return p;
 }
 
-template <bool SCALED>
+// QS = 0: X and Y through tmX / tmY (SCALED: the R-cone row factors of GemmArgs::kscale).  QS > 0: the Q-fold SYRK
+// (launch_gemm_nt_qfold): X and Y both come through tmX, tmY maps the slot rows T, and both operands are formed as
+// qalpha * A + qg * T before the DMMAs.
+template <bool SCALED, int QS = 0>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmY,
                const GemmArgs a) {
+  constexpr int NST = QS > 0 ? qf_stages(QS) : STAGES;
+  constexpr int TQ = QS > 0 ? qf_tq_doubles(QS) : 0;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   double* tiles = reinterpret_cast<double*>(smem_raw);
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)STAGES * STAGE_DOUBLES * 8);
-  uint64_t* empty = full + STAGES;
-  double* kscales = reinterpret_cast<double*>(smem_raw + (size_t)STAGES * STAGE_DOUBLES * 8 + 128);   // [STAGES][KT]
+  double* tqs = tiles + (size_t)NST * STAGE_DOUBLES;                                                // [NST][TQ]
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem_raw + (size_t)NST * (STAGE_DOUBLES + TQ) * 8);
+  uint64_t* empty = full + NST;
+  double* kscales = reinterpret_cast<double*>(smem_raw + (size_t)NST * (STAGE_DOUBLES + TQ) * 8 + 128);   // [NST][KT]
+  double* qgs = kscales + NST * KT;                                                                 // [NST][KT]
+  const uint8_t* qsl = reinterpret_cast<const uint8_t*>(qgs + NST * KT);                            // [NST][KT]
 
   // CTAs below tail0 own a whole tile; above it, ksplit consecutive CTAs share one (k tiles [kt0, kt1))
   const bool split = (int)blockIdx.x >= a.tail0 && a.ksplit > 1;
@@ -96,7 +127,7 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
 
   if (threadIdx.x == 0) {
 #pragma unroll
-    for (int s = 0; s < STAGES; ++s) {
+    for (int s = 0; s < NST; ++s) {
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], CONSUMER_WARPS);
     }
@@ -111,18 +142,35 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
       tma_prefetch_desc(&tmY);
       const int xr = (P.x_row0 + ti * BM) * 4;
       const int yr = (P.y_row0 + tj * BN) * 4;
-      const uint32_t bytes = (same ? 2u * BOX_BYTES : 4u * BOX_BYTES) + (SCALED ? (uint32_t)(KT * 8) : 0u);
+      const CUtensorMap* mY = QS > 0 ? &tmX : &tmY;        // (Q fold: one operand; tmY maps T)
+      uint32_t bytes = (same ? 2u * BOX_BYTES : 4u * BOX_BYTES) + (SCALED ? (uint32_t)(KT * 8) : 0u);
+      if (QS > 0) bytes += (same ? 2u : 4u) * (uint32_t)(HALF * QS * 8) + (uint32_t)(KT * (8 + 8 + 1));
       for (int kt = kt0; kt < kt1; ++kt) {
-        const int s = (kt - kt0) % STAGES;
-        const uint32_t ph = (uint32_t)((kt - kt0) / STAGES) & 1u;
+        const int s = (kt - kt0) % NST;
+        const uint32_t ph = (uint32_t)((kt - kt0) / NST) & 1u;
         mbar_wait(&empty[s], ph ^ 1u);
         double* st = tiles + (size_t)s * STAGE_DOUBLES;
         mbar_arrive_expect_tx(&full[s], bytes);
         tma_load_2d(st, &tmX, &full[s], xr, P.x_kq0 + kt * KQ);
         tma_load_2d(st + BOX_DOUBLES, &tmX, &full[s], xr + HALF * 4, P.x_kq0 + kt * KQ);
         if (!same) {
-          tma_load_2d(st + 2 * BOX_DOUBLES, &tmY, &full[s], yr, P.y_kq0 + kt * KQ);
-          tma_load_2d(st + 3 * BOX_DOUBLES, &tmY, &full[s], yr + HALF * 4, P.y_kq0 + kt * KQ);
+          tma_load_2d(st + 2 * BOX_DOUBLES, mY, &full[s], yr, P.y_kq0 + kt * KQ);
+          tma_load_2d(st + 3 * BOX_DOUBLES, mY, &full[s], yr + HALF * 4, P.y_kq0 + kt * KQ);
+        }
+        if (QS > 0) {
+          // the S x 128 slot rows of T for the X (and Y) rows of this k tile, then qalpha / qg / slot of its 32 rows
+          const int ktg = P.y_kq0 / KQ + kt;
+          double* tq = tqs + (size_t)s * TQ;
+          tma_load_2d(tq, &tmY, &full[s], xr, ktg * (QS / 4));
+          tma_load_2d(tq + HALF * QS, &tmY, &full[s], xr + HALF * 4, ktg * (QS / 4));
+          if (!same) {
+            tma_load_2d(tq + 2 * HALF * QS, &tmY, &full[s], yr, ktg * (QS / 4));
+            tma_load_2d(tq + 3 * HALF * QS, &tmY, &full[s], yr + HALF * 4, ktg * (QS / 4));
+          }
+          const size_t k0 = (size_t)ktg * KT;
+          bulk_load(kscales + s * KT, a.qalpha + k0, KT * 8, &full[s]);
+          bulk_load(qgs + s * KT, a.qg + k0, KT * 8, &full[s]);
+          bulk_load(qsl + s * KT, a.qslot + k0, KT, &full[s]);
         }
         if (SCALED)      // the 32 row factors of this k tile (1-D bulk copy onto the same barrier)
           asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
@@ -146,21 +194,35 @@ gemm_nt_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ 
   const int x_off = warp_m * BOX_DOUBLES + g * 4 + t;
   const int y_off = (same ? 0 : 2 * BOX_DOUBLES) + (warp_n >> 1) * BOX_DOUBLES + ((warp_n & 1) * 32 + g) * 4 + t;
 
+  // (Q fold) this thread's T rows: X rows g + 8 mi of its half, Y rows g + 8 ni of its 32 columns
+  const int tx_off = warp_m * HALF * QS + g * 4;
+  const int ty_off = (same ? 0 : 2 * HALF * QS) + (warp_n >> 1) * HALF * QS + ((warp_n & 1) * 32 + g) * 4;
+
   for (int kt = kt0; kt < kt1; ++kt) {
-    const int s = (kt - kt0) % STAGES;
-    const uint32_t ph = (uint32_t)((kt - kt0) / STAGES) & 1u;
+    const int s = (kt - kt0) % NST;
+    const uint32_t ph = (uint32_t)((kt - kt0) / NST) & 1u;
     mbar_wait(&full[s], ph);
     const double* st = tiles + (size_t)s * STAGE_DOUBLES;
     const double* xs = st + x_off;
     const double* ys = st + y_off;
     if (!(a.y_lower_tri && kt - kt0 > warp_n))
-#pragma unroll
+#pragma unroll (QS > 0 ? QUNROLL : KQ)
     for (int q = 0; q < KQ; ++q) {
       double av[8], bv[4];
 #pragma unroll
       for (int mi = 0; mi < 8; ++mi) av[mi] = xs[(q * HALF + mi * 8) * 4];
 #pragma unroll
       for (int ni = 0; ni < 4; ++ni) bv[ni] = ys[(q * HALF + ni * 8) * 4];
+      if (QS > 0) {                                   // fragment element (k = 4q + t, row r): alpha_k a + g_k T[r, slot(k)]
+        const int kk = s * KT + q * 4 + t;
+        const double al = kscales[kk], gk = qgs[kk];
+        const int sl = qsl[kk];
+        const double* tq = tqs + (size_t)s * TQ + (sl >> 2) * (HALF * 4) + (sl & 3);
+#pragma unroll
+        for (int mi = 0; mi < 8; ++mi) av[mi] = __fma_rn(gk, tq[tx_off + mi * 32], al * av[mi]);
+#pragma unroll
+        for (int ni = 0; ni < 4; ++ni) bv[ni] = __fma_rn(gk, tq[ty_off + ni * 32], al * bv[ni]);
+      }
       if (SCALED) {                                   // B fragment element (k = 4q + t, n = g): scale by w_k^2
         const double w = kscales[s * KT + q * 4 + t];
         const double w2 = w * w;
@@ -262,12 +324,15 @@ typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_
                                     CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion,
                                     CUtensorMapFloatOOBfill);
 PFN_encodeTiled g_encode = nullptr;
-std::atomic<unsigned long long> g_attr_set{0}, g_attr_set_scaled{0};
+std::atomic<unsigned long long> g_attr_set{0}, g_attr_set_scaled{0}, g_attr_set_q[4] = {};
 }  // namespace
 
 int gemm_nt_smem_bytes() { return SMEM_BYTES; }
 
-int make_q4_tensor_map(CUtensorMap* out, const double* base, int ld, long long kq_total) {
+int gemm_qfold_slots(int need) { return need <= 4 ? 4 : (need <= 16 ? (need + 3) / 4 * 4 : 0); }
+
+int make_q4_tensor_map(CUtensorMap* out, const double* base, int ld, long long kq_total, int box_kq) {
+  if (box_kq <= 0) box_kq = KQ;
   if (!g_encode) {
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
@@ -278,10 +343,10 @@ int make_q4_tensor_map(CUtensorMap* out, const double* base, int ld, long long k
     }
     g_encode = reinterpret_cast<PFN_encodeTiled>(fn);
   }
-  if (kq_total < KQ) kq_total = KQ;  // caller guarantees the allocation covers it
+  if (kq_total < box_kq) kq_total = box_kq;  // caller guarantees the allocation covers it
   cuuint64_t gdim[2] = {(cuuint64_t)ld * 4ull, (cuuint64_t)kq_total};
   cuuint64_t gstride[1] = {(cuuint64_t)ld * 32ull};
-  cuuint32_t box[2] = {(cuuint32_t)(HALF * 4), (cuuint32_t)KQ};
+  cuuint32_t box[2] = {(cuuint32_t)(HALF * 4), (cuuint32_t)box_kq};
   cuuint32_t estride[2] = {1, 1};
   CUresult r = g_encode(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 2, const_cast<double*>(base), gdim, gstride, box,
                         estride, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
@@ -312,14 +377,13 @@ int unpack_tile_major(const GemmArgs& a_in, cudaStream_t stream) {
   return 0;
 }
 
-int launch_gemm_nt(const GemmOperand& X, const GemmOperand& Y, const GemmArgs& a, cudaStream_t stream) {
-  CIP_TRY(ensure_dyn_smem((const void*)gemm_nt_kernel<false>, SMEM_BYTES, &g_attr_set));
-  if (a.kscale) CIP_TRY(ensure_dyn_smem((const void*)gemm_nt_kernel<true>, SMEM_BYTES, &g_attr_set_scaled));
+// grid of a launch: the split-K tail (b.ksplit, b.kchunk, b.tail0) and the CTA count; false: nothing to do
+static bool plan_launch(const GemmArgs& a, GemmArgs& b, long long& tiles, long long& ctas) {
   const int nsm = sm_count();      // one CTA per SM (192 KB of shared memory each): a wave is nsm tiles
   const long long all_tiles = a.lower ? (long long)a.ntm * (a.ntm + 1) / 2 : (long long)a.ntm * a.ntn;
-  const long long tiles = a.tile_count > 0 ? a.tile_count : all_tiles - a.tile_begin;
-  if (tiles <= 0 || (a.nk <= 0 && !a.Ctm)) return 0;      // (nk = 0 with tile-major output: the tiles are Cin, or zero)
-  GemmArgs b = a;
+  tiles = a.tile_count > 0 ? a.tile_count : all_tiles - a.tile_begin;
+  if (tiles <= 0 || (a.nk <= 0 && !a.Ctm)) return false;      // (nk = 0 with tile-major output: the tiles are Cin, or zero)
+  b = a;
   b.band = gemm_band();
   b.ksplit = 1;
   b.kchunk = a.nk;
@@ -341,15 +405,53 @@ int launch_gemm_nt(const GemmOperand& X, const GemmOperand& Y, const GemmArgs& a
       b.tail0 = (int)(tiles - tail);
     }
   }
-  const long long ctas = b.tail0 + (tiles - b.tail0) * b.ksplit;
-  if (a.kscale) gemm_nt_kernel<true><<<(unsigned)ctas, NUM_THREADS, SMEM_BYTES, stream>>>(X.map, Y.map, b);
-  else gemm_nt_kernel<false><<<(unsigned)ctas, NUM_THREADS, SMEM_BYTES, stream>>>(X.map, Y.map, b);
+  ctas = b.tail0 + (tiles - b.tail0) * b.ksplit;
+  return true;
+}
+
+static int finish_launch(const GemmArgs& b, long long tiles, cudaStream_t stream) {
   CIP_CHECK_LAUNCH();
   if (b.ksplit > 1) {
     splitk_reduce_kernel<<<(unsigned)(tiles - b.tail0), 256, 0, stream>>>(b);
     CIP_CHECK_LAUNCH();
   }
   return 0;
+}
+
+int launch_gemm_nt(const GemmOperand& X, const GemmOperand& Y, const GemmArgs& a, cudaStream_t stream) {
+  CIP_TRY(ensure_dyn_smem((const void*)gemm_nt_kernel<false>, SMEM_BYTES, &g_attr_set));
+  if (a.kscale) CIP_TRY(ensure_dyn_smem((const void*)gemm_nt_kernel<true>, SMEM_BYTES, &g_attr_set_scaled));
+  GemmArgs b;
+  long long tiles = 0, ctas = 0;
+  if (!plan_launch(a, b, tiles, ctas)) return 0;
+  if (a.kscale) gemm_nt_kernel<true><<<(unsigned)ctas, NUM_THREADS, SMEM_BYTES, stream>>>(X.map, Y.map, b);
+  else gemm_nt_kernel<false><<<(unsigned)ctas, NUM_THREADS, SMEM_BYTES, stream>>>(X.map, Y.map, b);
+  return finish_launch(b, tiles, stream);
+}
+
+// one Q-fold instance: QS slots per k tile
+template <int QS>
+static int launch_qfold_instance(const GemmOperand& X, const GemmOperand& T, const GemmArgs& a, cudaStream_t stream) {
+  CIP_TRY(ensure_dyn_smem((const void*)gemm_nt_kernel<false, QS>, qf_smem_bytes(QS), &g_attr_set_q[QS / 4 - 1]));
+  GemmArgs b;
+  long long tiles = 0, ctas = 0;
+  if (!plan_launch(a, b, tiles, ctas)) return 0;
+  gemm_nt_kernel<false, QS><<<(unsigned)ctas, NUM_THREADS, qf_smem_bytes(QS), stream>>>(X.map, T.map, b);
+  return finish_launch(b, tiles, stream);
+}
+
+int launch_gemm_nt_qfold(const GemmOperand& X, const GemmOperand& T, const GemmArgs& a, cudaStream_t stream) {
+  if (!a.sym || !a.lower || a.kscale || a.group || !a.qalpha || !a.qg || !a.qslot || gemm_qfold_slots(a.qs) != a.qs) {
+    set_error("launch_gemm_nt_qfold: needs a symmetric lower SYRK with qalpha / qg / qslot and qs = 4, 8, 12 or 16 "
+              "(qs = %d)", a.qs);
+    return -1;
+  }
+  switch (a.qs) {
+    case 4: return launch_qfold_instance<4>(X, T, a, stream);
+    case 8: return launch_qfold_instance<8>(X, T, a, stream);
+    case 12: return launch_qfold_instance<12>(X, T, a, stream);
+    default: return launch_qfold_instance<16>(X, T, a, stream);
+  }
 }
 
 }  // namespace cip

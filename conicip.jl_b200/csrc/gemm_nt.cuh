@@ -60,14 +60,31 @@ struct GemmArgs {
   // fields above are ignored).  tile_count must then be set.  nullptr: one product.
   const int4* group;
   int group_tiles;
+  // Q-cone scaling folded into the contraction (launch_gemm_nt_qfold): both operands are formed row by row as
+  //     Atil[k, j] = qalpha[k] * X[j, k] + qg[k] * T[j, kt * qs + qslot[k]]        (kt = k / 32)
+  // before the DMMAs, so C += Atil' Atil keeps the Gram form.  T (Q4, same ld as X) holds, for every 32-row k tile,
+  // `qs` contraction rows: one per Q cone that meets the tile (the cone's b' D A row, cone_qfold_t), zero otherwise.
+  // qalpha / qg / qslot cover every k row of the contraction (R rows: qg = 0).
+  const double* qalpha;
+  const double* qg;
+  const uint8_t* qslot;
+  int qs;
 };
 constexpr long long GEMM_WS_DOUBLES = 2048ll * 128 * 128;   // 2048 partial tiles (268 MB)
 
-// Creates a tensor map over a Q4 matrix (ld rows, kq_total quads).
-int make_q4_tensor_map(CUtensorMap* out, const double* base, int ld, long long kq_total);
+// Creates a tensor map over a Q4 matrix (ld rows, kq_total quads); box_kq: quads of contraction per TMA box
+// (0: the gemm_nt k tile, 8 quads).
+int make_q4_tensor_map(CUtensorMap* out, const double* base, int ld, long long kq_total, int box_kq = 0);
 
 // Launch on `stream`.
 int launch_gemm_nt(const GemmOperand& X, const GemmOperand& Y, const GemmArgs& a, cudaStream_t stream);
+
+// The symmetric SYRK C = Cin + Atil' Atil with the Q-cone scaling folded in (GemmArgs::qalpha ..): X is the only
+// operand (a.sym = 1, a.lower = 1), T its slot rows, mapped with box_kq = a.qs / 4.  a.qs must be a value of
+// gemm_qfold_slots: 4 (three pipeline stages), 8, 12 or 16 (two).
+int launch_gemm_nt_qfold(const GemmOperand& X, const GemmOperand& T, const GemmArgs& a, cudaStream_t stream);
+// the slot count a k tile meeting `need` distinct Q cones is given: `need` rounded up to a whole quad (0: above 16)
+int gemm_qfold_slots(int need);
 
 // Cout (Q4, ldc) <- the tile-major tiles [tile_begin, tile_begin + tile_count) of Ctm (same grid description as the launch)
 int unpack_tile_major(const GemmArgs& a, cudaStream_t stream);

@@ -86,6 +86,12 @@ int cone_maxstep(const ConeDesc& c, const double* x, const double* d, double d_s
 // Atil = F^-T A on the Q4 transposed panel (rows = columns of A, k = rows of A)
 int cone_scale_panel(const ConeDesc& c, Scaling Fi, const double* At4, double* Atil4, int ld, int m_pad,
                      int ncols, cudaStream_t st);
+// The T pass of the Q-fold SYRK (launch_gemm_nt_qfold): for every Q cone c and column j < ncols,
+//     t_c[j] = D_c * sum over the rows r of c, in row order, of b_r A[r, j]        (Fi: the inverse scaling)
+// -- the very dot product cone_scale_panel forms, 0 for a non-Woodbury block -- written to T4[j, kt * qs + slot] for
+// every 32-row k tile kt the cone meets, slot = qslot[first row of the cone in kt].  Other slots are left alone.
+int cone_qfold_t(const ConeDesc& c, Scaling Fi, const double* At4, int ld, int ncols, const uint8_t* qslot, int qs,
+                 double* T4, cudaStream_t st);
 // The same for R rows only (the diagonal pass), which also leaves e_j = round(log2 ||Atil[:, j]||) in colexp[ld]
 // (the fast SYRK's column equilibration).  colss: scale_panel_norms_chunks(m_pad) * ld doubles of scratch; ld % 256 == 0.
 int scale_panel_norms_chunks(int m_pad);

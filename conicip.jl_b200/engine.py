@@ -53,7 +53,7 @@ class Engine:
         opts.dist_chol = dist_chol
         opts.aug_rho = aug_rho
         opts.ngpus = int(ngpus)            # > 1: single-process multi-GPU handle (global vectors in and out)
-        opts.fold_scaling = int(fold_scaling)   # 0 auto, 1 always, 2 never (R-only problems: no Atil copy of A)
+        opts.fold_scaling = int(fold_scaling)   # 0 auto, 1 always, 2 never (R and Q cones: no Atil copy of A)
         opts.row_structure = int(row_structure)  # 1: singleton R rows on the diagonal, compact SYRK for the rest;
         #                                          2: also factor H as its diagonal plus the coupled block H_KK
         self.ngpus = max(1, int(ngpus))

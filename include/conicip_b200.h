@@ -66,10 +66,15 @@ typedef struct cip_options {
                            calling thread's single call -- the reference calls its kktsolver once from one process
                            (src/ConicIP.jl:667), so this is what `kktsolver = kktsolver_b200(ngpus = 8)` uses.
                            Every entry point below then takes and returns GLOBAL vectors; 0 / 1 = one device */
-  int    fold_scaling;  /* K = R^m only (every block of F diagonal): apply W^-2 to the operand fragments inside the
-                           SYRK instead of materialising Atil = F^-T A (src/kktsolvers.jl:33) -- halves the resident
-                           bytes (no second copy of A), costs ~1.5 % of the SYRK.  0: auto (fold when the second copy
-                           would not fit in free device memory), 1: always, 2: never */
+  int    fold_scaling;  /* K of R and Q cones (no S cones): form Atil = F^-T A (src/kktsolvers.jl:33) inside the SYRK
+                           instead of materialising it, so no second copy of A is kept.  K = R^m: W^-2 on the operand
+                           fragments (~1.5 % of the SYRK).  Q cones: each row is formed in registers as
+                           alpha_k a_k + g_k t_c from a per-call pass that stores the cone's row t_c = D_c b_c' A_c once
+                           per 32-row tile it meets -- qs rows per tile, qs = the most Q cones a tile meets rounded up to
+                           4, 8, 12 or 16, i.e. qs/32 of A (12.5 % for cones of dimension >= 31); ~+28 % of the SYRK
+                           (C3, one B200).  Cones of dimension 1 or 2, which crowd more than 16 cones into a tile, keep
+                           Atil.  0: auto (fold when the second copy would not fit in free device memory), 1: always where
+                           possible, 2: never */
   int    row_structure; /* single-device handles: 1 = classify the rows of A at LEVEL 1 and exploit them when forming
                            H (the reference keeps A sparse through this product, src/kktsolvers.jl:289-290).  R rows
                            with one non-zero go straight onto the diagonal of H; the other rows ("rest": every Q / S
