@@ -19,7 +19,7 @@ CONE_CODE = {"R": CONE_R, "Q": CONE_Q, "S": CONE_S}
 class Options(C.Structure):
     _fields_ = [("struct_size", C.c_int), ("device", C.c_int), ("reg_delta", C.c_double),
                 ("reg_eps_G", C.c_double), ("q_kind", C.c_int), ("verbose", C.c_int), ("dist_chol", C.c_int), ("aug_rho", C.c_double),
-                ("ngpus", C.c_int), ("fold_scaling", C.c_int), ("row_structure", C.c_int)]
+                ("ngpus", C.c_int), ("fold_scaling", C.c_int), ("row_structure", C.c_int), ("eliminate_y", C.c_int)]
 
 
 class StructureInfo(C.Structure):
@@ -30,6 +30,10 @@ class StructureInfo(C.Structure):
 class SplitInfo(C.Structure):
     _fields_ = [("struct_size", C.c_int), ("enabled", C.c_int), ("coupled_cols", C.c_int), ("diagonal_cols", C.c_int),
                 ("cols_from_rest", C.c_int), ("cols_from_Q", C.c_int), ("cols_from_G", C.c_int)]
+
+
+class KktFormInfo(C.Structure):
+    _fields_ = [("struct_size", C.c_int), ("eliminate_y", C.c_int), ("automatic", C.c_int)]
 
 
 class Stats(C.Structure):
@@ -101,7 +105,9 @@ SIGNATURES = {
     "cip_stats": (C.c_int, [C.c_void_p, C.POINTER(Stats)]),
     "cip_structure_info": (C.c_int, [C.c_void_p, C.POINTER(StructureInfo)]),
     "cip_split_info": (C.c_int, [C.c_void_p, C.POINTER(SplitInfo)]),
+    "cip_kkt_form_info": (C.c_int, [C.c_void_p, C.POINTER(KktFormInfo)]),
     "cip_get_H": (C.c_int, [C.c_void_p, _P, C.c_int]),
+    "cip_get_M": (C.c_int, [C.c_void_p, _P, C.c_int]),
     "cip_form_H": (C.c_int, [C.c_void_p]),
     "cip_factor_H": (C.c_int, [C.c_void_p]),
     "cip_solve_H": (C.c_int, [C.c_void_p, _P, _P]),

@@ -128,8 +128,10 @@ int vec_out_done(cip_engine* h, double* dst, const double* produced, size_t n) {
   return stage_out(h, dst, produced, n);
 }
 
-// give-up flag of the persistent sweeps with H's factor (none when row_structure = 2 left K empty)
+// give-up flag of the persistent sweeps with H's factor (none when row_structure = 2 left K empty; M's factor in the
+// m-space form)
 int* h_sweep_err(const cip_engine* h) {
+  if (h->ey.on) return h->ey.chol.sweep_err;
   return h->rs.sp.on ? (h->rs.sp.nK > 0 ? h->rs.sp.chol.sweep_err : nullptr) : h->cholH.sweep_err;
 }
 
@@ -302,6 +304,12 @@ int form_H(cip_engine* h) {
   }
   cudaStream_t s = h->stream;
   CIP_CUDA(cudaEventRecord(h->ev[0], s));
+  if (h->ey.on) {                       // m-space form: M = C + F'F (delta is part of D; the SYRK ran at cip_create)
+    CIP_TRY(ey_form_M(h));
+    CIP_CUDA(cudaEventRecord(h->ev[3], s));
+    h->st.syrk_flops = 0.0;
+    return 0;
+  }
   if (h->rs.on) {
     CIP_TRY(structure_form_H(h));
     if (h->opt.reg_delta != 0.0) {
@@ -375,7 +383,10 @@ int factor_H(cip_engine* h) {
   cudaStream_t s = h->stream;
   // row_structure = 2: H_KK is factored on its own plan and D by split_factor; the Schur block below runs on Z_K
   const RowStructure::Split& sp = h->rs.sp;
-  if (sp.on) {
+  const EliminateY& ey = h->ey;
+  if (ey.on) {
+    CIP_TRY(chol_factor(ey.chol, s));
+  } else if (sp.on) {
     CIP_TRY(split_factor(h));
   } else {
     // block-cyclic distributed factorisation when A is row-sharded (every rank holds the reduced H);
@@ -401,12 +412,13 @@ int factor_H(cip_engine* h) {
     // Two-level like the Cholesky: inside an outer panel of four 128-column panels every panel is solved against
     // inv(L_jj) and applied to the rest of the outer panel only; everything right of the outer panel gets ONE update
     // with K = 512, which amortises the C-tile read-modify-write that holds K = 128 tiles at a third of the pipe.
-    // (row_structure = 2: Z_K = G_K L_KK^-T over the K columns)
-    const CholPlan& L = sp.on ? sp.chol : h->cholH;
-    double* Z = sp.on ? sp.ZK4 : h->Z4;
-    const GemmOperand& mapZ = sp.on ? sp.mapZK : h->mapZ;
-    const int np = (sp.on ? sp.nK_pad : h->n_pad) / TILE, ptiles = h->p_pad / TILE;
-    if (np > 0) CIP_TRY(vec_copy(Z, sp.on ? sp.GK4 : h->G4, (size_t)h->p_pad * np * TILE, s));
+    // (row_structure = 2: Z_K = G_K L_KK^-T over the K columns; m-space form: Z = E' L^-T with L = chol(M),
+    //  S = P - Z Z')
+    const CholPlan& L = ey.on ? ey.chol : sp.on ? sp.chol : h->cholH;
+    double* Z = ey.on ? ey.Z4 : sp.on ? sp.ZK4 : h->Z4;
+    const GemmOperand& mapZ = ey.on ? ey.mapZ : sp.on ? sp.mapZK : h->mapZ;
+    const int np = (ey.on ? ey.mM : sp.on ? sp.nK_pad : h->n_pad) / TILE, ptiles = h->p_pad / TILE;
+    if (np > 0) CIP_TRY(vec_copy(Z, ey.on ? ey.Et4 : sp.on ? sp.GK4 : h->G4, (size_t)h->p_pad * np * TILE, s));
     auto z_trsm = [&](int jb) -> int {                       // Z[:, jb] <- Z[:, jb] inv(L_jj)'
       GemmArgs t{};
       t.lower = 0; t.ntm = ptiles; t.ntn = 1; t.sym = 0;
@@ -435,7 +447,7 @@ int factor_H(cip_engine* h) {
     GemmArgs a{};
     a.lower = 1; a.ntm = a.ntn = ptiles; a.sym = 1;
     a.x_row0 = a.y_row0 = 0; a.x_kq0 = a.y_kq0 = 0;
-    a.Cin = h->Sbase4; a.Cout = h->S4; a.ldc = h->p_pad; a.c_row0 = a.c_col0 = 0; a.alpha = 1.0;
+    a.Cin = h->Sbase4; a.Cout = h->S4; a.ldc = h->p_pad; a.c_row0 = a.c_col0 = 0; a.alpha = ey.on ? -1.0 : 1.0;
     a.ws = h->gemm_ws; a.ws_doubles = GEMM_WS_DOUBLES;
     if (sp.on && sp.g_in_D) {
       // + G_D diag(1/h) G_D': the folded-scaling SYRK over all of G with kscale = h^-1/2 on D and 0 on K
@@ -462,7 +474,7 @@ int factor_H(cip_engine* h) {
   cudaEventElapsedTime(&ms, h->ev[3], h->ev[4]); h->st.ms_chol = ms;
   cudaEventElapsedTime(&ms, h->ev[4], h->ev[5]); h->st.ms_schur = ms;
   cudaGetLastError();
-  const double nf = sp.on ? sp.nK : h->n;
+  const double nf = ey.on ? h->m : sp.on ? sp.nK : h->n;
   h->st.chol_flops = nf * nf * nf / 3.0;
   h->st.factors++;
   h->have_factor = true;
@@ -474,12 +486,13 @@ int factor_H(cip_engine* h) {
     hinfo[0] = col < h->n ? col + 1 : 0;
   }
   if (hinfo[0] != 0) {
-    set_error("Cholesky of H failed: non-positive pivot at column %d", hinfo[0]);
+    if (ey.on) set_error("Cholesky of M = F'F + A D^-1 A' failed: non-positive pivot at row %d of A", hinfo[0]);
+    else set_error("Cholesky of H failed: non-positive pivot at column %d", hinfo[0]);
     return hinfo[0];
   }
   if (hinfo[1] != 0) {
     set_error("Cholesky of the Schur complement failed: non-positive pivot at row %d", hinfo[1]);
-    return h->n + hinfo[1];
+    return (ey.on ? h->m : h->n) + hinfo[1];
   }
   return 0;
 }
@@ -766,6 +779,15 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
     CIP_TRY(engine_decide_fold(h, true, (size_t)(h->m_pad + h->aug_rows) * h->n_pad, &h->fold, at4_ahead));
     if (h->fold) h->qs = qs;
   }
+  // m-space form (opts.eliminate_y): decided against the n-space form as it now stands, before any of its buffers
+  CIP_TRY(ey_decide(h, shard, Q, ldq, Qs));
+  const bool ey = h->ey.on;
+  if (ey) {
+    h->fold = false;
+    h->qs = 0;
+    h->aug_rho = 0.0;                   // M is positive definite whenever F'F is: no augmentation
+    h->aug_rows = 0;
+  }
   // rows of the contraction the handle keeps in At4 and in the scaling arrays: a folded R + Q handle appends the
   // sqrt(rho) G rows to A there, with the row factor 1 and no cone term (qfold_alloc)
   const size_t k_rows = (size_t)h->m_pad + (h->qs > 0 ? h->aug_rows : 0);
@@ -781,22 +803,24 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   h->Fi.Ri = h->F.Ri;
 
   // ---- matrices
-  if (!(h->rs.on && As)) CIP_TRY(dev_alloc(h, &h->At4, k_rows * h->n_pad));   // CSC input with row structure: never dense
+  if (!(h->rs.on && As) && !ey) CIP_TRY(dev_alloc(h, &h->At4, k_rows * h->n_pad));   // CSC input with row structure: never dense
   if (h->qs > 0) CIP_TRY(qfold_alloc(h, qslot));
-  if (!h->rs.on && !h->fold) CIP_TRY(fast_syrk_plan(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0));
+  if (!h->rs.on && !h->fold && !ey) CIP_TRY(fast_syrk_plan(h, slist.empty() && qlist.empty() && h->aug_rows == 0 && m > 0));
   if (h->fast.on) CIP_TRY(dev_alloc(h, &h->Atil4, fast_syrk_atil_doubles(h)));
-  else if (!h->fold && !h->rs.on) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
+  else if (!h->fold && !h->rs.on && !ey) CIP_TRY(dev_alloc(h, &h->Atil4, (size_t)(h->m_pad + h->aug_rows) * h->n_pad));
   // row_structure = 2 keeps no n_pad^2 buffer: dense Q is staged in Qq4 until split_build has gathered Q_KK
   const bool split = h->rs.sp.on;
-  if (!split || (!Qs && h->opt.q_kind == 0)) CIP_TRY(dev_alloc(h, &h->Qq4, nn));
-  if (!split) CIP_TRY(dev_alloc(h, &h->H4, nn));
+  // the m-space form keeps none of Qq4, H4, Winv (ey_create)
+  if (!ey && (!split || (!Qs && h->opt.q_kind == 0))) CIP_TRY(dev_alloc(h, &h->Qq4, nn));
+  if (!split && !ey) CIP_TRY(dev_alloc(h, &h->H4, nn));
   CIP_TRY(dev_alloc(h, &h->gemm_ws, (size_t)GEMM_WS_DOUBLES));
-  if (!split) CIP_TRY(dev_alloc(h, &h->Winv, (size_t)h->n_pad * TILE));
+  if (!split && !ey) CIP_TRY(dev_alloc(h, &h->Winv, (size_t)h->n_pad * TILE));
   CIP_TRY(dev_alloc(h, &h->info, 4));
   cudaStream_t s = h->stream;
 
-  // Q
-  if (Qs && split) {
+  // Q (m-space form: its diagonal went to ey_decide)
+  if (ey) {
+  } else if (Qs && split) {
     CIP_TRY(split_classify_csc_Q(h, Qs));
   } else if (Qs) {
     CIP_TRY(upload_csc(h, h->Qq4, h->n_pad, Qs, 0));
@@ -835,8 +859,8 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   }
   if (h->Qq4) CIP_TRY(add_diag_q4(h->Qq4, h->n_pad, n, h->n_pad, 1.0, 1, s));  // identity on the padding
 
-  // A (transposed into Q4: rows = columns of A)
-  if (m > 0) {
+  // A (transposed into Q4: rows = columns of A; the m-space form keeps rows as rows, ey_create)
+  if (m > 0 && !ey) {
     if (!A && !As) { set_error("A is null"); return -1; }
     if (As && h->rs.on) {
       CIP_TRY(structure_build_csc(h, As));
@@ -859,8 +883,8 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
     }
     if (h->rs.on && !As) CIP_TRY(structure_build_dense(h));
   }
-  if (h->rs.on) {
-    // (structure_finish makes the operand map of the rest rows)
+  if (h->rs.on || ey) {
+    // (structure_finish makes the operand map of the rest rows; ey_create the one of A4)
   } else if (h->fold && h->qs > 0) {
     CIP_TRY(make_q4_tensor_map(&h->mapAt.map, h->At4, h->n_pad, (h->m_pad + h->aug_rows) / 4));
     CIP_TRY(make_q4_tensor_map(&h->mapTq.map, h->Tq4, h->n_pad, (long long)(h->m_pad + h->aug_rows) / 32 * h->qs / 4,
@@ -873,14 +897,14 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
   } else if (h->m_pad + h->aug_rows > 0) {
     CIP_TRY(make_q4_tensor_map(&h->mapAtil.map, h->Atil4, h->n_pad, (h->m_pad + h->aug_rows) / 4));
   }
-  if (!split) CIP_TRY(chol_make_plan(&h->cholH, h->H4, h->n_pad, h->Winv, h->info));
+  if (!split && !ey) CIP_TRY(chol_make_plan(&h->cholH, h->H4, h->n_pad, h->Winv, h->info));
 
   // G
   if (p > 0) {
     if (!G && !Gs) { set_error("G is null"); return -1; }
     const size_t pn = (size_t)h->p_pad * h->n_pad;
     CIP_TRY(dev_alloc(h, &h->G4, pn));
-    if (!split) CIP_TRY(dev_alloc(h, &h->Z4, pn));
+    if (!split && !ey) CIP_TRY(dev_alloc(h, &h->Z4, pn));
     CIP_TRY(dev_alloc(h, &h->S4, (size_t)h->p_pad * h->p_pad));
     CIP_TRY(dev_alloc(h, &h->Sbase4, (size_t)h->p_pad * h->p_pad));
     CIP_TRY(dev_alloc(h, &h->WinvS, (size_t)h->p_pad * TILE));
@@ -905,10 +929,14 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
                                  sqrt(h->aug_rho), s));
     CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, p, h->p_pad, 1.0, 1, s));
     if (h->opt.reg_eps_G != 0.0) CIP_TRY(add_diag_q4(h->Sbase4, h->p_pad, 0, p, h->opt.reg_eps_G, 1, s));
-    if (!split) CIP_TRY(make_q4_tensor_map(&h->mapZ.map, h->Z4, h->p_pad, h->n_pad / 4));
+    if (!split && !ey) CIP_TRY(make_q4_tensor_map(&h->mapZ.map, h->Z4, h->p_pad, h->n_pad / 4));
     CIP_TRY(chol_make_plan(&h->cholS, h->S4, h->p_pad, h->WinvS, h->info + 1));
   }
   if (h->rs.on) CIP_TRY(structure_finish(h));
+  if (ey) {
+    if (!A && !As) { set_error("A is null"); return -1; }
+    CIP_TRY(ey_create(h, A, lda, As, G, ldg, Gs));
+  }
 
   // ---- work vectors
   for (auto& v : h->nv) CIP_TRY(dev_alloc(h, &v, h->n_pad + 4));
@@ -925,6 +953,9 @@ int create_body(cip_engine* h, int n, int m, int p, const double* Q, int ldq, co
 }  // namespace
 
 namespace cip {
+int engine_upload_csc(cip_engine* h, double* dst, int ld, const cip_csc* M, int transpose) {
+  return upload_csc(h, dst, ld, M, transpose);
+}
 int engine_create_single(cip_handle* out, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,
                          const double* G, int ldg, const cip_csc* Qs, const cip_csc* As, const cip_csc* Gs,
                          int ncones, const int* cone_type, const int* cone_dim, const cip_options* opts) {
@@ -938,11 +969,16 @@ namespace {
 bool wants_multi(const cip_options* opts) {
   return opts && (size_t)opts->struct_size >= offsetof(cip_options, ngpus) + sizeof(int) && opts->ngpus > 1;
 }
-// a sharded handle with opts.row_structure = 1: refused before any device work
+// a sharded handle with opts.row_structure = 1 or opts.eliminate_y = 1: refused before any device work
 bool reject_sharded_structure(const cip_options* opts) {
   if (opts && (size_t)opts->struct_size >= offsetof(cip_options, row_structure) + sizeof(int) &&
       opts->row_structure != 0) {
     set_error("row_structure is supported on single-device handles only (ngpus = %d)", opts->ngpus);
+    return true;
+  }
+  if (opts && (size_t)opts->struct_size >= offsetof(cip_options, eliminate_y) + sizeof(int) &&
+      opts->eliminate_y == 1) {
+    set_error("eliminate_y = 1: the m-space form is supported on single-device handles only (ngpus = %d)", opts->ngpus);
     return true;
   }
   return false;
@@ -1017,6 +1053,7 @@ int cip_destroy(cip_handle h) {
   chol_free_plan(&h->cholH);
   chol_free_plan(&h->cholS);
   chol_free_plan(&h->rs.sp.chol);
+  chol_free_plan(&h->ey.chol);
   if (h->Hp) cudaFree(h->Hp);
   if (h->d_sws) cudaFree(h->d_sws);
   if (h->cs) cudaStreamDestroy(h->cs);
@@ -1047,6 +1084,7 @@ int cip_comm_init(cip_handle h, int nranks, int rank, const unsigned char id[128
   if (h->multi) { set_error("cip_comm_init: a single-process multi-GPU handle (opts.ngpus) owns its communicators"); return -1; }
   if (nranks <= 1) return 0;
   if (h->rs.on) { set_error("cip_comm_init: row_structure is supported on single-device handles only"); return -1; }
+  if (h->ey.on) { set_error("cip_comm_init: eliminate_y (the m-space form) is supported on single-device handles only"); return -1; }
   const NcclApi* api = nccl_api();
   if (!api) return -1;
   NcclId nid;
@@ -1209,45 +1247,50 @@ int cip_solve(cip_handle h, const double* ry, const double* rw, const double* rv
   if (h->p) CIP_TRY(stage_in(h, h->pv[0], rw, h->p));
   CIP_TRY(vec_in(h, h->mv[0], rv, h->m, &rvp));
   double* dvp = (dv != rv) ? vec_out(h, h->mv[5], dv, h->m) : h->mv[5];
-  // t1 = F^-T (F^-T v)                                   (src/kktsolvers.jl:326)
-  // (= inv(F'F) v; for the non-symmetric VecCongurance blocks this is inv(F) inv(F)' v, which is
-  //  what the 3x3 system requires -- the reference's pivot is only right for symmetric F, SURVEY 3b)
-  CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, rvp, h->mv[2], nullptr, h->mv[1], s));
-  // rhs = y + A' t1                                      (:327); single GPU: y is added in the mat-vec's second pass
-  if (h->rs.on) {
-    CIP_TRY(structure_AT(h, h->nv[2], h->mv[2], ryp, 0));
-  } else if (h->m && !h->comm) {
-    CIP_TRY(q4_mv_rows(h->nv[2], h->At4, h->n_pad, h->n, h->m, h->mv[2], h->partial, h->partial_cap, s, ryp));
+  if (h->ey.on) {
+    // m-space form: a = D^-1 (ry - G'b + A'c) after the m x m and p x p solves (eliminate_y.cu)
+    CIP_TRY(ey_solve(h, ryp, h->pv[0], rvp, h->nv[5], h->pv[4], dvp));
   } else {
-    if (h->m) CIP_TRY(q4_mv_rows(h->nv[1], h->At4, h->n_pad, h->n, h->m, h->mv[2], h->partial, h->partial_cap, s));
-    else CIP_TRY(fill_zero(h->nv[1], h->n, s));
-    CIP_TRY(allreduce(h, h->nv[1], h->n));
-    CIP_TRY(vec_axpby(h->nv[2], 1.0, ryp, 1.0, h->nv[1], h->n, s));
-  }
-  if (h->aug_rows > 0) {        // rhs += rho G' rw  (same (dy, dw) as the unaugmented system)
-    CIP_TRY(q4_mv_k(h->nv[4], h->G4, h->p_pad, h->p, h->n, h->pv[0], s));
-    CIP_TRY(vec_axpby(h->nv[2], 1.0, h->nv[2], h->aug_rho, h->nv[4], h->n, s));
-  }
-  // 2x2 solve with H = L L' and the Schur complement on G (:299)
-  if (h->rs.sp.on) {
-    CIP_TRY(split_solve(h, h->nv, h->pv, 0, h->p > 0));
-  } else {
-    CIP_TRY(chol_fwd(h->cholH, h->nv[2], h->nv[3], s));
-    if (h->p) {
-      CIP_TRY(q4_mv_rows(h->pv[1], h->Z4, h->p_pad, h->p, h->n, h->nv[3], h->partial, h->partial_cap, s));
-      CIP_TRY(vec_axpby(h->pv[2], 1.0, h->pv[1], -1.0, h->pv[0], h->p, s));
-      CIP_TRY(chol_fwd(h->cholS, h->pv[2], h->pv[3], s));
-      CIP_TRY(chol_bwd(h->cholS, h->pv[3], h->pv[4], s));
-      CIP_TRY(q4_mv_k(h->nv[4], h->Z4, h->p_pad, h->p, h->n, h->pv[4], s));
-      CIP_TRY(vec_axpby(h->nv[3], 1.0, h->nv[3], -1.0, h->nv[4], h->n, s));
+    // t1 = F^-T (F^-T v)                                   (src/kktsolvers.jl:326)
+    // (= inv(F'F) v; for the non-symmetric VecCongurance blocks this is inv(F) inv(F)' v, which is
+    //  what the 3x3 system requires -- the reference's pivot is only right for symmetric F, SURVEY 3b)
+    CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, rvp, h->mv[2], nullptr, h->mv[1], s));
+    // rhs = y + A' t1                                      (:327); single GPU: y is added in the mat-vec's second pass
+    if (h->rs.on) {
+      CIP_TRY(structure_AT(h, h->nv[2], h->mv[2], ryp, 0));
+    } else if (h->m && !h->comm) {
+      CIP_TRY(q4_mv_rows(h->nv[2], h->At4, h->n_pad, h->n, h->m, h->mv[2], h->partial, h->partial_cap, s, ryp));
+    } else {
+      if (h->m) CIP_TRY(q4_mv_rows(h->nv[1], h->At4, h->n_pad, h->n, h->m, h->mv[2], h->partial, h->partial_cap, s));
+      else CIP_TRY(fill_zero(h->nv[1], h->n, s));
+      CIP_TRY(allreduce(h, h->nv[1], h->n));
+      CIP_TRY(vec_axpby(h->nv[2], 1.0, ryp, 1.0, h->nv[1], h->n, s));
     }
-    CIP_TRY(chol_bwd(h->cholH, h->nv[3], h->nv[5], s));
-  }
-  // dv = t1 - F^-T F^-T (A dy)                           (:328)
-  if (h->m) {
-    if (h->rs.on) CIP_TRY(structure_A(h, h->mv[3], h->nv[5], 0));
-    else CIP_TRY(q4_mv_k(h->mv[3], h->At4, h->n_pad, h->n, h->m, h->nv[5], s));
-    CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, h->mv[3], dvp, h->mv[2], h->mv[1], s));   // t1 - (F'F)^-1 (A dy)
+    if (h->aug_rows > 0) {        // rhs += rho G' rw  (same (dy, dw) as the unaugmented system)
+      CIP_TRY(q4_mv_k(h->nv[4], h->G4, h->p_pad, h->p, h->n, h->pv[0], s));
+      CIP_TRY(vec_axpby(h->nv[2], 1.0, h->nv[2], h->aug_rho, h->nv[4], h->n, s));
+    }
+    // 2x2 solve with H = L L' and the Schur complement on G (:299)
+    if (h->rs.sp.on) {
+      CIP_TRY(split_solve(h, h->nv, h->pv, 0, h->p > 0));
+    } else {
+      CIP_TRY(chol_fwd(h->cholH, h->nv[2], h->nv[3], s));
+      if (h->p) {
+        CIP_TRY(q4_mv_rows(h->pv[1], h->Z4, h->p_pad, h->p, h->n, h->nv[3], h->partial, h->partial_cap, s));
+        CIP_TRY(vec_axpby(h->pv[2], 1.0, h->pv[1], -1.0, h->pv[0], h->p, s));
+        CIP_TRY(chol_fwd(h->cholS, h->pv[2], h->pv[3], s));
+        CIP_TRY(chol_bwd(h->cholS, h->pv[3], h->pv[4], s));
+        CIP_TRY(q4_mv_k(h->nv[4], h->Z4, h->p_pad, h->p, h->n, h->pv[4], s));
+        CIP_TRY(vec_axpby(h->nv[3], 1.0, h->nv[3], -1.0, h->nv[4], h->n, s));
+      }
+      CIP_TRY(chol_bwd(h->cholH, h->nv[3], h->nv[5], s));
+    }
+    // dv = t1 - F^-T F^-T (A dy)                           (:328)
+    if (h->m) {
+      if (h->rs.on) CIP_TRY(structure_A(h, h->mv[3], h->nv[5], 0));
+      else CIP_TRY(q4_mv_k(h->mv[3], h->At4, h->n_pad, h->n, h->m, h->nv[5], s));
+      CIP_TRY(cone_apply_invsq(h->cd, h->F, h->Fi, h->mv[3], dvp, h->mv[2], h->mv[1], s));   // t1 - (F'F)^-1 (A dy)
+    }
   }
   CIP_CUDA(cudaEventRecord(h->ev[7], s));
   CIP_TRY(stage_out(h, dy, h->nv[5], h->n));
@@ -1286,6 +1329,13 @@ int cip_solve_multi(cip_handle h, int nrhs, const double* ry, int ldy, const dou
   auto colw = [](double* p, int k, int ld) { return p ? p + (size_t)k * ld : nullptr; };
   if (h->multi) return multi_solve_multi(h, nrhs, ry, ldy, rw, ldw, rv, ldv, dy, dw, dv);
   if (!h->have_factor) { set_error("cip_solve_multi before cip_factor"); return -1; }
+  if (h->ey.on) {
+    // m-space form: column by column (each column is exactly cip_solve's)
+    for (int k = 0; k < nrhs; ++k)
+      CIP_TRY(cip_solve(h, col(ry, k, ldy), col(rw, k, ldw), col(rv, k, ldv), colw(dy, k, ldy), colw(dw, k, ldw),
+                        colw(dv, k, ldv)));
+    return 0;
+  }
   int k = 0;
   for (; k + 1 < nrhs; k += 2) {
     if (!h->nv2[0]) {
@@ -1387,7 +1437,9 @@ int cip_solve_H(cip_handle h, const double* rhs, double* x) {
   cudaStream_t s = h->stream;
   CIP_TRY(stage_in(h, h->nv[2], rhs, h->n));
   CIP_CUDA(cudaEventRecord(h->ev[6], s));
-  if (h->rs.sp.on) {
+  if (h->ey.on) {
+    CIP_TRY(ey_solve_H(h, h->nv[2], h->nv[5]));
+  } else if (h->rs.sp.on) {
     CIP_TRY(split_solve(h, h->nv, h->pv, 0, false));
   } else {
     CIP_TRY(chol_fwd(h->cholH, h->nv[2], h->nv[3], s));
@@ -1405,16 +1457,18 @@ int cip_mul_A(cip_handle h, int trans, const double* x, double* y) {
   cudaStream_t s = h->stream;
   if (!trans) {
     const double* xp;
-    CIP_TRY(vec_in(h, h->nv[6], x, h->n, &xp));
+    CIP_TRY(vec_in(h, h->nv[6], x, h->n, &xp, /*padded=*/h->ey.on));
     double* yp = vec_out(h, h->mv[6], y, h->m);
-    if (h->rs.on) CIP_TRY(structure_A(h, yp, xp, 0));
+    if (h->ey.on) CIP_TRY(q4_mv_rows(yp, h->ey.A4, h->ey.mM, h->m, h->n, xp, h->partial, h->partial_cap, s));
+    else if (h->rs.on) CIP_TRY(structure_A(h, yp, xp, 0));
     else CIP_TRY(q4_mv_k(yp, h->At4, h->n_pad, h->n, h->m, xp, s));
     CIP_TRY(vec_out_done(h, y, yp, h->m));
   } else {
     const double* xp;
     CIP_TRY(vec_in(h, h->mv[6], x, h->m, &xp, /*padded=*/true));
     double* yp = vec_out(h, h->nv[6], y, h->n);
-    if (h->rs.on) CIP_TRY(structure_AT(h, yp, xp, nullptr, 0));
+    if (h->ey.on) CIP_TRY(q4_mv_k(yp, h->ey.A4, h->ey.mM, h->m, h->n, xp, s));
+    else if (h->rs.on) CIP_TRY(structure_AT(h, yp, xp, nullptr, 0));
     else if (h->m) CIP_TRY(q4_mv_rows(yp, h->At4, h->n_pad, h->n, h->m, xp, h->partial, h->partial_cap, s));
     else CIP_TRY(fill_zero(yp, h->n, s));
     CIP_TRY(allreduce(h, yp, h->n));
@@ -1453,7 +1507,8 @@ int cip_mul_Q(cip_handle h, const double* x, double* y) {
   const double* xp;
   CIP_TRY(vec_in(h, h->nv[6], x, h->n, &xp, /*padded=*/true));
   double* yp = (y != x) ? vec_out(h, h->nv[7], y, h->n) : h->nv[7];
-  if (h->rs.sp.on) CIP_TRY(split_mul_Q(h, yp, xp));
+  if (h->ey.on) CIP_TRY(ey_mul_Q(h, yp, xp));
+  else if (h->rs.sp.on) CIP_TRY(split_mul_Q(h, yp, xp));
   else CIP_TRY(q4_mv_rows(yp, h->Qq4, h->n_pad, h->n, h->n, xp, h->partial, h->partial_cap, s));
   CIP_TRY(vec_out_done(h, y, yp, h->n));
   return finish(h);
@@ -1515,9 +1570,47 @@ int cip_split_info(cip_handle h, cip_split_t* out) {
   return 0;
 }
 
+int cip_kkt_form_info(cip_handle h, cip_kkt_form_t* out) {
+  CIP_TRY(check(h));
+  if (!out || out->struct_size < (int)sizeof(int)) {
+    set_error("cip_kkt_form_info: out->struct_size must be set");
+    return -1;
+  }
+  cip_kkt_form_t r{};
+  r.struct_size = out->struct_size;
+  r.eliminate_y = h->ey.on ? 1 : 0;      // (a multi-GPU front never has it on)
+  r.automatic = h->ey.automatic ? 1 : 0;
+  memcpy(out, &r, std::min<size_t>(sizeof(r), (size_t)out->struct_size));
+  return 0;
+}
+
+int cip_get_M(cip_handle h, double* out, int ldo) {
+  CIP_TRY(check(h));
+  if (!h->ey.on) {
+    set_error("cip_get_M: this handle factors the n x n H (eliminate_y is off); use cip_get_H");
+    return -1;
+  }
+  if (!out || ldo < h->m) { set_error("cip_get_M: bad output (ldo = %d < m = %d)", ldo, h->m); return -1; }
+  if (h->m == 0) return 0;
+  double* tmp = nullptr;
+  CIP_CUDA(cudaMalloc(&tmp, (size_t)h->m * h->m * 8));
+  const int rc = ey_get_M(h, tmp);
+  if (rc != 0) cudaFree(tmp);
+  CIP_TRY(rc);
+  CIP_CUDA(cudaMemcpy2DAsync(out, (size_t)ldo * 8, tmp, (size_t)h->m * 8, (size_t)h->m * 8, h->m, cudaMemcpyDefault,
+                             h->stream));
+  CIP_CUDA(cudaStreamSynchronize(h->stream));
+  cudaFree(tmp);
+  return 0;
+}
+
 int cip_get_H(cip_handle h, double* out, int ldo) {
   CIP_TRY(check(h));
   if (h->multi) return multi_simple(h, 3, out, ldo);
+  if (h->ey.on) {
+    set_error("cip_get_H: this handle eliminates y (eliminate_y) and has no n x n H; cip_get_M returns M = F'F + A D^-1 A'");
+    return -1;
+  }
   double* tmp = nullptr;
   CIP_CUDA(cudaMalloc(&tmp, (size_t)h->n * h->n * 8));
   const int rc = h->rs.sp.on ? split_get_H(h, tmp) : unpack_rows_q4(tmp, h->n, h->H4, h->n_pad, h->n, h->n, h->stream);

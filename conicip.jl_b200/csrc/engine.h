@@ -76,6 +76,25 @@ struct FastSyrk {
   double* M2 = nullptr;        // the level-2 sub-product tiles of one level-1 product, every pair (two != 0)
   int4* table = nullptr;       // GemmArgs::group entries: the leaves, the products of depth 0, 1, ..., the level-2 ones
 };
+
+// cip_options.eliminate_y (eliminate_y.cu): Q + delta I = D is diagonal and positive, so y is eliminated instead of v
+// and the m x m matrix M = F'F + A D^-1 A' is factored.  A is kept once, as A4 (Q4, rows = rows of A, ld = mM,
+// k = columns); C = A D^-1 A', E' = G D^-1 A' and P = G D^-1 G' are formed once at cip_create.  None of At4, Atil4,
+// Qq4, H4, Z4 (n-space) exist.
+struct EliminateY {
+  bool on = false, automatic = false;
+  int mM = 0;                       // round_up(m, TILE): order of the Q4 buffers of M
+  double* A4 = nullptr;             // mM x n_pad, k = columns of A
+  double *dinv = nullptr, *kscale = nullptr, *qdiag = nullptr;   // [n_pad + 4]: 1/D, D^-1/2, the diagonal of Q
+  double *C4 = nullptr, *M4 = nullptr, *Winv = nullptr;         // mM^2, mM^2 (M, then L), mM * TILE
+  double *Et4 = nullptr, *Z4 = nullptr;                          // p_pad x mM: E' = G D^-1 A', Z = E' L^-T
+  double *W = nullptr, *qbb = nullptr;                           // [r_total] W = R R' per S cone, [ncones] b'b
+  int* sidx = nullptr;              // [ncones]: position of an S cone in the S list (-1 otherwise)
+  double* v[4] = {};                // mM + 4 each: r1, t, c, scratch
+  std::vector<double> hq;           // LEVEL 1 only: the diagonal of Q (host), until ey_create uploads it
+  GemmOperand mapA{}, mapZ{};
+  CholPlan chol{};
+};
 }  // namespace cip
 
 struct cip_engine {
@@ -117,6 +136,7 @@ struct cip_engine {
   double aug_rho = 0.0;
   cip::RowStructure rs;    // opts.row_structure: At4 / Atil4 are not allocated
   cip::FastSyrk fast;      // the Winograd SYRK of form_H (sized at cip_create, dropped when a communicator is attached)
+  cip::EliminateY ey;      // opts.eliminate_y: the m-space form (no n_pad^2 buffer, no At4)
   std::vector<void*> owned;   // further device buffers freed by cip_destroy
   // work vectors
   double* nv[NV] = {};
@@ -157,6 +177,8 @@ const char* last_error_string();
 // fold the scaling into the SYRK? (opts.fold_scaling / CIP_FOLD_SCALING, else free memory against the mn-double
 // second copy plus `ahead` bytes not allocated yet); `can`: the fold applies to the rows of the SYRK
 int engine_decide_fold(cip_engine* h, bool can, size_t mn, bool* fold, size_t ahead = 0);
+// upload a CSC matrix (host or device arrays) and scatter it into a zero-initialised Q4 buffer (engine.cu)
+int engine_upload_csc(cip_engine* h, double* dst, int ld, const cip_csc* M, int transpose);
 // buffers / streams of the overlapped Gram reduction, once the communicator exists (engine.cu)
 int engine_setup_comm(cip_engine* h);
 
@@ -201,6 +223,21 @@ int split_add_delta(cip_engine* h, double delta);
 int split_solve(cip_engine* h, double** nv, double** pv, int b, bool schur);
 int split_mul_Q(cip_engine* h, double* y, const double* x);
 int split_get_H(cip_engine* h, double* tmp);   // n x n, column-major
+
+// ---- eliminate_y (eliminate_y.cu)
+// LEVEL 1, after the cone tables and the fold decision, before A, F or any n_pad^2 buffer is allocated: take the
+// m-space form?  Applies the option (and, in auto mode, the free-memory test of the n-space form); checks that Q is
+// diagonal and Q_jj + delta > 0.  `shard`: a shard of a multi-GPU handle (never).  Sets h->ey.on / automatic.
+int ey_decide(cip_engine* h, bool shard, const double* Q, int ldq, const cip_csc* Qs);
+// LEVEL 1, when h->ey.on: every buffer of the form, A4 and G4 uploaded, C, E', P formed, the Cholesky plans
+int ey_create(cip_engine* h, const double* A, int lda, const cip_csc* As, const double* G, int ldg, const cip_csc* Gs);
+// LEVEL 2: M4 = C + F'F (records ev[1], ev[2])
+int ey_form_M(cip_engine* h);
+// LEVEL 3, one column: the solve of cip_solve (device or staged pointers; dy / dv outputs of length n / m)
+int ey_solve(cip_engine* h, const double* ry, const double* rw, const double* rv, double* dy, double* dw, double* dv);
+int ey_solve_H(cip_engine* h, const double* rhs, double* x);      // x = H^-1 rhs, n-vectors on the device
+int ey_get_M(cip_engine* h, double* tmp);                          // m x m, column-major (device buffer)
+int ey_mul_Q(cip_engine* h, double* y, const double* x);           // y = Q x (diagonal, without delta)
 
 // ---- single-process multi-GPU front (multi.cu): same contracts as the C ABI entry points, global vectors
 int multi_create(cip_handle* out, int n, int m, int p, const double* Q, int ldq, const double* A, int lda,

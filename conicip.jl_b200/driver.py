@@ -17,7 +17,7 @@ import numpy as np
 
 from ._lib import OP_F, OP_FINVT, OP_FT
 from .blocks import Block, DeviceBlock, Diagonal
-from .kktsolver import kktsolver_b200
+from .kktsolver import kktsolver_b200, make_kktsolver
 
 
 @dataclass
@@ -63,15 +63,18 @@ class LocalReducer:
         return list(xs)
 
 
-def conicIP_native(Q, c, A, b, cone_dims, G=None, d=None, *, engine=None, ngpus=1, row_structure=0, **opts):
+def conicIP_native(Q, c, A, b, cone_dims, G=None, d=None, *, engine=None, ngpus=1, row_structure=0, eliminate_y=0,
+                   **opts):
     """Same problem statement and options as `conicIP`, but the loop itself runs inside the library
     (`cip_ipm_solve`, SURVEY 8f rank 1): one C call per solve.  Pass `engine=` to reuse a handle;
     `ngpus > 1` row-shards A over that many devices of this process (`cip_options.ngpus`);
     `row_structure=1` exploits the row structure of A when forming H (`cip_options.row_structure`);
-    `row_structure=2` also factors H as its diagonal plus the coupled block, with no n x n buffer."""
+    `row_structure=2` also factors H as its diagonal plus the coupled block, with no n x n buffer;
+    `eliminate_y=1` factors the m x m F'F + A D^-1 A' instead of H where Q + reg_delta I is diagonal and positive
+    (`cip_options.eliminate_y`; 0 = only when H would not fit, 2 = never)."""
     from .engine import Engine
     eng = engine or Engine(Q, A, G if (G is not None and G.shape[0]) else None, cone_dims, ngpus=ngpus,
-                           row_structure=row_structure)
+                           row_structure=row_structure, eliminate_y=eliminate_y)
     y, w, v, info = eng.ipm_solve(np.asarray(c, dtype=np.float64), np.asarray(b, dtype=np.float64),
                                   None if d is None else np.asarray(d, dtype=np.float64), **opts)
     sol = Solution(np.asarray(y), np.asarray(w), np.asarray(v), status=info["status"], Iter=info["Iter"],
@@ -85,7 +88,7 @@ def conicIP_native(Q, c, A, b, cone_dims, G=None, d=None, *, engine=None, ngpus=
 
 def conicIP(Q, c, A, b, cone_dims, G=None, d=None, *, kktsolver=kktsolver_b200,
             optTol=1e-6, DTB=0.01, verbose=False, maxRefinementSteps=3, maxIters=100,
-            infeasTol=None, refinementThreshold=None, reducer=None, global_cone_dims=None):
+            infeasTol=None, refinementThreshold=None, reducer=None, global_cone_dims=None, eliminate_y=0):
     import torch
 
     if not torch.cuda.is_available():
@@ -169,6 +172,10 @@ def conicIP(Q, c, A, b, cone_dims, G=None, d=None, *, kktsolver=kktsolver_b200,
     normd = -math.inf if p == 0 else nrm(d_t)
     normb = mnrm(b_t)
 
+    if eliminate_y != 0:              # cip_options.eliminate_y for the stock kktsolver (0 = its own default)
+        if kktsolver is not kktsolver_b200:
+            raise ValueError("eliminate_y= applies to the default kktsolver; bind it with make_kktsolver(eliminate_y=...)")
+        kktsolver = make_kktsolver(eliminate_y=eliminate_y)
     solve3x3gen = kktsolver(Q, A, G, cone_dims)                      # :667  LEVEL 1
     eng = solve3x3gen.engine
 

@@ -36,7 +36,8 @@ class Engine:
     """LEVEL-1 object: `kktsolver(Q, A, G, cone_dims)` (src/ConicIP.jl:667)."""
 
     def __init__(self, Q, A, G, cone_dims, *, reg_delta=0.0, reg_eps_G=0.0, device=-1,
-                 use_torch_stream=True, dist_chol=-1, aug_rho=-1.0, ngpus=1, fold_scaling=0, row_structure=0):
+                 use_torch_stream=True, dist_chol=-1, aug_rho=-1.0, ngpus=1, fold_scaling=0, row_structure=0,
+                 eliminate_y=0):
         L = lib()
         self.cone_dims = [(t, int(k)) for t, k in cone_dims]
         self.cone_type = np.array([CONE_CODE[t] for t, _ in self.cone_dims], dtype=np.int32)
@@ -56,6 +57,8 @@ class Engine:
         opts.fold_scaling = int(fold_scaling)   # 0 auto, 1 always, 2 never (R and Q cones: no Atil copy of A)
         opts.row_structure = int(row_structure)  # 1: singleton R rows on the diagonal, compact SYRK for the rest;
         #                                          2: also factor H as its diagonal plus the coupled block H_KK
+        opts.eliminate_y = int(eliminate_y)      # 0 auto (only when H would not fit), 1 wherever Q + reg_delta I is
+        #                                          diagonal and positive: factor the m x m F'F + A D^-1 A', 2 never
         self.ngpus = max(1, int(ngpus))
         self._torch = None
         self._use_torch_stream = use_torch_stream
@@ -423,6 +426,21 @@ class Engine:
         si.struct_size = C.sizeof(SplitInfo)
         check(lib().cip_split_info(self._h, C.byref(si)))
         return {k: getattr(si, k) for k, _ in SplitInfo._fields_ if k != "struct_size"}
+
+    def kkt_form_info(self):
+        """Which form the KKT system takes (`cip_kkt_form_info`): eliminate_y = 1 for the m-space form, automatic = 1
+        when the default option chose it because the n x n H would not fit."""
+        from ._lib import KktFormInfo
+        fi = KktFormInfo()
+        fi.struct_size = C.sizeof(KktFormInfo)
+        check(lib().cip_kkt_form_info(self._h, C.byref(fi)))
+        return {k: getattr(fi, k) for k, _ in KktFormInfo._fields_ if k != "struct_size"}
+
+    def get_M(self):
+        """m-space handles: M = F'F + A D^-1 A' (after a factorisation: its Cholesky factor), `cip_get_M`."""
+        out = np.zeros((self.m, self.m), order="F")
+        check(lib().cip_get_M(self._h, out.ctypes.data, max(self.m, 1)))
+        return out
 
     def get_H(self):
         out = np.zeros((self.n, self.n), order="F")

@@ -34,10 +34,13 @@ struct Options            # mirrors cip_options
     fold_scaling::Cint    # 0 auto, 1 always, 2 never: R-only problems without a second (scaled) copy of A
     row_structure::Cint   # 1: singleton R rows go onto the diagonal of H, the SYRK runs on the other rows (one GPU);
                           # 2: also factor H as its diagonal plus the coupled block H_KK (no n x n buffer)
+    eliminate_y::Cint     # 0 auto (only when H would not fit), 1: factor the m x m F'F + A D^-1 A' where
+                          # D = Q + reg_delta I is diagonal and positive (one GPU, row_structure = 0), 2 never
 end
-make_options(; device = -1, reg_delta = 0.0, q_kind = 0, ngpus = 1, fold_scaling = 0, row_structure = 0) =
+make_options(; device = -1, reg_delta = 0.0, q_kind = 0, ngpus = 1, fold_scaling = 0, row_structure = 0,
+             eliminate_y = 0) =
     Options(Cint(sizeof(Options)), Cint(device), reg_delta, 0.0, Cint(q_kind), Cint(0), Cint(-1), -1.0, Cint(ngpus),
-            Cint(fold_scaling), Cint(row_structure))
+            Cint(fold_scaling), Cint(row_structure), Cint(eliminate_y))
 
 lasterr() = unsafe_string(ccall((:cip_last_error, LIB), Cstring, ()))
 function check(rc::Cint)
@@ -58,13 +61,14 @@ Csc(M::SparseMatrixCSC{Float64,Int64}) = Csc(size(M, 1), size(M, 2), pointer(M.c
 mutable struct Engine
     h::Ptr{Cvoid}
     n::Int; m::Int; p::Int
-    function Engine(Q, A, G, cone_dims; reg_delta = 0.0, ngpus = 1, device = -1, fold_scaling = 0, row_structure = 0)
+    function Engine(Q, A, G, cone_dims; reg_delta = 0.0, ngpus = 1, device = -1, fold_scaling = 0, row_structure = 0,
+                    eliminate_y = 0)
         n = size(Q, 1); m = size(A, 1); p = size(G, 1)
         if A isa SparseMatrixCSC          # sparse LEVEL 1: no dense copy on the host (cip_create_csc)
             Qs = SparseMatrixCSC{Float64,Int64}(sparse(Q)); As = SparseMatrixCSC{Float64,Int64}(A)
             Gs = SparseMatrixCSC{Float64,Int64}(sparse(G))
             ct = Cint[CONE_CODE[t] for (t, _) in cone_dims]; cdim = Cint[k for (_, k) in cone_dims]
-            opts = Ref(make_options(; device, reg_delta, q_kind = 2, ngpus, fold_scaling, row_structure))
+            opts = Ref(make_options(; device, reg_delta, q_kind = 2, ngpus, fold_scaling, row_structure, eliminate_y))
             hp = Ref{Ptr{Cvoid}}(C_NULL)
             GC.@preserve Qs As Gs begin
                 rc = ccall((:cip_create_csc, LIB), Cint,
@@ -83,7 +87,7 @@ mutable struct Engine
         Gd = Matrix{Float64}(G)
         ct = Cint[CONE_CODE[t] for (t, _) in cone_dims]
         cdim = Cint[k for (_, k) in cone_dims]
-        opts = Ref(make_options(; device, reg_delta, q_kind = qk, ngpus, fold_scaling, row_structure))
+        opts = Ref(make_options(; device, reg_delta, q_kind = qk, ngpus, fold_scaling, row_structure, eliminate_y))
         hp = Ref{Ptr{Cvoid}}(C_NULL)
         rc = ccall((:cip_create, LIB), Cint,
                    (Ref{Ptr{Cvoid}}, Cint, Cint, Cint, Ptr{Cdouble}, Cint, Ptr{Cdouble}, Cint,

@@ -92,6 +92,27 @@ typedef struct cip_options {
                            avoid it).  cip_get_H scatters into n x n (zeros outside K x K and the diagonal); a
                            failing pivot is still reported as 1 + its global column.  CIP_ROW_STRUCTURE=2 selects it.
                            Sharded handles (ngpus > 1, cip_comm_init) reject 1 and 2. */
+  int    eliminate_y;   /* which variable the KKT system is reduced to.  The n-space form (every handle before this
+                           field) eliminates v and factors the n x n H = Q + A'(F'F)^-1 A.  The m-space form
+                           eliminates y instead; it needs D = Q + reg_delta*I diagonal with every entry > 0 and factors
+                           the m x m M = F'F + A D^-1 A' (C = A D^-1 A', E = A D^-1 G' and P = G D^-1 G' are formed
+                           once at cip_create), then the p x p S = P - E' M^-1 E.  A is kept once (no second copy, no
+                           n x n buffer), so wide problems (m << n, dense A, diagonal Q) fit where H would not.
+                           0 = auto (default): the m-space form only where it applies and the n-space form (after its
+                             fold_scaling decision) would not fit in free device memory -- every handle that can be
+                             created in the n-space form keeps it; choosing by cost is not done;
+                           1 = the m-space form wherever it applies; a handle where it does not (Q with an off-diagonal
+                             non-zero, Q_jj + reg_delta <= 0, row_structure != 0, ngpus > 1, m = 0) fails to create,
+                             and cip_comm_init on an m-space handle fails;
+                           2 = never.
+                           It applies to single-device handles with row_structure = 0: q_kind = 1; dense or CSC Q whose
+                           off-diagonal entries are all zero (checked at cip_create); Q = 0 (q_kind = 2, CSC Q == NULL)
+                           when reg_delta > 0.  aug_rho is not used (M is positive definite whenever F'F is).
+                           cip_factor then reports a failing pivot of M as 1 + its row of A and one of S as
+                           m + 1 + its row of G; cip_stats.ms_syrk times the assembly of M, syrk_flops is 0 (C was
+                           formed at cip_create) and chol_flops is m^3/3.  cip_get_H fails (see cip_get_M),
+                           cip_solve_H keeps its meaning (H^-1 rhs = D^-1 rhs - D^-1 A' M^-1 A D^-1 rhs) and cip_mul_Q
+                           returns Q x without reg_delta. */
 } cip_options;
 
 typedef struct cip_stats_t {
@@ -269,9 +290,20 @@ typedef struct cip_split_t {
   int cols_from_G;      /* columns where G has a non-zero, when aug_rho > 0 and p > 0 (else 0)             */
 } cip_split_t;
 int cip_split_info(cip_handle h, cip_split_t* out);
+/* Which form the KKT system of a handle takes (cip_options.eliminate_y). */
+typedef struct cip_kkt_form_t {
+  int struct_size;      /* = sizeof(cip_kkt_form_t), set by the caller                                      */
+  int eliminate_y;      /* 1: the m-space form (M = F'F + A D^-1 A' is factored), 0: the n-space form (H)   */
+  int automatic;        /* 1: eliminate_y = 0 (auto) chose the m-space form because H would not fit         */
+} cip_kkt_form_t;
+int cip_kkt_form_info(cip_handle h, cip_kkt_form_t* out);
 /* copy the current reduced matrix H (after cip_factor: its Cholesky factor L in the
- * lower triangle) into a column-major n*n buffer -- test/debug hook */
+ * lower triangle) into a column-major n*n buffer -- test/debug hook.  An m-space handle
+ * (cip_options.eliminate_y) has no H: the call fails, use cip_get_M. */
 int cip_get_H(cip_handle h, double* out, int ldo);
+/* m-space handles only: copy M = F'F + A D^-1 A' (after cip_factor: its Cholesky factor L)
+ * into a column-major m*m buffer, lower triangle as cip_get_H -- test/debug hook */
+int cip_get_M(cip_handle h, double* out, int ldo);
 /* form H = Q + (F^-T A)'(F^-T A) only (no factorisation) -- test/bench hook */
 int cip_form_H(cip_handle h);
 int cip_factor_H(cip_handle h);
